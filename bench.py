@@ -4,6 +4,7 @@ Terabyte-shape synthetic data (BASELINE.json metric), one process per GPU.
 
   python bench.py --gpus N --steps K --warmup W            (torchrun for N > 1)
   python bench.py --impl reference --gpus N --steps K --warmup W
+  python bench.py --steps K --dump-outputs DIR             (the last timed step's loss / predictions as .npy)
 
 A step = one full training iteration over one global batch: cache forward (probe + gather +
 pool), bottom/top MLPs (tcgen05 3xTF32 GEMMs, FP32 accuracy), pairwise-dot interaction fwd/bwd, BCE loss,
@@ -73,7 +74,16 @@ def parse():
     # measurement only: at a third of the timed region, enqueue this many GB of copy-engine host-to-device copies
     # (256 MB pinned chunks, side stream) beside the steps: what a cudaMemcpyAsync prefetch would cost the step
     ap.add_argument("--ce-probe-gb", type=float, default=0.0)
-    return ap.parse_args()
+    # what the last timed step returned to its caller (Trainer.step: the loss E and the predictions Z of rank 0's
+    # batch) as DIR/loss.npy and DIR/predictions.npy, float32; the inputs are seeded, so that two builds run with the
+    # same arguments can be compared output for output.  Not bit for bit: sums are accumulated in a different order
+    # from run to run, and two runs of the default workload (20 timed steps, one B200) differed by up to 2e-4
+    # relative in the predictions
+    ap.add_argument("--dump-outputs", type=str, default=None, metavar="DIR")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs dumps the GPU path's outputs; the reference arm has none")
+    return a
 
 
 def table_rows(wl, cap):
@@ -178,7 +188,6 @@ def cpu_reference_run(wl, ln_emb, steps, warmup, budget_s, dist, zipf_a):
     window of `look` steps so that the run fits the time budget."""
     import torch
     from oracle import oracle as O
-    from cdlrm_b200.main_no_ddp import ProcessArgs  # noqa: F401  (arg parity only)
     cores = os.cpu_count() or 1
     torch.set_num_threads(cores)
     try:        # torchrun exports OMP_NUM_THREADS=1: give numpy's BLAS / OpenMP pools all the host cores back
@@ -435,9 +444,9 @@ def gpu_run(a, wl, ln_emb):
         lo = b * lb
         if host is None:
             ids, X, Y = window(w)
-            E, _ = tr.step(X[lo:lo + lb], lS_o, ids[:, lo:lo + lb], Y[lo:lo + lb])
+            E, Z = tr.step(X[lo:lo + lb], lS_o, ids[:, lo:lo + lb], Y[lo:lo + lb])
             aggregate(j)
-            return E
+            return E, Z
         # end-to-end: inputs come from pinned host memory, the result goes back to the host
         hX, hI, hY = host
         E, _ = tr.step(hX[b].to(dev, non_blocking=True), lS_o, hI[b].to(dev, non_blocking=True),
@@ -506,14 +515,21 @@ def gpu_run(a, wl, ln_emb):
                 for _ in range(int(a.ce_probe_gb * 4)):
                     probe[1].copy_(probe[0], non_blocking=True)
                 probe[4].record()
-        one_step(j)
+        last = one_step(j)
         j += 1
         if (i + 1) % seg == 0 and i + 1 < K:
             m = torch.cuda.Event(enable_timing=True)
             m.record()
             marks.append((i + 1, m))
     ev1.record()
+    # copied behind the timed region, before the next step (a graph replay) overwrites the output buffers
+    dumped = [t.detach().clone() for t in last] if a.dump_outputs and rank == 0 else None
     torch.cuda.synchronize(dev)
+    if dumped is not None:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for name, t in zip(("loss", "predictions"), dumped):
+            np.save(os.path.join(a.dump_outputs, name + ".npy"), t.cpu().numpy().astype(np.float32))
+        log(f"last timed step's outputs written to {a.dump_outputs}")
     if cuprof:
         torch.cuda.profiler.stop()
     launches = int(lib.cdlrm_prof_launches(0))
