@@ -111,6 +111,9 @@ SIGNATURES = {
     "cdlrm_rngdev_raw": (C.c_int, [vp, vp, C.c_int64, vp]),
     "cdlrm_rngdev_exponential": (C.c_int, [vp, vp, C.c_int64, vp, vp]),
     "cdlrm_rngdev_draws": (C.c_uint64, [vp]),
+    "cdlrm_rngdev_get_state": (C.c_int, [vp, vp, C.POINTER(C.c_uint64), vp]),
+    "cdlrm_rngdev_set_state": (C.c_int, [vp, vp, C.c_uint64, vp]),
+    "cdlrm_cache_collect_valid": (C.c_int, [vp, C.c_int, C.c_int, vp, vp, c_i64p, vp, vp]),
     "cdlrm_rngdev_set_option": (C.c_int, [C.c_int, C.c_int64]),
     "cdlrm_exp_from_raw": (C.c_int, [vp, vp, C.c_int64, vp]),
     "cdlrm_plan_phase_b_dev": (C.c_int, [vp, vp, vp, C.c_int64, c_i64p, vp, vp, vp, vp, vp, vp, vp]),

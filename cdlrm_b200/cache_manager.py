@@ -87,6 +87,30 @@ class VictimRngDevice:
     def draws(self):
         return int(lib.cdlrm_rngdev_draws(self._h))
 
+    def snapshot(self, stream):
+        """(pinned int32 [625] state {x[624], pos}, draws, event): the state in the order of ``stream`` -- the state
+        tensor holds it once ``event`` has completed -- and the number of draws enqueued so far."""
+        state = torch.empty(625, dtype=torch.int32, pin_memory=True)
+        draws = ctypes.c_uint64()
+        check(lib.cdlrm_rngdev_get_state(self._h, _vp(state.data_ptr()), ctypes.byref(draws), _sp(stream)))
+        ev = torch.cuda.Event()
+        ev.record(stream)
+        return state, int(draws.value), ev
+
+    def get_state(self, stream=None):
+        """(uint32 numpy [625], draws) after everything enqueued on ``stream`` (default: current)."""
+        state, draws, ev = self.snapshot(stream or torch.cuda.current_stream(self.device))
+        ev.synchronize()
+        return state.numpy().view(np.uint32).copy(), draws
+
+    def set_state(self, state, draws, stream=None):
+        s = stream or torch.cuda.current_stream(self.device)
+        h = np.ascontiguousarray(np.asarray(state, dtype=np.uint32))
+        if h.shape != (625,):
+            raise ValueError("victim-stream state must hold 625 words, got shape %s" % (h.shape,))
+        check(lib.cdlrm_rngdev_set_state(self._h, _vp(h.ctypes.data), int(draws), _sp(s)))
+        s.synchronize()          # the host array may go away after the call
+
     def __del__(self):
         try:
             lib.cdlrm_rngdev_destroy(self._h)
@@ -576,6 +600,84 @@ class WindowPlanner:
         rec.wb_done = torch.cuda.Event(enable_timing=True)
         rec.wb_done.record(s)
 
+    # -- export of the cached rows into the master ----------------------------------------------------
+    # HBM staging of a copy-engine export, in rows of the grow-only "evict" buffer: the list is packed and written back
+    # in pieces of at most this many bytes
+    EXPORT_STAGE_BYTES = 2 << 30
+
+    def collect_valid(self, share=(0, 1)):
+        """Valid cache lines of every table whose set is in share r of W of the sets (cdlrm_cache_collect_valid), on the
+        planner's stream: (slots int32, ids int64 device tensors, offsets, counts); table k's list is
+        [off[k], off[k] + counts[k]), ascending by slot."""
+        s = self.stream
+        caps = [self.ways * int(S) for S in self.cg.cache_sizes]
+        off = [0] * self.T
+        for k in range(1, self.T):
+            off[k] = off[k - 1] + caps[k - 1]
+        h = torch.zeros(self.T, dtype=torch.int64).pin_memory()
+        with torch.cuda.stream(s):
+            slots = torch.empty(max(sum(caps), 1), dtype=torch.int32, device=self.dev)
+            ids = torch.empty(max(sum(caps), 1), dtype=torch.int64, device=self.dev)
+            check(lib.cdlrm_cache_collect_valid(self.ctx, int(share[0]), int(share[1]), _vp(slots.data_ptr()),
+                                                _vp(ids.data_ptr()), _lib.i64_array(off), _vp(h.data_ptr()), _sp(s)))
+        s.synchronize()
+        return slots, ids, off, h.tolist()
+
+    def write_cached_to_master(self, share=(0, 1)):
+        """master[k][id] = weight[k][slot] for every valid cache line of share r of W of the sets (what the eviction of
+        every cached row would write back); returns the number of rows.  ``pcie_mode`` "sm": the evict kernel writes the
+        master zero-copy (its PCIe-throttled grid).  "ce": the same kernel packs the rows into the HBM staging buffer
+        (at most EXPORT_STAGE_BYTES at a time) and cdlrm_host_writeback_rows scatters them into the master.  Runs on
+        the planner's stream after the current stream's work; returns when the rows are in the master."""
+        s = self.stream
+        s.wait_stream(torch.cuda.current_stream(self.dev))
+        slots, ids, off, cnt = self.collect_valid(share)
+        total = sum(cnt)
+        ce = self.pcie_mode == "ce" and not self.emb_tables.emb_l[0].weight.is_cuda
+        if not ce:
+            with torch.cuda.stream(s):
+                for k in range(self.T):
+                    if cnt[k]:
+                        check(lib.cdlrm_move_evict(self.ctx, k, _vp(ids[off[k]:].data_ptr()), _vp(slots[off[k]:].data_ptr()),
+                                                   None, cnt[k], None, 1, 0, _sp(s)))
+            s.synchronize()
+            return total
+        hid, hoff = self._ids_to_host("export_ids", ids, [(off[k], cnt[k]) for k in range(self.T)])
+        cap = max(1, min(total, self.EXPORT_STAGE_BYTES // (4 * self.dim)))
+        stage = self._buf("evict", cap)
+        rows_per, bufs, _evs = self._ce_chunks()
+
+        def flush(pieces):              # pieces: (table, offset in the table's list, rows, first staging row)
+            with torch.cuda.stream(s):
+                for k, o, n, r in pieces:
+                    check(lib.cdlrm_move_evict(self.ctx, k, _vp(ids[off[k] + o:].data_ptr()),
+                                               _vp(slots[off[k] + o:].data_ptr()), None, n, _vp(stage[r:].data_ptr()),
+                                               0, 0, _sp(s)))
+            Ws = [self.emb_tables.emb_l[k].weight.data for k, _o, _n, _r in pieces]
+            check(lib.cdlrm_host_writeback_rows(
+                self.dev.index, len(pieces), _lib.ptr_array([W.data_ptr() for W in Ws]),
+                _lib.i64_array([W.shape[0] for W in Ws]), self.dim,
+                _lib.ptr_array([hid.data_ptr() + 8 * (hoff[k] + o) for k, o, _n, _r in pieces]), None,
+                _lib.i64_array([n for _k, _o, n, _r in pieces]), _lib.ptr_array([stage[r:].data_ptr() for *_x, r in pieces]),
+                _vp(bufs[0].data_ptr()), _vp(bufs[1].data_ptr()), rows_per, 0, self.host_threads, _sp(s)))
+
+        pieces, used = [], 0
+        for k in range(self.T):
+            o = 0
+            while o < cnt[k]:
+                n = min(cnt[k] - o, cap - used)
+                pieces.append((k, o, n, used))
+                o += n
+                used += n
+                if used == cap:
+                    flush(pieces)
+                    pieces, used = [], 0
+        if pieces:
+            flush(pieces)
+        s.synchronize()
+        self._pin.pop("export_ids", None)         # a checkpoint-sized pinned list is not kept
+        return total
+
     # -- look-ahead staging -------------------------------------------------------------------
     def stage(self, rec):
         """Prefetch, on the planner's stream, everything window w+1 needs from the host master
@@ -921,17 +1023,28 @@ class Prefetcher(threading.Thread):
 
     def windows(self):
         """Generator of raw window id tensors [T, <= lookahead*mini_batch_size] in training
-        order: entry w covers steps [w*lookahead, (w+1)*lookahead) (SURVEY 3.4 invariant)."""
+        order: entry w covers steps [w*lookahead, (w+1)*lookahead) (SURVEY 3.4 invariant).  With
+        ``args.load_model`` the windows before the checkpoint's resume point are skipped (the loaders are
+        deterministic: the run that saved saw the same windows)."""
         per = self.args.lookahead
+        skip = 0
+        if getattr(self.args, "load_model", ""):
+            from .checkpoint import read_meta
+            skip = int(read_meta(self.args.load_model)["resume"]["window"])
+        w = 0
         for _epoch in range(self.args.nepochs):
             acc = []
             for _j, batch in enumerate(self.cache_ld):
                 acc.append(batch[2])
                 if len(acc) == per:
-                    yield torch.cat(acc, dim=1)
+                    if w >= skip:
+                        yield torch.cat(acc, dim=1)
+                    w += 1
                     acc = []
             if acc:
-                yield torch.cat(acc, dim=1)
+                if w >= skip:
+                    yield torch.cat(acc, dim=1)
+                w += 1
 
     @property
     def fifo_payload(self):

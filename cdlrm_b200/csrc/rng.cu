@@ -345,3 +345,28 @@ extern "C" int cdlrm_rngdev_exponential(cdlrm_rngdev* r, float* d_out, int64_t n
     if (rc) return rc;
     return cdlrm_exp_from_raw(d_raw_scratch, d_out, n, stream);
 }
+
+// Checkpoint of the device stream.  It keeps x[624] and pos (words of the current block already used) in HBM, and the host keeps the
+// number of draws, from which cdlrm_rngdev_raw derives pos: the two must agree.
+static int pos_of_draws(uint64_t draws) { return draws == 0 ? MT_N : (int)((draws * 2 - 1) % MT_N) + 1; }
+
+extern "C" int cdlrm_rngdev_get_state(cdlrm_rngdev* r, uint32_t* h_state, uint64_t* h_draws, cdlrm_stream stream) {
+    ARG_CHECK(r && h_state && h_draws);
+    CU_CHECK(cudaSetDevice(r->device));
+    CU_CHECK(cudaMemcpyAsync(h_state, r->d_state, sizeof(uint32_t) * (MT_N + 1), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+    *h_draws = r->draws;
+    return CDLRM_OK;
+}
+
+extern "C" int cdlrm_rngdev_set_state(cdlrm_rngdev* r, const uint32_t* h_state, uint64_t draws, cdlrm_stream stream) {
+    ARG_CHECK(r && h_state);
+    if ((int)h_state[MT_N] != pos_of_draws(draws)) {
+        cdlrm_set_error("rngdev state: position %u does not match %llu draws (expected %d)", h_state[MT_N],
+                        (unsigned long long)draws, pos_of_draws(draws));
+        return CDLRM_ERR_ARG;
+    }
+    CU_CHECK(cudaSetDevice(r->device));
+    CU_CHECK(cudaMemcpyAsync(r->d_state, h_state, sizeof(uint32_t) * (MT_N + 1), cudaMemcpyHostToDevice, (cudaStream_t)stream));
+    r->draws = draws;
+    return CDLRM_OK;
+}

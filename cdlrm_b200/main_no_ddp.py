@@ -21,6 +21,7 @@ import torch.distributed as dist
 import torch.nn as nn
 
 from . import _lib
+from . import checkpoint as ckpt
 from ._lib import check, lib
 from .cache_manager import Prefetcher, TorchGlobalRng, VictimRng, VictimRngDevice, WindowPlanner
 from .model_no_ddp import DLRM_Net, Embedding_Table_Cache_Group, Embedding_Table_Group, bce_mean, bce_mean_with_grad
@@ -419,6 +420,7 @@ class Trainer:
         # else rank 0 writes the whole list, as the reference's one eviction manager does)
         shared_master = bool(getattr(emb_tables, "_mapped_file", False)) or \
             all(bool(e.weight.is_shared()) for e in getattr(emb_tables, "emb_l", []))
+        self.shared_master = shared_master
         self.wb_sharded = (world > 1 and self.planner is not None and shared_master
                            and os.environ.get("CDLRM_WB_SHARDED", "1") != "0")
         # un-cached ids of a window (the same on every rank): one store sharded over the node's GPUs and read over
@@ -451,6 +453,15 @@ class Trainer:
         self.input_slots = 6             # stage_inputs: device-side input slots (host runs up to 5 steps ahead)
         self.keep_losses = False         # tests: keep every step's loss tensor (no sync) in loss_history
         self.loss_history = []
+        # position in the run (checkpoints): windows installed, steps run, steps of the installed window so far and
+        # in all; windows submitted and the steps each one holds; victim-stream state at the start of every plan
+        self._ln_bot, self._ln_top = [int(x) for x in ln_bot], [int(x) for x in ln_top]
+        self.window = self.global_step = self.steps_in_window = 0
+        self._window_steps = 0
+        self._n_submitted = 0
+        self._submitted_steps = []
+        self._rng_snaps = {}
+        self._finished = False
 
     # -- look-ahead -------------------------------------------------------------------------
     def submit_window(self, win_ids, own_ids=None):
@@ -479,6 +490,12 @@ class Trainer:
             own_ids = own_ids.to(self.dev, non_blocking=True).contiguous()
         else:
             own_ids = None
+        if isinstance(win_ids, torch.Tensor):
+            self._submitted_steps.append(-(-int(win_ids.shape[1]) // (self.local_batch * self.world)))
+        else:
+            self._submitted_steps.append(None)
+        idx = self._n_submitted
+        self._n_submitted += 1
         ev = torch.cuda.Event()
         ev.record(torch.cuda.current_stream(self.dev))   # ids produced on the current stream are ready
         prev = self._plan_thread
@@ -489,6 +506,8 @@ class Trainer:
             torch.cuda.set_device(self.dev)
             self.side.wait_event(ev)
             try:
+                # the victim-stream state this plan starts from: what a checkpoint at the boundary before it records
+                self._rng_snaps[idx] = self.planner.rng.snapshot(self.side)
                 # (copy-engine mode) evicted rows of the window just installed go back to the host master first
                 self.planner.flush_writeback()
                 if own_ids is not None:
@@ -522,9 +541,11 @@ class Trainer:
         self._plan_thread = threading.Thread(target=work, daemon=True)
         self._plan_thread.start()
 
-    def install_window(self):
+    def install_window(self, steps=None):
         """Window boundary (main_no_ddp.py:393-399): wait for the plan, average touched rows
-        over ranks, evict (rank 0 writes the master back), fill."""
+        over ranks, evict (rank 0 writes the master back), fill.  ``steps``: the number of training steps of this
+        window (default: from its ids when it was submitted as an id tensor, else ``lookahead``) -- where the next
+        window boundary is, for ``save_checkpoint`` / ``sync_master``."""
         t0 = time.perf_counter()
         rec = self._plan_q.get()
         if isinstance(rec, Exception):
@@ -547,6 +568,13 @@ class Trainer:
                                     average_on_writeback=self.args.average_on_writeback,
                                     wb_share=(self.rank, self.world) if self.wb_sharded else None)
         self._installed = rec            # keeps the loser store of this window alive
+        expected = self._submitted_steps.pop(0) if self._submitted_steps else None
+        self._window_steps = int(steps or expected or self.args.lookahead)
+        self.window += 1
+        self.steps_in_window = 0
+        self._finished = False
+        for i in [i for i in self._rng_snaps if i < self.window]:
+            del self._rng_snaps[i]
         t4 = time.perf_counter()
         self.caching_overhead.append(t4 - t0)
         # host milliseconds of the boundary: waiting for the plan, draining the stream for the device flags,
@@ -637,6 +665,8 @@ class Trainer:
 
     def step(self, X, lS_o, lS_i, T):
         self.steps_since_agg += 1
+        self.global_step += 1
+        self.steps_in_window += 1
         if getattr(self, "_graph", None) is not None and tuple(lS_i.shape) == tuple(self._g_in[1].shape):
             self._g_in[0].copy_(X, non_blocking=True)
             self._g_in[1].copy_(lS_i, non_blocking=True)
@@ -771,11 +801,184 @@ class Trainer:
             self._installed.wb_done.synchronize()
         torch.cuda.synchronize(self.dev)
         self.cache_group.check_device_flags()
+        self._finished = True
 
     def maybe_aggregate(self, j):
         if self.world > 1 and j > 0 and j % self.args.table_agg_freq == 0:     # :418-420
             broadcast_and_aggregate(self.cache_group, None, self.rank, self.args.table_agg_op)
             self.steps_since_agg = 0
+
+    # -- export, checkpoint, resume --------------------------------------------------------------
+    # A checkpoint describes the boundary before window w: every step of the windows < w has run, window w is neither
+    # installed nor counted as planned.  A plan(w) already in flight or staged is left alone (the run that saves goes
+    # on with it); the victim-stream state recorded is the one plan(w) started from, and a resumed Trainer plans w
+    # from the restored live tags and that state, as the uninterrupted run did.
+
+    def at_boundary(self):
+        """Every step of the installed window has run (or no window is installed yet)."""
+        return self.steps_in_window == (self._window_steps if self._installed is not None else 0)
+
+    def _need_planner(self, what):
+        if self.planner is None:
+            raise _lib.CdlrmError(f"{what} needs the look-ahead planner (not available under --strict-reference)")
+
+    def _quiesce(self):
+        """Wait for the plan thread and complete the pending eviction write-back: the master then holds every row
+        evicted so far, and nothing but the caller touches the cache or the master."""
+        if self._plan_thread is not None:
+            self._plan_thread.join()
+        self.planner.flush_writeback()
+        if self._installed is not None and self._installed.wb_done is not None:
+            self._installed.wb_done.synchronize()
+        torch.cuda.synchronize(self.dev)
+        self.cache_group.check_device_flags()
+
+    def _aggregate_replicas(self):
+        if self.world > 1:
+            broadcast_and_aggregate(self.cache_group, None, self.rank, self.args.table_agg_op)
+            self.steps_since_agg = 0
+            torch.cuda.synchronize(self.dev)
+
+    def sync_master(self):
+        """Write every valid cache line into the host master: afterwards ``emb_tables.emb_l[k].weight`` is the
+        trained table k.  Legal at a window boundary or after ``finish()``; under ``--average-on-writeback`` only
+        after ``finish()`` (the master's stale row of a cached id is part of its later eviction average).  In the
+        other modes it changes no later decision or value: the master row of a cached id is read by nobody before
+        the eviction of that id overwrites it (fills and the loser store read un-cached ids only).  At N > 1 the
+        replicas are aggregated first; each rank writes its share of the sets when the master is one shared object
+        (``wb_sharded``), else rank 0 writes everything.  Returns the number of rows this rank wrote."""
+        self._need_planner("sync_master")
+        if self.args.average_on_writeback and not self._finished:
+            raise _lib.CdlrmError("sync_master under --average-on-writeback needs finish() first: the master's rows of "
+                                  "cached ids are part of their later eviction averages")
+        if not self._finished and not self.at_boundary():
+            raise _lib.CdlrmError(f"sync_master: not at a window boundary ({self.steps_in_window} of "
+                                  f"{self._window_steps} steps of window {self.window - 1} have run)")
+        self._quiesce()
+        self._aggregate_replicas()
+        n = 0
+        if self.rank == 0 or self.wb_sharded:
+            n = self.planner.write_cached_to_master((self.rank, self.world) if self.wb_sharded else (0, 1))
+        if self.world > 1:
+            dist.barrier(group=self._host_group)
+        return n
+
+    def _dense_tensors(self):
+        if self.flat:
+            return [self.dlrm.flat_params]
+        return [p.data for p in self.dlrm.parameters()]
+
+    def checkpoint_fields(self):
+        """The meta data a checkpoint must share with this Trainer to be loaded into it (checkpoint.check_meta)."""
+        a, cg = self.args, self.cache_group
+        return {
+            "format": ckpt.FORMAT,
+            "shapes": {"ln_emb": [int(n) for n in cg.ln_emb], "dim": int(cg.dim), "ways": int(cg.num_ways),
+                       "num_sets": [int(S) for S in cg.cache_sizes], "aux_rows": int(cg.aux_table_size),
+                       "ln_bot": self._ln_bot, "ln_top": self._ln_top},
+            "args": {"seed": int(a.numpy_rand_seed), "cache_size": int(a.cache_size), "ways": int(a.num_ways),
+                     "lookahead": int(a.lookahead), "global_batch": int(a.mini_batch_size), "world_size": int(self.world),
+                     "table_agg_op": a.table_agg_op, "average_on_writeback": bool(a.average_on_writeback),
+                     "learning_rate": float(a.learning_rate), "lr_embeds": float(a.lr_embeds)},
+        }
+
+    def save_checkpoint(self, path, epoch=0):
+        """Write the state at the current window boundary into the directory ``path`` (checkpoint.py: written as
+        ``path.tmp``, then renamed into place).  Changes no training state: the cache rows are NOT written into the
+        master.  At N > 1 the replicas are aggregated first (the install of the next window then finds nothing dirty),
+        and rank 0 writes, with host barriers around the write.  ``epoch``: the epoch the resume point lies in.
+        ``last_checkpoint_s``: seconds of device-to-host copies and of file I/O."""
+        self._need_planner("save_checkpoint")
+        if not self.at_boundary():
+            raise _lib.CdlrmError(f"save_checkpoint: not at a window boundary ({self.steps_in_window} of "
+                                  f"{self._window_steps} steps of window {self.window - 1} have run)")
+        w = self.window
+        self._quiesce()
+        snap = self._rng_snaps.get(w)
+        if snap is None:                          # plan(w) not submitted: the stream stands where plan(w) will start
+            snap = self.planner.rng.snapshot(self.side)
+        state, draws, ev = snap
+        ev.synchronize()
+        self._aggregate_replicas()
+        meta = dict(self.checkpoint_fields(),
+                    resume={"epoch": int(epoch), "window": int(w), "global_step": int(self.global_step)},
+                    rng={"state": [int(x) for x in state.numpy().view(np.uint32)], "draws": int(draws)})
+        if self.world > 1:
+            dist.barrier(group=self._host_group)  # every rank's share of the write-back is in the shared master
+        d2h = 0.0
+        if self.rank == 0:
+            wr = ckpt.Writer(path)
+            t0 = time.perf_counter()
+            dense = torch.cat([t.reshape(-1) for t in self._dense_tensors()]).cpu()
+            d2h += time.perf_counter() - t0
+            wr.put("dense.bin", dense.numpy())
+            cg = self.cache_group
+            for k in range(len(cg.emb_l)):
+                t0 = time.perf_counter()
+                tags = cg.occupancy_tables[k].cpu()
+                rows = cg.emb_l[k].weight.data[:cg.num_ways * cg.cache_sizes[k]].cpu()
+                d2h += time.perf_counter() - t0
+                wr.put(f"tags_{k}.bin", tags.numpy())
+                wr.put(f"cache_{k}.bin", rows.numpy())
+                del tags, rows
+                M = self.emb_tables.emb_l[k].weight.data
+                wr.put(f"master_{k}.bin", (M.cpu() if M.is_cuda else M).numpy())    # straight from host storage
+            wr.commit(meta)
+            self.last_checkpoint_s = {"device_to_host": round(d2h, 4), "file_io": round(wr.io_s, 4)}
+        if self.world > 1:
+            dist.barrier(group=self._host_group)
+        return meta
+
+    def load_checkpoint(self, path):
+        """Restore a checkpoint into this freshly built Trainer (same arguments and shapes; a mismatch raises
+        ``checkpoint.CheckpointMismatch`` naming the field) and return the window w to submit next.  Restores the
+        live and the planner's tags, the cache rows, the master (at N > 1 rank 0 writes a shared master, the others
+        wait), the dense parameters and the victim-stream state as of the start of plan(w).  The CUDA graph is
+        captured afterwards, as usual."""
+        self._need_planner("load_checkpoint")
+        if self._installed is not None or self.global_step or self._n_submitted:
+            raise _lib.CdlrmError("load_checkpoint needs a freshly built Trainer")
+        meta = ckpt.read_meta(path)
+        ckpt.check_meta(meta, self.checkpoint_fields())
+        rd = ckpt.Reader(path, meta)
+        dev, cg = self.dev, self.cache_group
+        h2d = 0.0
+        for k in range(len(cg.emb_l)):
+            S, ways = cg.cache_sizes[k], cg.num_ways
+            tags = rd.read_into(f"tags_{k}.bin", np.empty((S, ways), np.int64))
+            rows = rd.read_into(f"cache_{k}.bin", np.empty((ways * S, cg.dim), np.float32))
+            t0 = time.perf_counter()
+            cg.occupancy_tables[k].copy_(torch.from_numpy(tags))
+            self.planner.plan_tags[k].copy_(cg.occupancy_tables[k])
+            cg.emb_l[k].weight.data[:ways * S].copy_(torch.from_numpy(rows))
+            h2d += time.perf_counter() - t0
+        if self.rank == 0 or not self.shared_master:
+            for k, E in enumerate(self.emb_tables.emb_l):
+                M = E.weight.data
+                if M.is_cuda:
+                    M.copy_(torch.from_numpy(rd.read_into(f"master_{k}.bin", np.empty(tuple(M.shape), np.float32))))
+                else:
+                    rd.read_into(f"master_{k}.bin", M.numpy())
+        dense_t = self._dense_tensors()
+        dense = rd.read_into("dense.bin", np.empty(sum(t.numel() for t in dense_t), np.float32))
+        t0 = time.perf_counter()
+        o = 0
+        with torch.no_grad():
+            for t in dense_t:
+                t.copy_(torch.from_numpy(dense[o:o + t.numel()]).view_as(t))
+                o += t.numel()
+        self.dlrm.invalidate_weight_splits()        # the hi / lo operand copies belong to the old weights
+        self.planner.rng.set_state(np.asarray(meta["rng"]["state"], dtype=np.uint32), meta["rng"]["draws"], self.side)
+        torch.cuda.synchronize(dev)
+        h2d += time.perf_counter() - t0
+        r = meta["resume"]
+        self.window = self._n_submitted = int(r["window"])
+        self.global_step = int(r["global_step"])
+        self.resume_epoch = int(r["epoch"])
+        self.last_checkpoint_s = {"host_to_device": round(h2d, 4), "file_io": round(rd.io_s, 4)}
+        if self.world > 1:
+            dist.barrier(group=self._host_group)
+        return self.window
 
 
 def _bcast_fifo_entry(item, rank, dev):
@@ -823,12 +1026,19 @@ def Run(rank, m_spa, ln_emb, ln_bot, ln_top, train_ld, test_ld, batch_fifo, evic
 
     ``--strict-reference``: the reference's literal loop (:393-425) on the same-named functions --
     ``load_caches_and_broadcast`` + ``wait_wrap`` at every window, ``cache_group(...)``, ``dlrm(...)``,
-    ``aggregate_gradients``, both optimizers, ``broadcast_and_aggregate`` on explicit slot windows."""
+    ``aggregate_gradients``, both optimizers, ``broadcast_and_aggregate`` on explicit slot windows.
+
+    ``--save-model PATH``: a checkpoint (Trainer.save_checkpoint) at the end of every epoch, replacing the previous
+    one, and ``sync_master()`` after the last step, so that ``emb_tables`` holds the trained tables when Run returns.
+    ``--load-model PATH``: resume at the checkpoint's window; the steps before it are skipped (``batch_fifo`` must
+    start at that window: ``Prefetcher`` skips the windows before it).  Neither works with ``--strict-reference``."""
     os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
     os.environ.setdefault("MASTER_PORT", str(args.master_port))
     if args.world_size > 1 and not dist.is_initialized():
         dist.init_process_group("nccl", rank=rank, world_size=args.world_size)
     strict = bool(getattr(args, "strict_reference", False))
+    if strict and (args.save_model or args.load_model):
+        raise _lib.CdlrmError("--save-model / --load-model need the look-ahead trainer (not --strict-reference)")
     tr = Trainer(args, m_spa, ln_emb, ln_bot, ln_top, emb_tables, rank=rank, world=args.world_size,
                  strict_reference=strict)
     dev, lb, L = tr.dev, tr.local_batch, args.lookahead
@@ -837,8 +1047,10 @@ def Run(rank, m_spa, ln_emb, ln_bot, ln_top, train_ld, test_ld, batch_fifo, evic
     torch.cuda.set_stream(torch.cuda.Stream(dev, priority=-1))
     share_occupancy_tables(tr.cache_group, occupancy_tables_fifos, rank)
     shared_fifo = args.world_size > 1 and not getattr(args, "fifo_per_rank", False)
-    n_windows = args.nepochs * math.ceil(len(train_ld) / L)
-    popped = 0
+    per_epoch = math.ceil(len(train_ld) / L)
+    n_windows = args.nepochs * per_epoch
+    start_w = tr.load_checkpoint(args.load_model) if args.load_model else 0
+    popped = start_w
 
     def next_entry():
         nonlocal popped
@@ -852,11 +1064,13 @@ def Run(rank, m_spa, ln_emb, ln_bot, ln_top, train_ld, test_ld, batch_fifo, evic
     total_time = total_loss = total_accu = 0.0
     total_iter = total_samp = 0
     idxs_window = []
-    if not strict:
+    if not strict and popped < n_windows:
         tr.submit_window(next_entry())
     step_no = 0
     for epoch in range(args.nepochs):
         for j, (X, lS_o, lS_i, T) in enumerate(train_ld):
+            if epoch * per_epoch + j // L < start_w:                                 # before the resume point
+                continue
             X, lS_o, lS_i, T = slice_batch(rank, lb, X, lS_o, lS_i, T)               # :388-391
             X, lS_i, T = (t.to(dev, non_blocking=True) for t in (X, lS_i, T))
             if j % L == 0:                                                           # :393-399
@@ -866,7 +1080,7 @@ def Run(rank, m_spa, ln_emb, ln_bot, ln_top, train_ld, test_ld, batch_fifo, evic
                     wait_wrap(load_caches_and_broadcast(tr.cache_group, batch_fifo, eviction_fifo, rank))
                     tr.caching_overhead.append(time.perf_counter() - t0)
                 else:
-                    tr.install_window()
+                    tr.install_window(steps=min(L, len(train_ld) - j))
                     nxt = next_entry()
                     if nxt is not None:
                         tr.submit_window(nxt)
@@ -915,8 +1129,12 @@ def Run(rank, m_spa, ln_emb, ln_bot, ln_top, train_ld, test_ld, batch_fifo, evic
                 # a test batch larger than the aux region raises IndexError in the reference (:176-179)
                 tr.cache_group.check_device_flags()
                 print('Test accuracy = {}%'.format(100 * (total_test_acc / max(test_samp, 1))))
+        if args.save_model and (epoch + 1) * per_epoch > start_w:
+            tr.save_checkpoint(args.save_model, epoch=epoch + 1)
     torch.cuda.synchronize(dev)
     tr.finish()
+    if args.save_model:
+        tr.sync_master()
     return tr
 
 

@@ -303,6 +303,16 @@ int cdlrm_agg_pack(cdlrm_ctx* ctx, const int32_t* slot_list, const int64_t* h_co
 int cdlrm_agg_unpack(cdlrm_ctx* ctx, const int32_t* slot_list, const int64_t* h_counts,
                      const float* buf, int clear_dirty, cdlrm_stream stream);
 
+/* ---- checkpoint / export of the trained tables (csrc/ckpt.cu).  No reference counterpart: the reference parses
+ *      --save-model / --load-model and ignores them, and its cache rows never reach the master at exit. --------------
+ * For every table k, the valid lines (live tag >= 0) whose set lies in rank `rank`'s share
+ * [S_k * rank / world, S_k * (rank + 1) / world) of the sets, in ascending slot order (slot = S_k * way + set):
+ * slots[h_list_off[k] + i] (int32) and ids[h_list_off[k] + i] (int64, the tag of that line), i < h_counts[k].
+ * The list of table k needs room for num_ways * S_k entries.  h_counts: pinned host int64 [num_tables], valid after
+ * `stream` is synchronised.  The shares of `world` ranks cover every valid line exactly once. */
+int cdlrm_cache_collect_valid(cdlrm_ctx* ctx, int rank, int world, int32_t* slots, int64_t* ids,
+                              const int64_t* h_list_off, int64_t* h_counts, cdlrm_stream stream);
+
 /* ---- host memory: pin (cudaHostRegister, mapped + portable) a master table that lives
  *      in ordinary or shared host memory (emb_tables.share_memory(), main_no_ddp.py:621-622)
  *      and return its device-visible address ---------------------------------------- */
@@ -410,6 +420,12 @@ int cdlrm_rngdev_raw(cdlrm_rngdev* rng, uint32_t* d_out, int64_t n_draws, cdlrm_
 int cdlrm_rngdev_exponential(cdlrm_rngdev* rng, float* d_out, int64_t n, uint32_t* d_raw_scratch,
                              cdlrm_stream stream);
 uint64_t cdlrm_rngdev_draws(const cdlrm_rngdev* rng);
+/* Checkpoint of the stream: h_state = 625 host words {x[624], pos}.  get: copies the state in stream order
+ * (cudaMemcpyAsync on `stream`: pinned h_state is valid once the stream has reached the copy) and writes the
+ * number of draws enqueued so far to *h_draws.  set: replaces the state in stream order; pos must be the one that
+ * `draws` implies (an error otherwise). */
+int cdlrm_rngdev_get_state(cdlrm_rngdev* rng, uint32_t* h_state, uint64_t* h_draws, cdlrm_stream stream);
+int cdlrm_rngdev_set_state(cdlrm_rngdev* rng, const uint32_t* h_state, uint64_t draws, cdlrm_stream stream);
 /* key 0: smallest request (32-bit words) generated chunk-parallel by mt19937 jump-ahead (default 0: every request of
  * two or more chunks of 2.56 M words); -1 = always the sequential single-CTA kernel.  Same stream either way. */
 int cdlrm_rngdev_set_option(int key, int64_t value);
