@@ -10,19 +10,20 @@
 // TMEM: relative error ~2^-21 per product, the same order as an FP32 FMA chain.
 //
 // One GEMM kernel serves forward, data-gradient and weight-gradient:
-//     D[M,N] = A[M,K] * B[N,K]^T        A, B row-major with K contiguous ("K-major"),
+//     D[M,N] = A[M,K] * B[N,K]^T
+// Each operand is read either K-major (row-major [M|N, K], K contiguous) or MN-major (row-major
+// [K, M|N], the M or N index contiguous: the transpose of a tensor that is stored row-major anyway).
 // A_hi/A_lo/B_hi/B_lo are four tensors in HBM, moved by TMA (128-byte swizzle) into a
 // 3-stage shared-memory ring; one elected thread of a persistent CTA issues tcgen05.mma.kind::tf32
 // (128x128x8, 12 per 32-wide k-block: 4 k-steps x 3 products) into a 128-column TMEM
 // accumulator; four epilogue warps read it back with tcgen05.ld and apply the fused
-// epilogue (bias, ReLU / sigmoid, ReLU-backward mask, hi/lo split of the result in
-// row-major AND transposed form -- the operand layouts the next GEMM needs -- or a
-// split-K atomic accumulation for the weight gradient).
-//   forward    Y  = act(X W^T + b)        A = X [B,K],      B = W   [N,K]
-//   dgrad      dX = (dZ W) * relu'(X)     A = dZ [B,N],     B = W^T [K,N]
-//   wgrad      dW = dZ^T X , db = dZ^T 1  A = dZ^T [N,B],   B = [X^T ; 1] [K+1,B]   (split-K)
-// The transposed copies are written by the epilogues that produce the tensors (the TMEM
-// lane = row mapping makes the transposed store the coalesced one).
+// epilogue (bias, ReLU / sigmoid, ReLU-backward mask, hi/lo split of the result row-major,
+// per-32-row column sums of the result, or a split-K reduce-add for the weight gradient).
+//   forward    Y  = act(X W^T + b)        A = X [B,K]   K-major,    B = W   [N,K]  K-major
+//   dgrad      dX = (dZ W) * relu'(X)     A = dZ [B,N]  K-major,    B = W^T from W [N,K]  MN-major
+//   wgrad      dW = dZ^T X                A = dZ^T from dZ [B,N]  MN-major,  B = X^T from X [B,K]  MN-major  (split-K)
+// The bias gradient db = column sums of dZ is taken where dZ is produced (dgrad epilogue, split_kernel,
+// narrow_bwd_kernel) as partial sums per 32 rows, reduced in a fixed order by unpack_batch_kernel.
 #include <cuda.h>
 
 #include "common.cuh"
@@ -52,8 +53,11 @@ constexpr int GEMM_SMEM = STAGES * STAGE_BYTES + EPI_WARPS * STG_BYTES + 1024 /*
 // depth, the k-block size or the number of TMA instructions.  (A_hi x [B_hi ; B_lo] as ONE
 // 128 x 256 x 8 MMA -- hi*hi and hi*lo side by side in TMEM -- is what the issuer does; it
 // saves an instruction, not the second read of A_hi.)
-// kind::tf32, FP32 accumulate, A and B K-major, M = 128, N = n
-__host__ __device__ constexpr uint32_t idesc_tf32(int n) { return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(BM >> 4) << 24); }
+// kind::tf32, FP32 accumulate, M = 128, N = n; bits 15 / 16: A / B MN-major instead of K-major
+__host__ __device__ constexpr uint32_t idesc_tf32(int n, int a_mn, int b_mn) {
+    return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)a_mn << 15) | ((uint32_t)b_mn << 16) | ((uint32_t)(n >> 3) << 17) |
+           ((uint32_t)(BM >> 4) << 24);
+}
 
 enum { ACT_NONE = 0, ACT_RELU = 1, ACT_SIGMOID = 2 };
 
@@ -71,15 +75,16 @@ struct Epi {
     int64_t ld_mask;
     int out_c;                   // 1: fp32 result row-major through map_c (2: reduce-add into it, split-K)
     int out_split;               // 1: hi/lo split row-major through map_c_hi / map_c_lo
-    int out_t;                   // 1: hi/lo split transposed through map_t_hi / map_t_lo
+    int a_mn, b_mn;              // 1: the operand is MN-major (see make_mn_map), 0: K-major
+    float* colsum;               // sums of the result over each group of 32 rows: colsum[(row / 32) * N + col] (or null)
 };
 
-// tensor maps of one launch: 4 operand maps (box 32 x 128, 128-byte swizzle) and up to 5 result
-// maps (box 32 x 32: row-major ones with the 128-byte swizzle, transposed ones dense)
+// tensor maps of one launch: 2 operand maps (128-byte swizzle) and up to 3 result maps (box 32 x 32,
+// 128-byte swizzle)
 struct Maps {
-    CUtensorMap a, b;            // operands: {K, rows, 2}: the hi and lo tensors are one 3-D tensor
+    CUtensorMap a, b;            // operands, hi and lo as one tensor: K-major {K, rows, 2}, MN-major {32, K, MN / 32, 2}
     CUtensorMap b_half;          // B again with a {BK, BN/2, 1} box: one CTA's share of a multicast B tile
-    CUtensorMap c, c_hi, c_lo, t_hi, t_lo;
+    CUtensorMap c, c_hi, c_lo;
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -119,6 +124,14 @@ __device__ __forceinline__ void tma_load_pair(uint32_t dst, const CUtensorMap* m
     asm volatile(
         "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
         ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(0), "r"(smem_u32(bar))
+        : "memory");
+}
+// MN-major operand tile: 4-D map {32, K, MN / 32, 2 (hi, lo)}, box {32, BK, 4, 2}; lands as hi then lo, each
+// four 32-wide column blocks of BK rows x 128 bytes (128-byte swizzle, 32-byte atoms: make_smem_desc_mn)
+__device__ __forceinline__ void tma_load_mn(uint32_t dst, const CUtensorMap* map, int k, int mn0, uint64_t* bar) {
+    asm volatile(
+        "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5}], [%6];"
+        ::"r"(dst), "l"(map), "r"(0), "r"(k), "r"(mn0 / 32), "r"(0), "r"(smem_u32(bar))
         : "memory");
 }
 // one half (BN/2 rows) of the hi (c2 = 0) or lo (c2 = 1) B tile, written to the same shared-memory offset of
@@ -186,6 +199,21 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr) {
     d |= (uint64_t)((8 * BK * 4) >> 4) << 32;
     d |= (uint64_t)1 << 46;
     d |= (uint64_t)(BK == 32 ? 2 : 4) << 61;
+    return d;
+}
+// MN-major: 32 MN elements (128 bytes) per row, one row per k.  For 32-bit (tf32) operands the tensor core takes
+// MN-major data only in the 128-byte swizzle with 32-byte atomicity (layout type 1, SWIZZLE_128B_BASE32B: 32-byte
+// chunks of a row XOR-ed with the row index mod 4; 4-row atoms), which the TMA writes with
+// CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B.  The plain 128-byte swizzle is read as a different layout.
+// The 32-wide column blocks are one TMA box (BK rows) apart (LBO), 4-row groups along K 512 bytes apart (SBO);
+// a k-step of 8 covers two atoms, so the next k-step starts 1024 bytes further on.
+__device__ __forceinline__ uint64_t make_smem_desc_mn(uint32_t saddr) {
+    uint64_t d = 0;
+    d |= (uint64_t)((saddr >> 4) & 0x3fff);
+    d |= (uint64_t)((32 * BK * 4) >> 4) << 16;
+    d |= (uint64_t)(4 * 128 >> 4) << 32;
+    d |= (uint64_t)1 << 46;
+    d |= (uint64_t)1 << 61;
     return d;
 }
 
@@ -273,8 +301,11 @@ gemm3x_tf32_kernel(const __grid_constant__ Maps maps, const Epi ep) {
                     const uint32_t base = smem_u32(smem + s * STAGE_BYTES);
                     const int k = (kb0 + i) * BK;
                     mbar_arrive_expect_tx(&full_bar[s], STAGE_BYTES);      // A + the whole B tile (own half + the peer's)
-                    tma_load_pair(base, &maps.a, k, m0, &full_bar[s]);
-                    if (cl == 2) {
+                    if (ep.a_mn) tma_load_mn(base, &maps.a, k, m0, &full_bar[s]);
+                    else tma_load_pair(base, &maps.a, k, m0, &full_bar[s]);
+                    if (ep.b_mn) {
+                        tma_load_mn(base + 2 * TILE_BYTES, &maps.b, k, n0, &full_bar[s]);
+                    } else if (cl == 2) {
                         const uint32_t off = (uint32_t)cr * (TILE_BYTES / 2);
                         tma_load_3d_mc(base + 2 * TILE_BYTES + off, &maps.b_half, k, n0 + cr * (BN / 2), 0, &full_bar[s], cl_mask);
                         tma_load_3d_mc(base + 3 * TILE_BYTES + off, &maps.b_half, k, n0 + cr * (BN / 2), 1, &full_bar[s], cl_mask);
@@ -303,16 +334,18 @@ gemm3x_tf32_kernel(const __grid_constant__ Maps maps, const Epi ep) {
                         TRACE(1, it);
                         tc_fence_after();
                         const uint32_t base = smem_u32(smem + s * STAGE_BYTES);
-                        const uint64_t a_hi = make_smem_desc(base);
-                        const uint64_t a_lo = make_smem_desc(base + TILE_BYTES);
-                        const uint64_t b_hi = make_smem_desc(base + 2 * TILE_BYTES);
+                        const uint64_t a_hi = ep.a_mn ? make_smem_desc_mn(base) : make_smem_desc(base);
+                        const uint64_t a_lo = ep.a_mn ? make_smem_desc_mn(base + TILE_BYTES) : make_smem_desc(base + TILE_BYTES);
+                        const uint64_t b_hi = ep.b_mn ? make_smem_desc_mn(base + 2 * TILE_BYTES) : make_smem_desc(base + 2 * TILE_BYTES);
+                        // per k-step of 8: 32 bytes along a K-major row, 8 rows of 128 bytes in an MN-major tile
+                        const uint64_t step_a = ep.a_mn ? (8 * 128) >> 4 : (8 * 4) >> 4, step_b = ep.b_mn ? (8 * 128) >> 4 : (8 * 4) >> 4;
+                        const uint32_t id_big = idesc_tf32(2 * BN, ep.a_mn, ep.b_mn), id_small = idesc_tf32(BN, ep.a_mn, ep.b_mn);
 #pragma unroll
                         for (int k = 0; k < ((ep.dbg & 4) ? 0 : BK / 8); ++k) {
-                            const uint64_t adv = (uint64_t)((k * 8 * 4) >> 4);      // 32 bytes per k-step, in 16-byte units
                             const uint32_t acc = (i > i0 || k > 0) ? 1u : 0u;
                             // [big | small] (+)= A_hi [B_hi ; B_lo]^T, then small += A_lo B_hi^T
-                            tc_mma_tf32(d_big, a_hi + adv, b_hi + adv, idesc_tf32(2 * BN), acc);
-                            tc_mma_tf32(d_small, a_lo + adv, b_hi + adv, idesc_tf32(BN), 1u);
+                            tc_mma_tf32(d_big, a_hi + k * step_a, b_hi + k * step_b, id_big, acc);
+                            tc_mma_tf32(d_small, a_lo + k * step_a, b_hi + k * step_b, id_small, 1u);
                         }
                         // the stage is free once these MMAs have read it -- in cluster mode the peer must know too
                         if (cl == 2) tc_commit_mc(&empty_bar[s], cl_mask);
@@ -324,8 +357,8 @@ gemm3x_tf32_kernel(const __grid_constant__ Maps maps, const Epi ep) {
         }
     } else {
         // ===== epilogue: warp w may touch TMEM lanes [32*(w%4), +32); two warps per quarter, 64 columns each =====
-        // Results leave through shared memory and TMA stores (32 x 32 fp32 tiles: row-major ones in the
-        // 128-byte swizzle, transposed ones dense); the TMA clips rows >= M and columns >= N.
+        // Results leave through shared memory and TMA stores (32 x 32 fp32 tiles in the 128-byte swizzle);
+        // the TMA clips rows >= M and columns >= N.
         const int ew = warp - 2, q = warp & 3, half = ew >> 2;
         uint8_t* stg = stg_base + ew * STG_BYTES;
         const uint32_t stg_u32 = smem_u32(stg);
@@ -420,7 +453,6 @@ gemm3x_tf32_kernel(const __grid_constant__ Maps maps, const Epi ep) {
                     store_pending = true;
                 };
                 float4* t_row = reinterpret_cast<float4*>(stg + lane * 128);
-                float* t_col = reinterpret_cast<float*>(stg);
                 if (ep.out_c) {
                     stage_begin();
 #pragma unroll
@@ -440,15 +472,24 @@ gemm3x_tf32_kernel(const __grid_constant__ Maps maps, const Epi ep) {
                     for (int j = 0; j < 8; ++j) t_row[j ^ sw] = make_float4(lo_of(4 * j), lo_of(4 * j + 1), lo_of(4 * j + 2), lo_of(4 * j + 3));
                     stage_end(&maps.c_lo, col0, r0, false);
                 }
-                if (ep.out_t) {
-                    stage_begin();
+                if (ep.colsum && r0 < ep.M) {
+                    // column sums over this warp's 32 rows: a butterfly reduce-scatter that halves the columns a
+                    // lane keeps at every step, so that lane j ends with the sum of column col0 + j
+                    if (!row_ok) {
 #pragma unroll
-                    for (int j = 0; j < 32; ++j) t_col[j * 32 + lane] = hi_of(j);
-                    stage_end(&maps.t_hi, r0, col0, false);
-                    stage_begin();
+                        for (int j = 0; j < 32; ++j) vv[j] = 0.f;
+                    }
 #pragma unroll
-                    for (int j = 0; j < 32; ++j) t_col[j * 32 + lane] = lo_of(j);
-                    stage_end(&maps.t_lo, r0, col0, false);
+                    for (int o = 16; o > 0; o >>= 1) {
+                        const bool upper = (lane & o) != 0;
+#pragma unroll
+                        for (int j = 0; j < o; ++j) {
+                            const float send = upper ? vv[j] : vv[j + o];
+                            const float keep = upper ? vv[j + o] : vv[j];
+                            vv[j] = keep + __shfl_xor_sync(0xffffffffu, send, o);
+                        }
+                    }
+                    if (col0 + lane < ep.N) ep.colsum[(int64_t)(r0 >> 5) * ep.N + col0 + lane] = vv[0];
                 }
             }
         }
@@ -466,42 +507,41 @@ gemm3x_tf32_kernel(const __grid_constant__ Maps maps, const Epi ep) {
 }
 
 // ------------------------------------------------------------------------------------
-// split: dst = f(src) as hi/lo TF32 pairs, row-major [rows, ld_o] and/or transposed
-// [cols, ld_t]; f is the identity or the activation derivative applied to an upstream
-// gradient (relu': src * (y > 0), sigmoid': src * y * (1 - y)).
+// split: dst = f(src) as hi/lo TF32 pairs, row-major [rows, ld_o]; f is the identity or the
+// activation derivative applied to an upstream gradient (relu': src * (y > 0), sigmoid':
+// src * y * (1 - y)).  With colsum: the sums of dst over each 32-row block, colsum[(r / 32) * cols + c]
+// (the bias gradient's partial sums when dst is a gradient w.r.t. a pre-activation).
 // ------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) split_kernel(const float* __restrict__ src, int64_t lds, int rows, int cols,
                                                     const float* __restrict__ y, int64_t ldy, int dmode,
                                                     float* __restrict__ hi, float* __restrict__ lo, int64_t ld_o,
-                                                    float* __restrict__ thi, float* __restrict__ tlo, int64_t ld_t) {
+                                                    float* __restrict__ colsum) {
     pdl_enter();
-    __shared__ float s_hi[32][33], s_lo[32][33];
+    __shared__ float s_sum[8][33];
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;      // 32 x 8
     const int r0 = blockIdx.y * 32, c0 = blockIdx.x * 32;
+    float sum = 0.f;
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
         const int r = r0 + ty + 8 * i, c = c0 + tx;
-        float h = 0.f, l = 0.f;
         if (r < rows && c < cols) {
             float v = src[(int64_t)r * lds + c];
             if (dmode == ACT_RELU) v = y[(int64_t)r * ldy + c] > 0.f ? v : 0.f;
             else if (dmode == ACT_SIGMOID) { const float p = y[(int64_t)r * ldy + c]; v = v * p * (1.f - p); }
-            h = tf32_hi(v);
-            l = tf32_lo(v, h);
-            if (hi) { hi[(int64_t)r * ld_o + c] = h; lo[(int64_t)r * ld_o + c] = l; }
+            const float h = tf32_hi(v);
+            hi[(int64_t)r * ld_o + c] = h;
+            lo[(int64_t)r * ld_o + c] = tf32_lo(v, h);
+            sum += v;
         }
-        s_hi[ty + 8 * i][tx] = h;
-        s_lo[ty + 8 * i][tx] = l;
     }
-    if (!thi) return;
+    if (!colsum) return;                                          // kernel-uniform
+    s_sum[ty][tx] = sum;
     __syncthreads();
+    if (ty == 0 && c0 + tx < cols) {
+        float t = 0.f;
 #pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const int c = c0 + ty + 8 * i, r = r0 + tx;
-        if (r < rows && c < cols) {
-            thi[(int64_t)c * ld_t + r] = s_hi[tx][ty + 8 * i];
-            tlo[(int64_t)c * ld_t + r] = s_lo[tx][ty + 8 * i];
-        }
+        for (int i = 0; i < 8; ++i) t += s_sum[i][tx];
+        colsum[(int64_t)blockIdx.y * cols + c0 + tx] = t;
     }
 }
 
@@ -510,7 +550,6 @@ constexpr int MAX_LAYERS = 8;
 struct SplitJob {
     const float* src; int64_t lds; int rows, cols;
     float *hi, *lo; int64_t ld_o;
-    float *thi, *tlo; int64_t ld_t;
     int tiles_x, tile0;          // 32 x 32 tiles per row of tiles, first global tile of this job
     const float* grad;           // SGD fused in front of the split: src <- src - lr * grad (dense, row stride lds); or null
 };
@@ -524,7 +563,6 @@ struct SplitBatch {
 };
 __global__ void __launch_bounds__(256) split_batch_kernel(const __grid_constant__ SplitBatch sb) {
     pdl_enter();
-    __shared__ float s_hi[32][33], s_lo[32][33];
     if (sb.vec && (int)blockIdx.x >= sb.tiles) {
         const int64_t i = (int64_t)((int)blockIdx.x - sb.tiles) * 256 + threadIdx.x;
         if (i < sb.vec_n) sb.vec[i] = fmaf(-sb.lr, sb.vec_grad[i], sb.vec[i]);
@@ -540,55 +578,70 @@ __global__ void __launch_bounds__(256) split_batch_kernel(const __grid_constant_
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
         const int r = r0 + ty + 8 * i, c = c0 + tx;
-        float h = 0.f, l = 0.f;
         if (r < jb.rows && c < jb.cols) {
             float v = jb.src[(int64_t)r * jb.lds + c];
             if (jb.grad) {
                 v = fmaf(-sb.lr, jb.grad[(int64_t)r * jb.lds + c], v);
                 const_cast<float*>(jb.src)[(int64_t)r * jb.lds + c] = v;
             }
-            h = tf32_hi(v);
-            l = tf32_lo(v, h);
+            const float h = tf32_hi(v);
             jb.hi[(int64_t)r * jb.ld_o + c] = h;
-            jb.lo[(int64_t)r * jb.ld_o + c] = l;
-        }
-        s_hi[ty + 8 * i][tx] = h;
-        s_lo[ty + 8 * i][tx] = l;
-    }
-    __syncthreads();
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const int c = c0 + ty + 8 * i, r = r0 + tx;
-        if (r < jb.rows && c < jb.cols) {
-            jb.thi[(int64_t)c * jb.ld_t + r] = s_hi[tx][ty + 8 * i];
-            jb.tlo[(int64_t)c * jb.ld_t + r] = s_lo[tx][ty + 8 * i];
+            jb.lo[(int64_t)r * jb.ld_o + c] = tf32_lo(v, h);
         }
     }
 }
 
-// dW [N, K] and db [N] of every layer out of the padded split-K accumulators, ONE launch
+// dW [N, K] of every layer out of the padded split-K accumulators and db [N] out of the partial column
+// sums [parts, N] of dZ, ONE launch.  The first db_blocks blocks reduce 32 bias columns each (8 row groups of
+// threads, then the 8 group sums in order: a fixed summation order, the same result on every run); the
+// others copy dW.
 struct UnpackJob {
     const float* acc; int64_t ldp; int N, K;
     float *dW, *db;
-    int64_t e0;                  // first global element of this job
+    const float* dbp;            // [parts, N] partial column sums of dZ
+    int64_t e0;                  // first global dW element of this job
+    int c0;                      // first global bias column of this job
 };
 struct UnpackBatch {
     UnpackJob job[MAX_LAYERS];
     int n;
-    int64_t total;
+    int64_t total;               // dW elements of all jobs
+    int columns, parts;          // bias columns of all jobs; partial sums per column
+    int db_blocks;
 };
 __global__ void __launch_bounds__(256) unpack_batch_kernel(const __grid_constant__ UnpackBatch ub) {
     pdl_enter();
-    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < ub.total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+    if ((int)blockIdx.x < ub.db_blocks) {
+        __shared__ float s_sum[8][33];
+        const int gc = blockIdx.x * 32 + tx;
+        int j = 0;
+#pragma unroll 1
+        while (j + 1 < ub.n && gc >= ub.job[j + 1].c0) ++j;
+        const UnpackJob& jb = ub.job[j];
+        const int c = gc - jb.c0;
+        float t = 0.f;
+        if (gc < ub.columns)
+            for (int p = ty; p < ub.parts; p += 8) t += jb.dbp[(int64_t)p * jb.N + c];
+        s_sum[ty][tx] = t;
+        __syncthreads();
+        if (ty == 0 && gc < ub.columns) {
+            t = 0.f;
+#pragma unroll
+            for (int i = 0; i < 8; ++i) t += s_sum[i][tx];
+            jb.db[c] = t;
+        }
+        return;
+    }
+    const int64_t stride = (int64_t)(gridDim.x - ub.db_blocks) * blockDim.x;
+    for (int64_t i = (blockIdx.x - ub.db_blocks) * (int64_t)blockDim.x + threadIdx.x; i < ub.total; i += stride) {
         int j = 0;
 #pragma unroll 1
         while (j + 1 < ub.n && i >= ub.job[j + 1].e0) ++j;
         const UnpackJob& jb = ub.job[j];
         const int64_t e = i - jb.e0;
-        const int n = (int)(e / (jb.K + 1)), k = (int)(e - (int64_t)n * (jb.K + 1));
-        const float v = jb.acc[(int64_t)n * jb.ldp + k];
-        if (k < jb.K) jb.dW[(int64_t)n * jb.K + k] = v;
-        else jb.db[n] = v;
+        const int n = (int)(e / jb.K), k = (int)(e - (int64_t)n * jb.K);
+        jb.dW[(int64_t)n * jb.K + k] = jb.acc[(int64_t)n * jb.ldp + k];
     }
 }
 
@@ -641,21 +694,22 @@ __global__ void __launch_bounds__(256) narrow_fwd_kernel(const float* __restrict
     }
 }
 
-// g[r] = dy[r] * act'(y[r]);  dwp[k] += sum_r g[r] x[r, k],  dwp[K] += sum_r g[r]  (weight / bias gradient, split
-// over row chunks, atomics into the zeroed accumulator);  dZ[r, k] = g[r] W[k] * (x[r, k] > 0) as hi/lo split,
-// row-major and transposed (the operands of the layer below), or plain FP32 into dx when this is layer 0.
+// g[r] = dy[r] * act'(y[r]);  dwp[k] += sum_r g[r] x[r, k] (weight gradient, split over row chunks, atomics into the
+// zeroed accumulator);  dbp[r / 32] = sum of g over each 32-row block (bias gradient partials);  dZ[r, k] =
+// g[r] W[k] * (x[r, k] > 0) as hi/lo split (the operands of the layer below) with its column sums per 32 rows in
+// colsum[(r / 32) * K + k], or plain FP32 into dx when this is layer 0.
 // Block = 32 columns x NARROW_ROWS rows (32 x 32 sub-tiles), 32 x 8 threads.
 constexpr int NARROW_ROWS = 64;     // 8 x 128 CTAs at batch 8192, K = 256 (32 x 128 rows left half the SMs idle: ncu 18 us)
+constexpr int NARROW_SUBS = NARROW_ROWS / 32;
 __global__ void __launch_bounds__(256) narrow_bwd_kernel(const float* __restrict__ dy, int64_t lddy,
                                                          const float* __restrict__ y, int64_t ldy, int act,
                                                          const float* __restrict__ x_hi, const float* __restrict__ x_lo,
                                                          int64_t ldx, int rows, int K, const float* __restrict__ W,
                                                          int relu_mask, float* __restrict__ g_hi, float* __restrict__ g_lo,
-                                                         int64_t ld_o, float* __restrict__ gt_hi, float* __restrict__ gt_lo,
-                                                         int64_t ld_t, float* __restrict__ dx, int64_t lddx,
-                                                         float* __restrict__ dwp) {
+                                                         int64_t ld_o, float* __restrict__ colsum, float* __restrict__ dx,
+                                                         int64_t lddx, float* __restrict__ dwp, float* __restrict__ dbp) {
     pdl_enter();
-    __shared__ float s_hi[32][33], s_lo[32][33], s_g[NARROW_ROWS];
+    __shared__ float s_sum[1 + NARROW_SUBS][8][33], s_g[NARROW_ROWS];
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
     const int c0 = blockIdx.x * 32, r0 = blockIdx.y * NARROW_ROWS;
     if (threadIdx.x < NARROW_ROWS) {
@@ -666,14 +720,12 @@ __global__ void __launch_bounds__(256) narrow_bwd_kernel(const float* __restrict
     const int c = c0 + tx;
     const float w = c < K ? __ldg(W + c) : 0.f;
     float wsum = 0.f;
-#pragma unroll 1
-    for (int sub = 0; sub < NARROW_ROWS / 32; ++sub) {
-        const int rb = r0 + sub * 32;
-        if (rb >= rows) break;                                    // block-uniform
+#pragma unroll
+    for (int sub = 0; sub < NARROW_SUBS; ++sub) {
+        float dsum = 0.f;
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
             const int rl = sub * 32 + ty + 8 * i, r = r0 + rl;
-            float h = 0.f, l = 0.f;
             if (r < rows && c < K) {
                 const float g = s_g[rl];
                 const float xh = x_hi[(int64_t)r * ldx + c];
@@ -682,50 +734,35 @@ __global__ void __launch_bounds__(256) narrow_bwd_kernel(const float* __restrict
                 if (relu_mask) v = xh > 0.f ? v : 0.f;
                 if (dx) dx[(int64_t)r * lddx + c] = v;
                 if (g_hi) {
-                    h = tf32_hi(v);
-                    l = tf32_lo(v, h);
+                    const float h = tf32_hi(v);
                     g_hi[(int64_t)r * ld_o + c] = h;
-                    g_lo[(int64_t)r * ld_o + c] = l;
+                    g_lo[(int64_t)r * ld_o + c] = tf32_lo(v, h);
                 }
+                dsum += v;
             }
-            s_hi[ty + 8 * i][tx] = h;
-            s_lo[ty + 8 * i][tx] = l;
         }
-        if (gt_hi) {                                              // kernel-uniform
-            __syncthreads();
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                const int cc = c0 + ty + 8 * i, r = rb + tx;
-                if (r < rows && cc < K) {
-                    gt_hi[(int64_t)cc * ld_t + r] = s_hi[tx][ty + 8 * i];
-                    gt_lo[(int64_t)cc * ld_t + r] = s_lo[tx][ty + 8 * i];
-                }
-            }
-            __syncthreads();
-        }
+        s_sum[1 + sub][ty][tx] = dsum;
     }
-    // column sums over the block's rows: reduce the 8 row groups through shared memory
+    // column sums over the 8 row groups of threads, in order: warp 0 the weight gradient, warp 1 + sub the dZ
+    // partials of sub-tile sub; warp 1 + NARROW_SUBS the bias gradient partials (one column block does that)
+    s_sum[0][ty][tx] = wsum;
     __syncthreads();
-    s_hi[ty][tx] = wsum;
-    __syncthreads();
-    if (ty == 0 && c < K) {
+    if (ty <= NARROW_SUBS && c < K) {
         float t = 0.f;
 #pragma unroll
-        for (int i = 0; i < 8; ++i) t += s_hi[i][tx];
-        atomicAdd(dwp + c, t);
+        for (int i = 0; i < 8; ++i) t += s_sum[ty][i][tx];
+        if (ty == 0) atomicAdd(dwp + c, t);
+        else if (colsum && r0 + (ty - 1) * 32 < rows) colsum[(int64_t)(r0 / 32 + ty - 1) * K + c] = t;
     }
-    if (blockIdx.x == 0 && ty == 1) {                             // bias gradient: one column block adds sum_r g[r]
-        float t = 0.f;
+    if (blockIdx.x == 0 && ty == 1 + NARROW_SUBS) {
 #pragma unroll
-        for (int r = 0; r < NARROW_ROWS; r += 32) t += s_g[tx + r];
+        for (int sub = 0; sub < NARROW_SUBS; ++sub) {
+            float t = s_g[sub * 32 + tx];
 #pragma unroll
-        for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
-        if (tx == 0) atomicAdd(dwp + K, t);
+            for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
+            if (tx == 0 && r0 + sub * 32 < rows) dbp[r0 / 32 + sub] = t;
+        }
     }
-}
-
-__global__ void fill_kernel(float* p, int64_t n, float v) {
-    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) p[i] = v;
 }
 
 // ------------------------------------------------------------------------------------
@@ -747,9 +784,9 @@ EncodeTiledFn get_encode() {
     return fn;
 }
 
-// [rows, inner] fp32, row stride ld elements (multiple of 4); box = box_inner x box_rows; out-of-range
-// box elements read as zero and are not written
-// operand pair: hi at `hi`, lo at `lo` (same shape and row stride, lo behind hi) as one {inner, rows, 2} tensor;
+// Tensors are [rows, inner] fp32 with a row stride of ld elements (multiple of 4); out-of-range box elements read as
+// zero and are not written.
+// K-major operand pair: hi at `hi`, lo at `lo` (same shape and row stride, lo behind hi) as one {inner, rows, 2} tensor;
 // box = BK x box_rows x 2, swizzle width = one BK row
 int make_pair_map(CUtensorMap* m, const float* hi, const float* lo, int64_t inner, int64_t rows, int64_t ld, int box_rows,
                   int box_depth = 2) {
@@ -779,7 +816,40 @@ int make_pair_map(CUtensorMap* m, const float* hi, const float* lo, int64_t inne
     return CDLRM_OK;
 }
 
-int make_map(CUtensorMap* m, const float* base, int64_t inner, int64_t rows, int64_t ld, int box_rows, bool swizzle, int box_inner = 32) {
+// MN-major operand pair: row-major [rows = K, ld] with the MN index contiguous, hi at `hi`, lo behind it, as one
+// 4-D tensor {32, K, MN / 32, 2} (strides ld, 32 elements, lo - hi) whose box {32, BK, 4, 2} is a 128-wide tile
+// of BK rows in four 32-wide column blocks, in the 128-byte swizzle with 32-byte atoms (make_smem_desc_mn).  The row stride must cover the 32-wide column
+// blocks (ld >= 32 * ceil(mn / 32)): elements mn .. of the last block are the row's padding, and only reach
+// results at rows / columns >= mn, which the stores clip.
+int make_mn_map(CUtensorMap* m, const float* hi, const float* lo, int64_t mn, int64_t rows, int64_t ld) {
+    EncodeTiledFn enc = get_encode();
+    if (!enc) {
+        cdlrm_set_error("cuTensorMapEncodeTiled is not available from the driver");
+        return CDLRM_ERR_CUDA;
+    }
+    const int64_t gap = (const char*)lo - (const char*)hi, blocks = (mn + 31) / 32;
+    if (((uintptr_t)hi & 15) || (ld & 3) || mn <= 0 || rows <= 0 || ld < 32 * blocks || gap < rows * ld * 4 || (gap & 15)) {
+        cdlrm_set_error("MN-major operand pair must be 16-byte aligned, row stride a multiple of 4 covering whole 32-wide "
+                        "column blocks, lo behind hi (hi %p lo %p mn %lld ld %lld)", (const void*)hi, (const void*)lo,
+                        (long long)mn, (long long)ld);
+        return CDLRM_ERR_ARG;
+    }
+    cuuint64_t dims[4] = {32, (cuuint64_t)rows, (cuuint64_t)blocks, 2};
+    cuuint64_t strides[3] = {(cuuint64_t)ld * 4, 128, (cuuint64_t)gap};
+    cuuint32_t box[4] = {32, (cuuint32_t)BK, (cuuint32_t)(BM / 32), 2};
+    cuuint32_t estr[4] = {1, 1, 1, 1};
+    CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, (void*)hi, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                     CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) {
+        cdlrm_set_error("cuTensorMapEncodeTiled (MN-major pair) failed (%d): mn %lld rows %lld ld %lld gap %lld", (int)r,
+                        (long long)mn, (long long)rows, (long long)ld, (long long)gap);
+        return CDLRM_ERR_CUDA;
+    }
+    return CDLRM_OK;
+}
+
+// result map: box 32 x 32, 128-byte swizzle
+int make_map(CUtensorMap* m, const float* base, int64_t inner, int64_t rows, int64_t ld) {
     EncodeTiledFn enc = get_encode();
     if (!enc) {
         cdlrm_set_error("cuTensorMapEncodeTiled is not available from the driver");
@@ -791,11 +861,10 @@ int make_map(CUtensorMap* m, const float* base, int64_t inner, int64_t rows, int
     }
     cuuint64_t dims[2] = {(cuuint64_t)inner, (cuuint64_t)rows};
     cuuint64_t strides[1] = {(cuuint64_t)ld * 4};
-    cuuint32_t box[2] = {(cuuint32_t)box_inner, (cuuint32_t)box_rows};
+    cuuint32_t box[2] = {32, 32};
     cuuint32_t estr[2] = {1, 1};
     CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     !swizzle ? CU_TENSOR_MAP_SWIZZLE_NONE : (box_inner == 32 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B),
-                     CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) {
         cdlrm_set_error("cuTensorMapEncodeTiled failed (%d): inner %lld rows %lld ld %lld", (int)r, (long long)inner, (long long)rows, (long long)ld);
@@ -812,9 +881,6 @@ struct Out {
     float* c_hi = nullptr;       // hi/lo split [M, N] row-major
     float* c_lo = nullptr;
     int64_t ld_split = 0;
-    float* t_hi = nullptr;       // hi/lo split transposed [N, M]
-    float* t_lo = nullptr;
-    int64_t ld_t = 0;
 };
 
 int g_narrow = 1;    // 1: a last layer with one output column runs on the SIMT narrow kernels; cdlrm_mlp_set_option(2, .)
@@ -829,6 +895,7 @@ int g_num_sms = 0;
 int g_dbg = 0;
 long long* g_trace = nullptr;
 
+// A and B as hi/lo pairs with row stride lda / ldb: K-major unless ep.a_mn / ep.b_mn
 int launch_gemm(const float* a_hi, const float* a_lo, int64_t lda, const float* b_hi, const float* b_lo, int64_t ldb,
                 Epi ep, const Out& o, int splits, cudaStream_t s) {
     if (!g_num_sms) {
@@ -843,23 +910,19 @@ int launch_gemm(const float* a_hi, const float* a_lo, int64_t lda, const float* 
     Maps mp;
     memset(&mp, 0, sizeof(mp));
     int rc;
-    if ((rc = make_pair_map(&mp.a, a_hi, a_lo, ep.K, ep.M, lda, BM))) return rc;
-    if ((rc = make_pair_map(&mp.b, b_hi, b_lo, ep.K, ep.N, ldb, BN))) return rc;
+    static_assert(BM == BN && BK == 32, "an MN-major tile is one box of four 32-wide column blocks of BK rows");
+    if ((rc = ep.a_mn ? make_mn_map(&mp.a, a_hi, a_lo, ep.M, ep.K, lda) : make_pair_map(&mp.a, a_hi, a_lo, ep.K, ep.M, lda, BM))) return rc;
+    if ((rc = ep.b_mn ? make_mn_map(&mp.b, b_hi, b_lo, ep.N, ep.K, ldb) : make_pair_map(&mp.b, b_hi, b_lo, ep.K, ep.N, ldb, BN))) return rc;
     ep.out_c = o.c ? (o.reduce ? 2 : 1) : 0;
     ep.out_split = o.c_hi ? 1 : 0;
-    ep.out_t = o.t_hi ? 1 : 0;
     if (ep.out_c && ep.out_split) {
         cdlrm_set_error("a GEMM writes either the fp32 result or its hi/lo split row-major, not both");
         return CDLRM_ERR_ARG;
     }
-    if (o.c && (rc = make_map(&mp.c, o.c, ep.N, ep.M, o.ldc, 32, true))) return rc;
+    if (o.c && (rc = make_map(&mp.c, o.c, ep.N, ep.M, o.ldc))) return rc;
     if (o.c_hi) {
-        if ((rc = make_map(&mp.c_hi, o.c_hi, ep.N, ep.M, o.ld_split, 32, true))) return rc;
-        if ((rc = make_map(&mp.c_lo, o.c_lo, ep.N, ep.M, o.ld_split, 32, true))) return rc;
-    }
-    if (o.t_hi) {
-        if ((rc = make_map(&mp.t_hi, o.t_hi, ep.M, ep.N, o.ld_t, 32, false))) return rc;
-        if ((rc = make_map(&mp.t_lo, o.t_lo, ep.M, ep.N, o.ld_t, 32, false))) return rc;
+        if ((rc = make_map(&mp.c_hi, o.c_hi, ep.N, ep.M, o.ld_split))) return rc;
+        if ((rc = make_map(&mp.c_lo, o.c_lo, ep.N, ep.M, o.ld_split))) return rc;
     }
     const int num_kb = (ep.K + BK - 1) / BK;
     if (splits < 1) splits = 1;
@@ -874,8 +937,9 @@ int launch_gemm(const float* a_hi, const float* a_lo, int64_t lda, const float* 
     ep.dbg = g_dbg;
     ep.trace = g_trace;
     ep.seg_kb = g_seg_kb > 0 ? g_seg_kb * (32 / BK) : num_kb;      // the option counts k-blocks of 32
-    // optional: CTA pairs along M share the B tile of every k-block (half each, multicast): 25 % less L2 -> SM traffic
-    ep.cluster = (g_cluster == 2 && tiles_m % 2 == 0 && g_num_sms >= 2) ? 2 : 1;
+    // optional: CTA pairs along M share the B tile of every k-block (half each, multicast): 25 % less L2 -> SM traffic.
+    // K-major B only (the half-tile map is K-major).
+    ep.cluster = (g_cluster == 2 && !ep.b_mn && tiles_m % 2 == 0 && g_num_sms >= 2) ? 2 : 1;
     int grid;
     if (ep.cluster == 2) {
         if ((rc = make_pair_map(&mp.b_half, b_hi, b_lo, ep.K, ep.N, ldb, BN / 2, 1))) return rc;
@@ -894,41 +958,49 @@ int launch_gemm(const float* a_hi, const float* a_lo, int64_t lda, const float* 
 }
 
 int launch_split(const float* src, int64_t lds, int rows, int cols, const float* y, int64_t ldy, int dmode, float* hi,
-                 float* lo, int64_t ld_o, float* thi, float* tlo, int64_t ld_t, cudaStream_t s) {
+                 float* lo, int64_t ld_o, float* colsum, cudaStream_t s) {
     if (rows <= 0 || cols <= 0) return CDLRM_OK;
     dim3 grid((cols + 31) / 32, (rows + 31) / 32);
-    LAUNCH_PDL(K_MLP_SPLIT, s, split_kernel, grid, 256, 0, src, lds, rows, cols, y, ldy, dmode, hi, lo, ld_o, thi, tlo, ld_t);
+    LAUNCH_PDL(K_MLP_SPLIT, s, split_kernel, grid, 256, 0, src, lds, rows, cols, y, ldy, dmode, hi, lo, ld_o, colsum);
     CU_CHECK(cudaGetLastError());
     return CDLRM_OK;
 }
 
 inline int64_t pad4(int64_t v) { return (v + 3) & ~(int64_t)3; }
+// row stride of the hi/lo splits of weights, activations and gradients: whole 32-wide blocks, so that every
+// MN-major box stays inside its row (make_mn_map)
+inline int64_t pad32(int64_t v) { return (v + 31) & ~(int64_t)31; }
+inline int64_t parts32(int64_t rows) { return (rows + 31) / 32; }
 inline int64_t align256(int64_t v) { return (v + 255) & ~(int64_t)255; }
 
 }  // namespace
 
 // One MLP (bottom or top): dims[0..L], batch capacity, the layer that ends in a sigmoid.
 // Workspace carve-up (all fp32, every region 256-byte aligned):
-//   per layer l:  w_hi/w_lo [N_l, pad4(K_l)]   wt_hi/wt_lo [K_l, pad4(N_l)]
+//   per layer l:  w_hi/w_lo [N_l, pad32(K_l)]
 //   per level i = 0..L (activation entering layer i; level L is the output):
-//        x_hi/x_lo [cap, pad4(D_i)]   xt_hi/xt_lo [D_i + 1, pad4(cap)]  (last row = ones: bias gradient)
-//        g_hi/g_lo [cap, pad4(D_i)]   gt_hi/gt_lo [D_i, pad4(cap)]      (gradient w.r.t. the pre-activation)
+//        x_hi/x_lo [cap, pad32(D_i)]   (i < L)
+//        g_hi/g_lo [cap, pad32(D_i)]   (i > 0, gradient w.r.t. the pre-activation)
 //   y_out [cap, pad4(D_L)]  fp32 output of the last layer (activation derivative input)
+//   per layer l:  dwp [N_l, pad4(K_l)]  split-K accumulator of dW (back to back: one memset)
+//   per layer l:  dbp [ceil(cap / 32), N_l]  column sums of g_{l+1} per 32 rows (db partials)
+// The weight-gradient GEMM reads g and x MN-major and the data-gradient GEMM reads w MN-major: no
+// transposed copy of any of them exists.
 struct cdlrm_mlp {
     int device = 0;
     int L = 0;
     int cap = 0;
     int sigmoid_layer = -1;
     std::vector<int> D;
-    std::vector<float*> w_hi, w_lo, wt_hi, wt_lo;
-    std::vector<float*> x_hi, x_lo, xt_hi, xt_lo, g_hi, g_lo, gt_hi, gt_lo;
-    std::vector<float*> dwp;     // per layer: split-K accumulator [N_l, pad4(K_l + 1)]
+    std::vector<float*> w_hi, w_lo;
+    std::vector<float*> x_hi, x_lo, g_hi, g_lo;
+    std::vector<float*> dwp;     // per layer: split-K accumulator [N_l, pad4(K_l)]
+    std::vector<float*> dbp;     // per layer: partial bias gradients [ceil(cap / 32), N_l]
     float* y_out = nullptr;
     int64_t dwp_bytes = 0;       // the dwp regions are carved back to back
     int last_batch = 0;
     bool last_narrow = false;    // the last forward ran its final layer on the narrow kernels
     const float* last_W = nullptr;   // FP32 weights of that layer (the narrow backward reads them)
-    bool ones_set = false;
     bool w_presplit = false;     // cdlrm_mlp_sgd_split left the splits of the CURRENT weights behind: the next forward skips its own
     int num_sms = 148;
     // weight-gradient GEMMs on a stream of their own beside the data-gradient chain (cdlrm_mlp_backward)
@@ -946,31 +1018,26 @@ static int64_t mlp_carve(cdlrm_mlp* m, char* base) {
         return p;
     };
     const int L = m->L;
-    const int64_t cap = m->cap, capp = pad4(m->cap);
-    m->w_hi.assign(L, nullptr); m->w_lo.assign(L, nullptr); m->wt_hi.assign(L, nullptr); m->wt_lo.assign(L, nullptr);
+    const int64_t cap = m->cap;
+    m->w_hi.assign(L, nullptr); m->w_lo.assign(L, nullptr);
     for (int l = 0; l < L; ++l) {
         const int64_t K = m->D[l], N = m->D[l + 1];
-        m->w_hi[l] = take(N * pad4(K)); m->w_lo[l] = take(N * pad4(K));
-        m->wt_hi[l] = take(K * pad4(N)); m->wt_lo[l] = take(K * pad4(N));
+        m->w_hi[l] = take(N * pad32(K)); m->w_lo[l] = take(N * pad32(K));
     }
-    m->x_hi.assign(L + 1, nullptr); m->x_lo.assign(L + 1, nullptr); m->xt_hi.assign(L + 1, nullptr); m->xt_lo.assign(L + 1, nullptr);
-    m->g_hi.assign(L + 1, nullptr); m->g_lo.assign(L + 1, nullptr); m->gt_hi.assign(L + 1, nullptr); m->gt_lo.assign(L + 1, nullptr);
+    m->x_hi.assign(L + 1, nullptr); m->x_lo.assign(L + 1, nullptr);
+    m->g_hi.assign(L + 1, nullptr); m->g_lo.assign(L + 1, nullptr);
     for (int i = 0; i <= L; ++i) {
         const int64_t Di = m->D[i];
-        if (i < L) {
-            m->x_hi[i] = take(cap * pad4(Di)); m->x_lo[i] = take(cap * pad4(Di));
-            m->xt_hi[i] = take((Di + 1) * capp); m->xt_lo[i] = take((Di + 1) * capp);
-        }
-        if (i > 0) {
-            m->g_hi[i] = take(cap * pad4(Di)); m->g_lo[i] = take(cap * pad4(Di));
-            m->gt_hi[i] = take(Di * capp); m->gt_lo[i] = take(Di * capp);
-        }
+        if (i < L) { m->x_hi[i] = take(cap * pad32(Di)); m->x_lo[i] = take(cap * pad32(Di)); }
+        if (i > 0) { m->g_hi[i] = take(cap * pad32(Di)); m->g_lo[i] = take(cap * pad32(Di)); }
     }
     m->y_out = take(cap * pad4(m->D[L]));
     m->dwp.assign(L, nullptr);
     const int64_t dwp0 = off;
-    for (int l = 0; l < L; ++l) m->dwp[l] = take((int64_t)m->D[l + 1] * pad4(m->D[l] + 1));
+    for (int l = 0; l < L; ++l) m->dwp[l] = take((int64_t)m->D[l + 1] * pad4(m->D[l]));
     m->dwp_bytes = off - dwp0;
+    m->dbp.assign(L, nullptr);
+    for (int l = 0; l < L; ++l) m->dbp[l] = take(parts32(cap) * m->D[l + 1]);
     return off;
 }
 
@@ -1084,8 +1151,7 @@ extern "C" int cdlrm_mlp_join(cdlrm_mlp* m, cdlrm_stream stream) {
     return CDLRM_OK;
 }
 
-// SGD step of the weight matrices of up to two MLPs fused with the hi/lo split (row-major and transposed) of the
-// UPDATED weights, plus plain SGD on one extra vector (the biases): ONE launch instead of the optimizer's axpy and one
+// SGD step of the weight matrices of up to two MLPs fused with the hi/lo split of the UPDATED weights, plus plain SGD on one extra vector (the biases): ONE launch instead of the optimizer's axpy and one
 // split launch at the head of each forward -- which sat on the critical path of the step (before the bottom MLP's
 // first GEMM, and between the interaction and the top MLP).
 extern "C" int cdlrm_mlp_sgd_split(int n_mlps, cdlrm_mlp* const* mlps, float* const* h_W, const float* const* h_dW, float lr,
@@ -1102,8 +1168,7 @@ extern "C" int cdlrm_mlp_sgd_split(int n_mlps, cdlrm_mlp* const* mlps, float* co
             const int K = m->D[l], N = m->D[l + 1];
             SplitJob& jb = sb.job[j];
             jb.src = h_W[j]; jb.grad = h_dW[j]; jb.lds = K; jb.rows = N; jb.cols = K;
-            jb.hi = m->w_hi[l]; jb.lo = m->w_lo[l]; jb.ld_o = pad4(K);
-            jb.thi = m->wt_hi[l]; jb.tlo = m->wt_lo[l]; jb.ld_t = pad4(N);
+            jb.hi = m->w_hi[l]; jb.lo = m->w_lo[l]; jb.ld_o = pad32(K);
             jb.tiles_x = (K + 31) / 32; jb.tile0 = tiles;
             tiles += jb.tiles_x * ((N + 31) / 32);
         }
@@ -1135,22 +1200,13 @@ extern "C" int cdlrm_mlp_forward(cdlrm_mlp* m, const float* x, int64_t ldx, int3
     cudaStream_t s = (cudaStream_t)stream;
     CU_CHECK(cudaSetDevice(m->device));
     const int L = m->L;
-    const int64_t capp = pad4(m->cap);
     int rc;
-    if (m->pending_join) {      // weight-gradient GEMMs of the last backward still read the transposed activations
+    if (m->pending_join) {      // weight-gradient GEMMs of the last backward still read the activations
         CU_CHECK(cudaStreamWaitEvent(s, m->ev_done, 0));
         m->pending_join = false;
     }
-    if (!m->ones_set) {     // the ones rows of the transposed activations (bias gradient); lo part = 0
-        for (int i = 0; i < L; ++i) {
-            LAUNCH(K_MLP_SPLIT, s, (fill_kernel<<<64, 256, 0, s>>>(m->xt_hi[i] + (int64_t)m->D[i] * capp, capp, 1.f)));
-            LAUNCH(K_MLP_SPLIT, s, (fill_kernel<<<64, 256, 0, s>>>(m->xt_lo[i] + (int64_t)m->D[i] * capp, capp, 0.f)));
-        }
-        CU_CHECK(cudaGetLastError());
-        m->ones_set = true;
-    }
-    // weights: W [N,K] -> hi/lo K-major and transposed (the dgrad operand), all layers in one launch -- unless the
-    // optimizer step that produced these weights already did it (cdlrm_mlp_sgd_split)
+    // weights: W [N,K] -> hi/lo (K-major for the forward, MN-major for the dgrad), all layers in one launch --
+    // unless the optimizer step that produced these weights already did it (cdlrm_mlp_sgd_split)
     if (m->w_presplit) {
         for (int l = 0; l < L; ++l) ARG_CHECK(h_W[l] && h_b[l]);
         m->w_presplit = false;
@@ -1162,8 +1218,7 @@ extern "C" int cdlrm_mlp_forward(cdlrm_mlp* m, const float* x, int64_t ldx, int3
             const int K = m->D[l], N = m->D[l + 1];
             SplitJob& jb = sb.job[l];
             jb.src = h_W[l]; jb.grad = nullptr; jb.lds = K; jb.rows = N; jb.cols = K;
-            jb.hi = m->w_hi[l]; jb.lo = m->w_lo[l]; jb.ld_o = pad4(K);
-            jb.thi = m->wt_hi[l]; jb.tlo = m->wt_lo[l]; jb.ld_t = pad4(N);
+            jb.hi = m->w_hi[l]; jb.lo = m->w_lo[l]; jb.ld_o = pad32(K);
             jb.tiles_x = (K + 31) / 32; jb.tile0 = tiles;
             tiles += jb.tiles_x * ((N + 31) / 32);
         }
@@ -1173,7 +1228,7 @@ extern "C" int cdlrm_mlp_forward(cdlrm_mlp* m, const float* x, int64_t ldx, int3
         CU_CHECK(cudaGetLastError());
     }
     // input
-    if ((rc = launch_split(x, ldx, batch, m->D[0], nullptr, 0, ACT_NONE, m->x_hi[0], m->x_lo[0], pad4(m->D[0]), m->xt_hi[0], m->xt_lo[0], capp, s))) return rc;
+    if ((rc = launch_split(x, ldx, batch, m->D[0], nullptr, 0, ACT_NONE, m->x_hi[0], m->x_lo[0], pad32(m->D[0]), nullptr, s))) return rc;
     for (int l = 0; l < L; ++l) {
         const int K = m->D[l], N = m->D[l + 1];
         Epi ep = {};
@@ -1182,13 +1237,12 @@ extern "C" int cdlrm_mlp_forward(cdlrm_mlp* m, const float* x, int64_t ldx, int3
         ep.bias = h_b[l];
         ep.act = (l == m->sigmoid_layer) ? ACT_SIGMOID : ((m->sigmoid_layer == -2 && l == L - 1) ? ACT_NONE : ACT_RELU);
         if (l + 1 < L) {
-            o.c_hi = m->x_hi[l + 1]; o.c_lo = m->x_lo[l + 1]; o.ld_split = pad4(N);
-            o.t_hi = m->xt_hi[l + 1]; o.t_lo = m->xt_lo[l + 1]; o.ld_t = capp;
+            o.c_hi = m->x_hi[l + 1]; o.c_lo = m->x_lo[l + 1]; o.ld_split = pad32(N);
         } else {
             o.c = m->y_out; o.ldc = pad4(N);
         }
         if (l == L - 1 && N == 1 && g_narrow) {      // narrow last layer: row-wise dot products, writes y_out and y
-            LAUNCH_PDL(K_MLP_SPLIT, s, narrow_fwd_kernel, (batch + 7) / 8, 256, 0, m->x_hi[l], m->x_lo[l], pad4(K), batch, K,
+            LAUNCH_PDL(K_MLP_SPLIT, s, narrow_fwd_kernel, (batch + 7) / 8, 256, 0, m->x_hi[l], m->x_lo[l], pad32(K), batch, K,
                        h_W[l], h_b[l], ep.act, m->y_out, pad4(N), y, ldy);
             CU_CHECK(cudaGetLastError());
             m->last_batch = batch;
@@ -1196,7 +1250,7 @@ extern "C" int cdlrm_mlp_forward(cdlrm_mlp* m, const float* x, int64_t ldx, int3
             m->last_W = h_W[l];
             return CDLRM_OK;
         }
-        if ((rc = launch_gemm(m->x_hi[l], m->x_lo[l], pad4(K), m->w_hi[l], m->w_lo[l], pad4(K), ep, o, 1, s))) return rc;
+        if ((rc = launch_gemm(m->x_hi[l], m->x_lo[l], pad32(K), m->w_hi[l], m->w_lo[l], pad32(K), ep, o, 1, s))) return rc;
     }
     CU_CHECK(cudaMemcpy2DAsync(y, ldy * 4, m->y_out, pad4(m->D[L]) * 4, (size_t)m->D[L] * 4, batch, cudaMemcpyDeviceToDevice, s));
     m->last_batch = batch;
@@ -1216,7 +1270,6 @@ extern "C" int cdlrm_mlp_backward(cdlrm_mlp* m, const float* dy, int64_t lddy, f
     cudaStream_t s = (cudaStream_t)stream;
     CU_CHECK(cudaSetDevice(m->device));
     const int L = m->L;
-    const int64_t capp = pad4(m->cap);
     int rc;
     if (m->pending_join) {      // a deferred join nobody asked for: the previous backward's dW must be complete
         CU_CHECK(cudaStreamWaitEvent(s, m->ev_done, 0));
@@ -1225,13 +1278,15 @@ extern "C" int cdlrm_mlp_backward(cdlrm_mlp* m, const float* dy, int64_t lddy, f
     // The weight-gradient GEMMs are leaves of the backward: they run on a stream of their own, each behind the
     // event that marks its dZ ready, so that their CTAs fill the SMs the data-gradient chain (the critical path)
     // leaves idle at its tile-count tails and launch gaps.  Legal inside a stream capture (fork / join by events).
+    // db_l = column sums of g_{l+1}: whatever writes g_{l+1} (this split, the narrow kernel or the data-gradient
+    // epilogue of layer l + 1) also writes its partial sums per 32 rows into dbp[l]; the unpack reduces them.
     const bool side = g_wgrad_side != 0 && m->s2 != nullptr;
     cudaStream_t sw = side ? m->s2 : s;
-    // gradient w.r.t. the last pre-activation: dy * act'(y), as hi/lo, row-major and transposed
+    // gradient w.r.t. the last pre-activation: dy * act'(y), as hi/lo
     const int last_act = (L - 1 == m->sigmoid_layer) ? ACT_SIGMOID : (m->sigmoid_layer == -2 ? ACT_NONE : ACT_RELU);
     const bool narrow = m->last_narrow;
-    if (!narrow && (rc = launch_split(dy, lddy, batch, m->D[L], m->y_out, pad4(m->D[L]), last_act, m->g_hi[L], m->g_lo[L], pad4(m->D[L]),
-                                      m->gt_hi[L], m->gt_lo[L], capp, s))) return rc;
+    if (!narrow && (rc = launch_split(dy, lddy, batch, m->D[L], m->y_out, pad4(m->D[L]), last_act, m->g_hi[L], m->g_lo[L], pad32(m->D[L]),
+                                      m->dbp[L - 1], s))) return rc;
     CU_CHECK(cudaMemsetAsync(m->dwp[0], 0, (size_t)m->dwp_bytes, s));      // every layer's split-K accumulator
     for (int l = L - 1; l >= 0; --l) {
         const int K = m->D[l], N = m->D[l + 1];
@@ -1242,58 +1297,70 @@ extern "C" int cdlrm_mlp_backward(cdlrm_mlp* m, const float* dy, int64_t lddy, f
             dim3 grid((K + 31) / 32, (batch + NARROW_ROWS - 1) / NARROW_ROWS);
             const bool below = l > 0;
             LAUNCH_PDL(K_MLP_SPLIT, s, narrow_bwd_kernel, grid, 256, 0, dy, lddy, m->y_out, pad4(N), last_act, m->x_hi[l],
-                       m->x_lo[l], pad4(K), batch, K, m->last_W, below ? 1 : 0, below ? m->g_hi[l] : nullptr,
-                       below ? m->g_lo[l] : nullptr, pad4(K), below ? m->gt_hi[l] : nullptr, below ? m->gt_lo[l] : nullptr, capp,
-                       below ? nullptr : dx, lddx, m->dwp[l]);
+                       m->x_lo[l], pad32(K), batch, K, m->last_W, below ? 1 : 0, below ? m->g_hi[l] : nullptr,
+                       below ? m->g_lo[l] : nullptr, pad32(K), below ? m->dbp[l - 1] : nullptr, below ? nullptr : dx, lddx,
+                       m->dwp[l], m->dbp[l]);
             CU_CHECK(cudaGetLastError());
             continue;
         }
-        // wgrad: [dW | db] = dZ^T [X^T ; 1]: split-K over the batch, TMA reduce-add into a zeroed
-        // padded accumulator, then unpacked into the dense dW / db the optimizer sees
+        // wgrad: dW = dZ^T X with both operands read MN-major out of the row-major dZ [B, N] and X [B, K]: split-K
+        // over the batch, TMA reduce-add into a zeroed padded accumulator, then unpacked into the dense dW the
+        // optimizer sees
         {
-            const int64_t ldp = pad4(K + 1);
             Epi ep = {};
             Out o;
-            ep.M = N; ep.N = K + 1; ep.K = batch;
-            o.c = m->dwp[l]; o.ldc = ldp; o.reduce = true;
+            ep.M = N; ep.N = K; ep.K = batch;
+            ep.a_mn = 1; ep.b_mn = 1;
+            o.c = m->dwp[l]; o.ldc = pad4(K); o.reduce = true;
             if (side) {         // dZ of this layer (and, the first time, the zeroed accumulators) are ready on s
                 CU_CHECK(cudaEventRecord(m->ev_g, s));
                 CU_CHECK(cudaStreamWaitEvent(sw, m->ev_g, 0));
             }
-            if ((rc = launch_gemm(m->gt_hi[l + 1], m->gt_lo[l + 1], capp, m->xt_hi[l], m->xt_lo[l], capp, ep, o, 0 /*auto split-K*/, sw))) return rc;
+            if ((rc = launch_gemm(m->g_hi[l + 1], m->g_lo[l + 1], pad32(N), m->x_hi[l], m->x_lo[l], pad32(K), ep, o, 0 /*auto split-K*/, sw))) return rc;
         }
-        // dgrad: dX = dZ W, then the ReLU mask of the layer below -> its dZ (split, both layouts)
+        // dgrad: dX = dZ W with W read MN-major, then the ReLU mask of the layer below -> its dZ (split) and the
+        // partial column sums of that dZ (the bias gradient of layer l - 1)
         if (l > 0) {
             Epi ep = {};
             Out o;
             ep.M = batch; ep.N = K; ep.K = N;
-            ep.mask = m->x_hi[l]; ep.ld_mask = pad4(K);     // x_l = relu(...) > 0  <=>  its hi part > 0
-            o.c_hi = m->g_hi[l]; o.c_lo = m->g_lo[l]; o.ld_split = pad4(K);
-            o.t_hi = m->gt_hi[l]; o.t_lo = m->gt_lo[l]; o.ld_t = capp;
-            if ((rc = launch_gemm(m->g_hi[l + 1], m->g_lo[l + 1], pad4(N), m->wt_hi[l], m->wt_lo[l], pad4(N), ep, o, 1, s))) return rc;
+            ep.b_mn = 1;
+            ep.mask = m->x_hi[l]; ep.ld_mask = pad32(K);    // x_l = relu(...) > 0  <=>  its hi part > 0
+            ep.colsum = m->dbp[l - 1];
+            o.c_hi = m->g_hi[l]; o.c_lo = m->g_lo[l]; o.ld_split = pad32(K);
+            if ((rc = launch_gemm(m->g_hi[l + 1], m->g_lo[l + 1], pad32(N), m->w_hi[l], m->w_lo[l], pad32(K), ep, o, 1, s))) return rc;
         } else if (dx) {
             Epi ep = {};
             Out o;
             ep.M = batch; ep.N = K; ep.K = N;
+            ep.b_mn = 1;
             o.c = dx; o.ldc = lddx;
-            if ((rc = launch_gemm(m->g_hi[l + 1], m->g_lo[l + 1], pad4(N), m->wt_hi[l], m->wt_lo[l], pad4(N), ep, o, 1, s))) return rc;
+            if ((rc = launch_gemm(m->g_hi[l + 1], m->g_lo[l + 1], pad32(N), m->w_hi[l], m->w_lo[l], pad32(K), ep, o, 1, s))) return rc;
         }
     }
     // the dense dW / db the optimizer sees, all layers in one launch
     {
         UnpackBatch ub;
         int64_t total = 0;
+        int columns = 0;
         for (int l = 0; l < L; ++l) {
             UnpackJob& jb = ub.job[l];
-            jb.acc = m->dwp[l]; jb.ldp = pad4(m->D[l] + 1); jb.N = m->D[l + 1]; jb.K = m->D[l];
-            jb.dW = h_dW[l]; jb.db = h_db[l]; jb.e0 = total;
-            total += (int64_t)jb.N * (jb.K + 1);
+            jb.acc = m->dwp[l]; jb.ldp = pad4(m->D[l]); jb.N = m->D[l + 1]; jb.K = m->D[l];
+            jb.dW = h_dW[l]; jb.db = h_db[l]; jb.dbp = m->dbp[l];
+            jb.e0 = total; jb.c0 = columns;
+            total += (int64_t)jb.N * jb.K;
+            columns += jb.N;
         }
         ub.n = L;
         ub.total = total;
+        ub.columns = columns;
+        ub.parts = (int)parts32(batch);
+        ub.db_blocks = (columns + 31) / 32;
         int blocks = (int)((total + 255) / 256);
         if (blocks > 1184) blocks = 1184;
-        // the unpack reads the split-K accumulators of the narrow layer (written on s) and of the GEMMs (on sw)
+        blocks += ub.db_blocks;
+        // the unpack reads the db partials and the narrow layer's accumulator (written on s) and the GEMMs'
+        // split-K accumulators (on sw)
         const bool deferred = side && m->defer_join;
         if (side) {
             if (deferred) {
