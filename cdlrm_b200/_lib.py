@@ -32,6 +32,7 @@ SIGNATURES = {
     "cdlrm_ctx_check": (C.c_int, [vp, vp, c_u32p]),
     "cdlrm_embed_fwd": (C.c_int, [vp, C.c_int, C.c_int, vp, C.c_int64, vp, C.c_int64, C.c_int32, C.c_int32,
                                   vp, C.c_int64, vp, C.c_int64, vp, vp, C.c_int64, vp]),
+    "cdlrm_embed_fwd_eval": (C.c_int, [vp, C.c_int, C.c_int, vp, C.c_int64, C.c_int32, vp, C.c_int64, vp]),
     "cdlrm_embed_bwd_plan_bytes": (C.c_int64, [C.c_int, C.c_int32]),
     "cdlrm_embed_bwd_plan": (C.c_int, [vp, C.c_int, C.c_int, vp, C.c_int64, C.c_int32, vp, vp]),
     "cdlrm_embed_bwd_sgd": (C.c_int, [vp, C.c_int, C.c_int, vp, C.c_int32, vp, C.c_int64, vp, C.c_int64,
@@ -117,7 +118,18 @@ SIGNATURES = {
     "cdlrm_rngdev_set_option": (C.c_int, [C.c_int, C.c_int64]),
     "cdlrm_exp_from_raw": (C.c_int, [vp, vp, C.c_int64, vp]),
     "cdlrm_plan_phase_b_dev": (C.c_int, [vp, vp, vp, C.c_int64, c_i64p, vp, vp, vp, vp, vp, vp, vp]),
+    "cdlrm_eval_create": (C.c_int, [C.POINTER(vp), C.c_int, C.c_int64]),
+    "cdlrm_eval_destroy": (C.c_int, [vp]),
+    "cdlrm_eval_reset": (C.c_int, [vp, vp]),
+    "cdlrm_eval_accumulate": (C.c_int, [vp, vp, C.c_int64, vp, C.c_int64, C.c_int32, vp]),
+    "cdlrm_eval_result": (C.c_int, [vp, vp, vp]),
 }
+
+
+class EvalStats(C.Structure):
+    """cdlrm_eval_stats (include/cdlrm_b200.h)."""
+    _fields_ = [("samples", C.c_int64), ("positives", C.c_int64), ("negatives", C.c_int64), ("correct", C.c_int64),
+                ("loss_sum", C.c_double), ("auc_2u", C.c_uint64), ("flags", C.c_uint32), ("reserved", C.c_uint32)]
 
 
 class CdlrmError(RuntimeError):

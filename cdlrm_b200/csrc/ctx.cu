@@ -260,7 +260,8 @@ static const char* const g_knames[K_COUNT] = {
     "embed_fwd", "embed_miss", "pool", "bwd_plan", "bwd_sgd", "bwd_sgd_multi", "interact_fwd", "interact_bwd",
     "plan_bitmap_set", "plan_compact", "plan_probe", "plan_surv", "plan_select", "plan_lists",
     "move_evict", "move_gather", "move_fill", "move_scatter", "agg_mark", "agg_or", "agg_collect",
-    "agg_pack", "agg_unpack", "misc", "rng_mt19937", "rng_exp", "mlp_gemm", "mlp_split", "null"};
+    "agg_pack", "agg_unpack", "misc", "rng_mt19937", "rng_exp", "mlp_gemm", "mlp_split", "embed_fwd_eval", "eval_metrics",
+    "null"};
 
 void cdlrm_prof_mark(int id, cudaStream_t s, int end) {
     if (!end) g_launches.fetch_add(1, std::memory_order_relaxed);

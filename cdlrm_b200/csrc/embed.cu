@@ -80,6 +80,46 @@ __device__ __forceinline__ int probe_line(const int64_t* __restrict__ tags, int6
     return way;
 }
 
+// Tag probe of one id: its cache slot num_sets * way + set, or -1 when it is not cached.  An id outside its table
+// raises the sticky flag 2 (IndexError in the reference, master.weight[missing], :176) and matches nothing.
+template <int WAYS>
+__device__ __forceinline__ int64_t probe_slot(const TableDesc& T, int64_t id, int ways, uint32_t* __restrict__ flags) {
+    if ((uint64_t)id >= (uint64_t)T.n_rows) {
+        atomicOr(flags, 2u);
+        return -1;
+    }
+    const int64_t s = set_index(id, T.num_sets);
+    const int way = probe_line<WAYS>(T.tags, s, id, ways);
+    return way < 0 ? -1 : T.num_sets * way + s;
+}
+
+// Source row of an un-cached id: its copy in the loser store of the installed window (ascending ids: bucket index,
+// then binary search; L may be null), else the master row (zero-copy PCIe).
+__device__ __forceinline__ const float* miss_row(const LoserDesc* __restrict__ L, const float* __restrict__ master,
+                                                 int64_t id, int dim) {
+    if (L) {
+        const int64_t n = L->n;
+        int64_t lo = 0, hi = n;                // first index with ids[idx] >= id
+        if (L->bucket) {                       // bucket index: the answer lies in [bucket[b], bucket[b + 1]]
+            const int64_t bk = id >> L->shift;
+            lo = __ldg(L->bucket + bk);
+            hi = __ldg(L->bucket + bk + 1);
+        }
+        while (lo < hi) {
+            const int64_t mid = (lo + hi) >> 1;
+            if (__ldg(L->ids + mid) < id) lo = mid + 1; else hi = mid;
+        }
+        if (lo < n && __ldg(L->ids + lo) == id) {
+            if (L->shard) {                    // sharded store: the row is in the HBM of rank lo / shard (NVLink)
+                const int64_t owner = lo / L->shard;
+                return L->peer[owner] + (lo - owner * L->shard) * dim;
+            }
+            return L->rows + lo * dim;         // local HBM
+        }
+    }
+    return master + id * dim;
+}
+
 template <int WAYS, int G, bool COPY>
 __global__ void __launch_bounds__(FWD_NT) fwd_fused_kernel(const TableDesc* __restrict__ tabs, int tb,
                                                             const int64_t* __restrict__ ids, int64_t ld_ids, int n_idx,
@@ -93,18 +133,13 @@ __global__ void __launch_bounds__(FWD_NT) fwd_fused_kernel(const TableDesc* __re
     const int w = blockIdx.x * (FWD_NT / 32) + (threadIdx.x >> 5);
     if (w >= words) return;
     const TableDesc& T = tabs[tb + t];
-    const int64_t S = T.num_sets;
     const int j0 = w * 32, j = j0 + lane;
     const bool valid = j < n_idx;
-    int64_t id = valid ? __ldg(ids + (int64_t)t * ld_ids + j) : 0;
-    if ((uint64_t)id >= (uint64_t)T.n_rows) {     // IndexError in the reference (master.weight[missing], :176)
-        atomicOr(flags, 2u);                      // sticky; K2 gives the position a zero row and slot -1
-        id = -1;                                  // matches no live tag that could be read as a hit of a real id
-    }
-    const int64_t s = set_index(id < 0 ? 0 : id, S);
-    const int way = id < 0 ? -1 : probe_line<WAYS>(T.tags, s, id, ways);
-    const bool miss = valid && way < 0;
-    const int32_t slot = (valid && way >= 0) ? (int32_t)(S * way + s) : -1;
+    const int64_t id = valid ? __ldg(ids + (int64_t)t * ld_ids + j) : 0;
+    // an id outside its table is a miss: K2 gives the position a zero row and slot -1
+    const int64_t sl = probe_slot<WAYS>(T, id, ways, flags);
+    const bool miss = valid && sl < 0;
+    const int32_t slot = valid ? (int32_t)sl : -1;
     if (valid) slots[(int64_t)t * ld_slots + j] = slot;
     const uint32_t mm = __ballot_sync(0xffffffffu, miss);
     if (lane == 0) missmap[(int64_t)t * words + w] = mm;
@@ -181,17 +216,7 @@ __global__ void __launch_bounds__(MISS_NT) fwd_miss_kernel(const TableDesc* __re
     const int64_t aux_base = T.num_sets * ways;
     const int cpr = dim / VEC;
     // loser store of the installed window: ascending ids + their master rows staged in HBM
-    const int64_t* __restrict__ l_ids = nullptr;
-    const float* __restrict__ l_rows = nullptr;
-    const LoserDesc* __restrict__ l_desc = nullptr;
-    int64_t l_n = 0, l_shard = 0;
-    const int32_t* __restrict__ l_bucket = nullptr;
-    int l_shift = 0;
-    if (losers) {
-        l_desc = losers + tb + t;
-        l_ids = l_desc->ids; l_rows = l_desc->rows; l_n = l_desc->n; l_shard = l_desc->shard;
-        l_bucket = l_desc->bucket; l_shift = l_desc->shift;
-    }
+    const LoserDesc* __restrict__ l_desc = losers ? losers + tb + t : nullptr;
     // warp `warp` owns words w_lo + warp, w_lo + warp + NW, ... ; its running ordinal starts at the
     // popcount of the range's words that precede each of them, recomputed per word (ranges are short)
     for (int w = w_lo + warp; w < w_hi; w += NW) {
@@ -218,26 +243,7 @@ __global__ void __launch_bounds__(MISS_NT) fwd_miss_kernel(const TableDesc* __re
                 }
             } else {
                 aux_l = aux_base + ord;
-                int64_t lo = 0, hi = l_n;              // first index with l_ids[idx] >= id
-                if (l_bucket) {                        // bucket index: the answer lies in [bucket[b], bucket[b + 1]]
-                    const int64_t bk = id >> l_shift;
-                    lo = __ldg(l_bucket + bk);
-                    hi = __ldg(l_bucket + bk + 1);
-                }
-                while (lo < hi) {
-                    const int64_t mid = (lo + hi) >> 1;
-                    if (__ldg(l_ids + mid) < id) lo = mid + 1; else hi = mid;
-                }
-                if (lo < l_n && __ldg(l_ids + lo) == id) {
-                    if (l_shard) {              // sharded store: the row is in the HBM of rank lo / shard (NVLink)
-                        const int64_t owner = lo / l_shard;
-                        src_l = l_desc->peer[owner] + (lo - owner * l_shard) * dim;
-                    } else {
-                        src_l = l_rows + lo * dim;                                     // local HBM
-                    }
-                } else {
-                    src_l = master + id * dim;                                         // zero-copy PCIe
-                }
+                src_l = miss_row(l_desc, master, id, dim);
                 slots[(int64_t)t * ld_slots + j] = (int32_t)aux_l;
             }
         }
@@ -268,6 +274,63 @@ __global__ void __launch_bounds__(MISS_NT) fwd_miss_kernel(const TableDesc* __re
                     if (COPY) reinterpret_cast<V*>(out + (int64_t)t * ld_out + (int64_t)(w * 32 + b[u]) * dim)[c] = v[u];
                 }
             }
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------
+// Read-only lookup for evaluation (one id per bag): a warp owns 32 consecutive ids of one table; lane l probes id l
+// and resolves its source row -- the cache row on a hit, else the loser store of the installed window or the master
+// (probe_slot / miss_row, as K1 / K2) -- then groups of G lanes copy the 32 rows to out[], U rows in flight per group.
+// Writes out[] only: no slots, aux rows, miss bitmap, miss counts or dirty bits, so any batch size works.  An id
+// outside its table raises flag 2 and gets a zero row.
+// ------------------------------------------------------------------------------
+template <int WAYS, int VEC>
+__global__ void __launch_bounds__(FWD_NT) fwd_eval_kernel(const TableDesc* __restrict__ tabs, int tb,
+                                                           const int64_t* __restrict__ ids, int64_t ld_ids, int n_idx,
+                                                           const LoserDesc* __restrict__ losers,
+                                                           float* __restrict__ out, int64_t ld_out, int dim, int ways,
+                                                           int G, uint32_t* __restrict__ flags) {
+    pdl_enter();
+    using V = typename VecT<VEC>::type;
+    constexpr int U = 4;
+    const int t = blockIdx.y;
+    const int lane = threadIdx.x & 31;
+    const int j0 = (blockIdx.x * (FWD_NT / 32) + (threadIdx.x >> 5)) * 32;
+    if (j0 >= n_idx) return;
+    const TableDesc& T = tabs[tb + t];
+    const int j = j0 + lane;
+    const float* src = nullptr;
+    if (j < n_idx) {
+        const int64_t id = __ldg(ids + (int64_t)t * ld_ids + j);
+        const int64_t sl = probe_slot<WAYS>(T, id, ways, flags);
+        if (sl >= 0) src = T.weight + sl * dim;
+        else if ((uint64_t)id < (uint64_t)T.n_rows) src = miss_row(losers ? losers + tb + t : nullptr, T.master, id, dim);
+    }
+    const unsigned long long src_bits = (unsigned long long)src;
+    float* tout = out + (int64_t)t * ld_out;
+    const int cpr = dim / VEC;
+    const int NGW = 32 / G, gl = lane % G, g = lane / G;
+    // every group runs the same number of iterations (NGW * U divides 32 or exceeds it): the shuffles stay warp-wide
+    for (int r0 = g; r0 < 32; r0 += NGW * U) {
+        unsigned long long sp[U];
+        int row[U];
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+            const int r = r0 + u * NGW;
+            sp[u] = __shfl_sync(0xffffffffu, src_bits, r < 32 ? r : 0);
+            row[u] = (r < 32 && j0 + r < n_idx) ? j0 + r : -1;
+        }
+        for (int c = gl; c < cpr; c += G) {
+            V v[U];
+#pragma unroll
+            for (int u = 0; u < U; ++u) {
+                vzero(v[u]);
+                if (row[u] >= 0 && sp[u]) v[u] = reinterpret_cast<const V*>(sp[u])[c];
+            }
+#pragma unroll
+            for (int u = 0; u < U; ++u)
+                if (row[u] >= 0) reinterpret_cast<V*>(tout + (int64_t)row[u] * dim)[c] = v[u];
         }
     }
 }
@@ -901,6 +964,54 @@ extern "C" int cdlrm_embed_fwd(cdlrm_ctx* c, int tb, int tc, const int64_t* ids,
         else LAUNCH(K_POOL, s, pool_kernel<1><<<pg, 256, 0, s>>>(c->d_tabs, tb, slots, ld_slots, offsets, ld_off, n_idx, n_bags, out, ld_out, bag_ids, ld_bag, c->dim, G));
         CU_CHECK(cudaGetLastError());
     }
+    return CDLRM_OK;
+}
+
+extern "C" int cdlrm_embed_fwd_eval(cdlrm_ctx* c, int tb, int tc, const int64_t* ids, int64_t ld_ids, int32_t n_idx,
+                                    float* out, int64_t ld_out, cdlrm_stream stream) {
+    ARG_CHECK(c && ids && out);
+    ARG_CHECK(tb >= 0 && tc > 0 && tb + tc <= c->T);
+    ARG_CHECK(n_idx >= 0);
+    cudaStream_t s = (cudaStream_t)stream;
+    CU_CHECK(cudaSetDevice(c->device));
+    for (int k = tb; k < tb + tc; ++k) {
+        if (!c->tabs[k].weight || !c->tabs[k].tags || !c->tabs[k].master) {
+            cdlrm_set_error("table %d: cache or master not bound", k);
+            return CDLRM_ERR_STATE;
+        }
+    }
+    int rc = cdlrm_sync_tabs(c, s);
+    if (rc) return rc;
+    if (n_idx == 0) return CDLRM_OK;
+    bool al16 = true, al8 = true, tags16 = true;
+    for (int k = tb; k < tb + tc; ++k) {
+        al16 = al16 && ((uintptr_t)c->tabs[k].master % 16 == 0);
+        al8 = al8 && ((uintptr_t)c->tabs[k].master % 8 == 0);
+        tags16 = tags16 && ((uintptr_t)c->tabs[k].tags % 16 == 0);
+    }
+    int vec = pick_vec(c->dim, out, nullptr, ld_out, c->dim);
+    if (vec == 4 && !al16) vec = 2;
+    if (vec == 2 && !al8) vec = 1;
+    const int cpr = c->dim / vec;
+    const int G = pow2_ceil(cpr) > 32 ? 32 : pow2_ceil(cpr);
+    const int words = (n_idx + 31) / 32;
+    dim3 grid((words + FWD_NT / 32 - 1) / (FWD_NT / 32), tc);
+    const int wsel = !tags16 ? 0 : (c->ways == 16 ? 16 : c->ways == 8 ? 8 : c->ways == 4 ? 4 : c->ways == 2 ? 2 : 0);
+#define LAUNCH_EVAL(WW, VV) LAUNCH_PDL(K_EMBED_EVAL, s, (fwd_eval_kernel<WW, VV>), grid, FWD_NT, 0, c->d_tabs, tb, ids, ld_ids, n_idx, c->d_losers, out, ld_out, c->dim, c->ways, G, c->d_flags)
+#define EVAL_V(WW)                                  \
+    if (vec == 4) { LAUNCH_EVAL(WW, 4); }           \
+    else if (vec == 2) { LAUNCH_EVAL(WW, 2); }      \
+    else { LAUNCH_EVAL(WW, 1); }
+    switch (wsel) {
+        case 16: EVAL_V(16) break;
+        case 8: EVAL_V(8) break;
+        case 4: EVAL_V(4) break;
+        case 2: EVAL_V(2) break;
+        default: EVAL_V(0) break;
+    }
+#undef EVAL_V
+#undef LAUNCH_EVAL
+    CU_CHECK(cudaGetLastError());
     return CDLRM_OK;
 }
 

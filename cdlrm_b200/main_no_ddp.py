@@ -8,7 +8,9 @@ Kept verbatim as an interface (reference file:line): ``ProcessArgs`` (:34-145),
 (:309-321), ``Run`` (:324-502).
 """
 import argparse
+import collections
 import ctypes
+import itertools
 import math
 import os
 import queue
@@ -24,9 +26,14 @@ from . import _lib
 from . import checkpoint as ckpt
 from ._lib import check, lib
 from .cache_manager import Prefetcher, TorchGlobalRng, VictimRng, VictimRngDevice, WindowPlanner
-from .model_no_ddp import DLRM_Net, Embedding_Table_Cache_Group, Embedding_Table_Group, bce_mean, bce_mean_with_grad
+from .model_no_ddp import (DLRM_Net, Embedding_Table_Cache_Group, Embedding_Table_Group, EvalForward, bce_mean,
+                           bce_mean_with_grad)
 
 _vp = ctypes.c_void_p
+
+# Trainer.evaluate: loss = mean BCE, accuracy = share of round(z) == t, auc = exact ROC AUC (NaN with one class only)
+EvalResult = collections.namedtuple("EvalResult", "samples loss accuracy auc positives negatives")
+_ONE_ID_PER_BAG = "evaluate needs one id per bag: lS_o must be arange(batch) for every table"
 
 # (flag, type or "flag", default) -- spelling and defaults of main_no_ddp.py:34-145
 _FLAGS = [
@@ -833,6 +840,15 @@ class Trainer:
         torch.cuda.synchronize(self.dev)
         self.cache_group.check_device_flags()
 
+    def quiesce_ranks(self):
+        """Collective over the ranks (call it on every rank at the same point): each rank completes its own plan and
+        its share of the pending eviction write-back, then a host barrier.  Afterwards the master holds every row
+        evicted by any rank, and no rank writes it again before the next window boundary, which waits for every rank."""
+        self._need_planner("quiesce_ranks")
+        self._quiesce()
+        if self.world > 1:
+            dist.barrier(group=self._host_group)
+
     def _aggregate_replicas(self):
         if self.world > 1:
             broadcast_and_aggregate(self.cache_group, None, self.rank, self.args.table_agg_op)
@@ -980,6 +996,164 @@ class Trainer:
             dist.barrier(group=self._host_group)
         return self.window
 
+    # -- evaluation -------------------------------------------------------------------------------
+    class _EvalState:
+        """What ``evaluate`` keeps across calls: the forward (its own MLP handles), the metrics object, the CUDA graph
+        of one evaluation step with its static inputs, and the rotating device slots of host batches."""
+
+        def __init__(self, tr):
+            self.fwd = EvalForward(tr.cache_group, tr.dlrm)
+            self.handle, self.cap = None, 0
+            self.graph = self.graph_key = self.static = None
+            self.warm = set()           # batch shapes that ran eagerly once (a capture follows on the next batch)
+            self.slots, self.slot_no = {}, 0
+            self.copy_stream = None
+            self.offsets_ok = None      # the last host lS_o found to be arange(batch) (loaders reuse one tensor)
+
+        def drop_graph(self):
+            if self.graph is not None:
+                torch.cuda.synchronize()
+            self.graph = self.graph_key = self.static = None
+            self.warm.clear()
+
+        def __del__(self):
+            try:
+                if self.handle is not None:
+                    lib.cdlrm_eval_destroy(self.handle)
+            except Exception:
+                pass
+
+    def _eval_inputs(self, ev, X, lS_i, T):
+        """Device tensors of one test batch.  Host batches are copied on a copy stream of the evaluator's own into two
+        rotating device slots per shape (never the training input slots of ``stage_inputs``)."""
+        dev = self.dev
+        if X.is_cuda and lS_i.is_cuda and T.is_cuda:
+            return (X.to(dev, dtype=torch.float32), lS_i.to(dev, dtype=torch.int64), T.to(dev, dtype=torch.float32)), None
+        if ev.copy_stream is None:
+            ev.copy_stream = _lib.new_stream(dev, priority=-1)
+        key = (tuple(X.shape), tuple(lS_i.shape), tuple(T.shape))
+        pair = ev.slots.get(key)
+        if pair is None:
+            pair = ev.slots[key] = [(torch.empty(key[0], dtype=torch.float32, device=dev),
+                                     torch.empty(key[1], dtype=torch.int64, device=dev),
+                                     torch.empty(key[2], dtype=torch.float32, device=dev),
+                                     torch.cuda.Event(), torch.cuda.Event()) for _ in range(2)]
+        ev.slot_no += 1
+        Xd, Id, Td, ready, free = pair[ev.slot_no % 2]
+        cs, cur = ev.copy_stream, torch.cuda.current_stream(dev)
+        cs.wait_event(free)                 # the evaluation step that last read this slot is enqueued before it
+        with torch.cuda.stream(cs):
+            Xd.copy_(X, non_blocking=True)
+            Id.copy_(lS_i, non_blocking=True)
+            Td.copy_(T, non_blocking=True)
+            ready.record(cs)
+        cur.wait_event(ready)
+        return (Xd, Id, Td), free
+
+    def _eval_step(self, ev, X, ids, T):
+        """Predictions of one batch, accumulated into the metrics on the current stream: a replay of the captured
+        step for the graph's shape, else eagerly with the same kernels.  The first shape that runs twice is captured."""
+        dev = self.dev
+        cur = torch.cuda.current_stream(dev)
+        B = int(T.shape[0])
+        key = (tuple(X.shape), tuple(ids.shape), tuple(T.shape))
+        if ev.fwd.reserve(B, dev):
+            ev.drop_graph()             # a captured step holds the old MLP handles
+        use_graph = not getattr(self.args, "no_cuda_graph", False)
+        if use_graph and ev.graph is None and key in ev.warm:
+            torch.cuda.synchronize(dev)
+            ev.static = (torch.empty_like(X), torch.empty_like(ids), torch.empty_like(T))
+            ev.graph = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(ev.graph, capture_error_mode="thread_local"):
+                sx, si, st = ev.static
+                p = ev.fwd(sx, si)
+                check(lib.cdlrm_eval_accumulate(ev.handle, _vp(p.data_ptr()), p.stride(0), _vp(st.data_ptr()),
+                                                st.stride(0), B, _vp(torch.cuda.current_stream(dev).cuda_stream)))
+            ev.graph_key = key
+        if ev.graph is not None and ev.graph_key == key:
+            sx, si, st = ev.static
+            sx.copy_(X)
+            si.copy_(ids)
+            st.copy_(T)
+            ev.graph.replay()
+            return
+        p = ev.fwd(X, ids)
+        check(lib.cdlrm_eval_accumulate(ev.handle, _vp(p.data_ptr()), p.stride(0), _vp(T.data_ptr()), T.stride(0), B,
+                                        _vp(cur.cuda_stream)))
+        ev.warm.add(key)
+
+    def evaluate(self, loader, max_samples=None):
+        """Forward-only pass over ``loader`` (``(X, lS_o, lS_i, T)`` batches, one id per bag, CPU or CUDA tensors) on the
+        trained model, returning ``EvalResult``: samples, mean BCE loss, accuracy (round(z) == t), exact ROC AUC,
+        positives and negatives.  The model read is the cached rows plus the host master: ``_quiesce`` first joins the
+        plan thread and completes this rank's pending eviction write-back (``last_quiesce_s``: seconds it took).  At
+        N > 1 with a shared master every rank writes back a share of the evicted rows: call ``quiesce_ranks()`` on
+        every rank first (``Run`` does), so that the other ranks' shares have landed too.  Nothing the training step
+        reads or writes is touched, so training goes on as if no evaluation had happened.  One host sync at the end.
+        ``max_samples``: capacity of the metrics (default ``len(loader)`` times the first batch size).  Raises
+        ``ValueError`` for a prediction outside [0, 1] or a label outside {0, 1}, ``CdlrmError`` for offsets that are
+        not one id per bag."""
+        self._need_planner("evaluate")
+        t0 = time.perf_counter()
+        self._quiesce()
+        self.last_quiesce_s = time.perf_counter() - t0
+        dev = self.dev
+        ev = getattr(self, "_ev", None)
+        if ev is None:
+            ev = self._ev = Trainer._EvalState(self)
+        it = iter(loader)
+        first = next(it, None)
+        if first is None:
+            return EvalResult(0, float("nan"), float("nan"), float("nan"), 0, 0)
+        cap = int(max_samples) if max_samples is not None else len(loader) * int(first[3].shape[0])
+        if cap > ev.cap:
+            ev.drop_graph()             # the captured step accumulates into the old metrics object
+            if ev.handle is not None:
+                check(lib.cdlrm_eval_destroy(ev.handle))
+                ev.handle, ev.cap = None, 0
+            h = _vp()
+            check(lib.cdlrm_eval_create(ctypes.byref(h), dev.index, cap))
+            ev.handle, ev.cap = h, cap
+        cur = torch.cuda.current_stream(dev)
+        ev.fwd.begin()
+        check(lib.cdlrm_eval_reset(ev.handle, _vp(cur.cuda_stream)))
+        seen = 0
+        off_bad = torch.zeros((), dtype=torch.bool, device=dev)
+        for X, lS_o, lS_i, T in itertools.chain([first], it):
+            B = int(T.shape[0])
+            if int(lS_i.shape[1]) != B or int(lS_o.shape[1]) != B or X.shape[0] != B:
+                raise _lib.CdlrmError("evaluate needs one id per bag (lS_i and lS_o of shape [tables, batch])")
+            if lS_o is not ev.offsets_ok:
+                if not lS_o.is_cuda:
+                    if not bool((lS_o == torch.arange(B, dtype=lS_o.dtype)).all()):
+                        raise _lib.CdlrmError(_ONE_ID_PER_BAG)
+                    ev.offsets_ok = lS_o
+                else:                       # checked on the device, read at the one sync below
+                    torch.logical_or(off_bad, (lS_o != torch.arange(B, dtype=lS_o.dtype, device=lS_o.device)).any().to(dev),
+                                     out=off_bad)
+            seen += B
+            if seen > ev.cap:
+                raise _lib.CdlrmError(f"evaluate: more than {ev.cap} samples (pass max_samples)")
+            (Xd, Id, Td), free = self._eval_inputs(ev, X, lS_i, T)
+            self._eval_step(ev, Xd, Id, Td)
+            if free is not None:
+                free.record(cur)
+        st = _lib.EvalStats()
+        check(lib.cdlrm_eval_result(ev.handle, _vp(ctypes.addressof(st)), _vp(cur.cuda_stream)))
+        self.cache_group.check_device_flags()
+        if bool(off_bad):
+            raise _lib.CdlrmError(_ONE_ID_PER_BAG)
+        if st.flags & 4:
+            raise _lib.CdlrmError(f"evaluate: more than {ev.cap} samples")
+        if st.flags & 1:
+            raise ValueError("evaluate: a prediction outside [0, 1] or NaN")
+        if st.flags & 2:
+            raise ValueError("evaluate: a label outside {0, 1}")
+        n, P, N = int(st.samples), int(st.positives), int(st.negatives)
+        auc = float(st.auc_2u) / (2.0 * P * N) if P > 0 and N > 0 else float("nan")
+        return EvalResult(n, st.loss_sum / n if n else float("nan"), int(st.correct) / n if n else float("nan"), auc,
+                          P, N)
+
 
 def _bcast_fifo_entry(item, rank, dev):
     """One shared ``batch_fifo`` read by rank 0 only (the reference's wiring, main_no_ddp.py:624,638-643): rank 0
@@ -1013,6 +1187,11 @@ def slice_batch(rank, local_batch_size, X, lS_o, lS_i, T):
     return X[lo:hi, :], lS_o[:, :local_batch_size], lS_i[:, lo:hi], T[lo:hi, :]
 
 
+def _print_eval(r):
+    print('Test accuracy = {}%'.format(100 * r.accuracy))
+    print('Test loss = {}, AUC = {}'.format(r.loss, r.auc))
+
+
 def Run(rank, m_spa, ln_emb, ln_bot, ln_top, train_ld, test_ld, batch_fifo, eviction_fifo, occupancy_tables_fifos,
         emb_tables, args):
     """main_no_ddp.py:324-502.  ``batch_fifo`` carries one entry per window in training order: the reference's
@@ -1031,7 +1210,11 @@ def Run(rank, m_spa, ln_emb, ln_bot, ln_top, train_ld, test_ld, batch_fifo, evic
     ``--save-model PATH``: a checkpoint (Trainer.save_checkpoint) at the end of every epoch, replacing the previous
     one, and ``sync_master()`` after the last step, so that ``emb_tables`` holds the trained tables when Run returns.
     ``--load-model PATH``: resume at the checkpoint's window; the steps before it are skipped (``batch_fifo`` must
-    start at that window: ``Prefetcher`` skips the windows before it).  Neither works with ``--strict-reference``."""
+    start at that window: ``Prefetcher`` skips the windows before it).  Neither works with ``--strict-reference``.
+
+    The test pass (``--test-freq`` and the end of the epoch, rank 0) is ``Trainer.evaluate``: accuracy, loss and AUC
+    on the GPU; ``--strict-reference`` keeps the reference's eager loop.  ``--inference-only``: build the Trainer, load
+    ``--load-model`` if given, evaluate ``test_ld`` once and return (one GPU, not with ``--strict-reference``)."""
     os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
     os.environ.setdefault("MASTER_PORT", str(args.master_port))
     if args.world_size > 1 and not dist.is_initialized():
@@ -1039,8 +1222,17 @@ def Run(rank, m_spa, ln_emb, ln_bot, ln_top, train_ld, test_ld, batch_fifo, evic
     strict = bool(getattr(args, "strict_reference", False))
     if strict and (args.save_model or args.load_model):
         raise _lib.CdlrmError("--save-model / --load-model need the look-ahead trainer (not --strict-reference)")
+    if args.inference_only and (strict or args.world_size > 1):
+        raise _lib.CdlrmError("--inference-only evaluates on one GPU with the look-ahead trainer "
+                              "(--world-size 1, not --strict-reference)")
     tr = Trainer(args, m_spa, ln_emb, ln_bot, ln_top, emb_tables, rank=rank, world=args.world_size,
                  strict_reference=strict)
+    if args.inference_only:          # the model of --load-model, else the freshly initialised one; nothing is trained
+        if args.load_model:
+            tr.load_checkpoint(args.load_model)
+        if test_ld is not None:
+            _print_eval(tr.evaluate(test_ld))
+        return tr
     dev, lb, L = tr.dev, tr.local_batch, args.lookahead
     # training on a high-priority stream: the look-ahead planner (side stream, default priority) only
     # takes the SM slots the training step leaves free
@@ -1116,9 +1308,14 @@ def Run(rank, m_spa, ln_emb, ln_bot, ln_top, train_ld, test_ld, batch_fifo, evic
                 print('Epoch {}: Finished {}/{} in {} ms/it. Caching overhead = {}. Loss = {}, Train Acc = {}'.format(
                     epoch, j, len(train_ld), gT, ovh, L_, A / mbs))
                 total_time, total_iter = 0.0, 0
-            if rank == 0 and test_ld is not None and ((args.test_freq > 0 and j > 0 and j % args.test_freq == 0)
-                                                      or j == len(train_ld) - 1):
+            test_point = (args.test_freq > 0 and j > 0 and j % args.test_freq == 0) or j == len(train_ld) - 1
+            if test_point and not strict and args.world_size > 1:
+                tr.quiesce_ranks()          # every rank's share of the write-back lands before rank 0 reads the master
+            if rank == 0 and test_ld is not None and test_point:
                 print('Testing at {}/{}....'.format(j, len(train_ld)))
+                if not strict:
+                    _print_eval(tr.evaluate(test_ld))
+                    continue
                 test_samp = total_test_acc = 0
                 with torch.no_grad():
                     for _i, (Xt, lS_ot, lS_it, Tt) in enumerate(test_ld):
@@ -1204,8 +1401,10 @@ def _rank_main(rank, args, shm_prefix=None):
     args.fifo_per_rank = True
     if not args.fifo_payload:
         args.fifo_payload = "tuples" if args.strict_reference else "ids"
-    cm = Prefetcher(args, emb_tables, batch_fifo, eviction_fifo, finish_event, cache_ld)             # :630
-    cm.start()
+    cm = None
+    if not args.inference_only:
+        cm = Prefetcher(args, emb_tables, batch_fifo, eviction_fifo, finish_event, cache_ld)         # :630
+        cm.start()
     try:
         tr = Run(rank, m_spa, ln_emb, ln_bot, ln_top, train_ld, test_ld, batch_fifo, eviction_fifo, [], emb_tables,
                  args)
@@ -1219,7 +1418,8 @@ def _rank_main(rank, args, shm_prefix=None):
                         os.unlink(f"{shm_prefix}_{k}.bin")
                     except OSError:
                         pass
-    cm.join(timeout=5)
+    if cm is not None:
+        cm.join(timeout=5)
     return tr
 
 
@@ -1234,6 +1434,9 @@ def main(argv=None):
     if args.test_num_workers < 0:
         args.test_num_workers = args.num_workers
     _derive_topology(args)                               # argument errors before any process is spawned
+    if args.inference_only and (args.world_size > 1 or args.strict_reference):
+        sys.exit("ERROR: --inference-only evaluates on one GPU with the look-ahead trainer: use --world-size 1 and "
+                 "no --strict-reference")
     if args.world_size <= 1:
         args.world_size = 1
         return _rank_main(0, args)

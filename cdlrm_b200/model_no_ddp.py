@@ -808,6 +808,80 @@ class _MlpFn(torch.autograd.Function):
         return (None, dx, None) + tuple(grads)
 
 
+class EvalForward:
+    """Forward-only pass of a trained ``Embedding_Table_Cache_Group`` + ``DLRM_Net`` for evaluation, one id per bag:
+    read-only lookup (cdlrm_embed_fwd_eval: cache row, else the installed window's loser store, else the master),
+    bottom MLP, interaction, top MLP.  The MLPs run on cdlrm_mlp handles of its own, sized for the evaluation batch:
+    the training handles, their workspaces and the context's miss bitmap are never resized or written, so a training
+    step captured in a CUDA graph keeps every pointer it holds.  Every launch goes to the current stream."""
+
+    def __init__(self, cache_group, dlrm):
+        self.cg, self.dlrm = cache_group, dlrm
+        sig = getattr(dlrm, "_sigmoid", {})
+        self.mlp = {"bot": _MlpState(dlrm.bot_l, sig.get("bot", -1)), "top": _MlpState(dlrm.top_l, sig.get("top", -1))}
+
+    def begin(self):
+        """Start of an evaluation: the next forward of each MLP splits the current weights into its hi / lo operands."""
+        for st in self.mlp.values():
+            if st.handle is not None:
+                check(lib.cdlrm_mlp_invalidate_split(st.handle))
+
+    def reserve(self, batch, dev):
+        """Size both MLP handles for ``batch``; True when a handle was (re)allocated (graphs holding it are void)."""
+        old = [st.handle for st in self.mlp.values()]
+        for st in self.mlp.values():
+            st.ensure(batch, dev)
+        return [st.handle for st in self.mlp.values()] != old
+
+    def _mlp(self, which, x):
+        st = self.mlp[which]
+        if self.dlrm.mlp_impl != "tcgen05":
+            return (self.dlrm.bot_l if which == "bot" else self.dlrm.top_l)(x)
+        dev, B = x.device, x.shape[0]
+        if x.dtype != torch.float32 or x.stride(1) != 1:
+            x = x.contiguous().float()
+        if st.handle is None or B > st.cap:
+            raise _lib.CdlrmError(f"EvalForward: batch {B} above the reserved capacity (reserve() first)")
+        y = torch.empty(B, st.dims[-1], dtype=torch.float32, device=dev)
+        Ws = [m.weight if m.weight.is_contiguous() else m.weight.contiguous() for m in st.linears]
+        bs = [m.bias if m.bias.is_contiguous() else m.bias.contiguous() for m in st.linears]
+        check(lib.cdlrm_mlp_forward(st.handle, _vp(x.data_ptr()), x.stride(0), B,
+                                    _lib.ptr_array([w.data_ptr() for w in Ws]), _lib.ptr_array([b.data_ptr() for b in bs]),
+                                    _vp(y.data_ptr()), y.stride(0), _stream_ptr(dev)))
+        return y
+
+    @torch.no_grad()
+    def __call__(self, X, ids):
+        """X: float32 [B, m_den], ids: int64 [T, B], both on the device; returns the predictions [B, 1]."""
+        cg, net = self.cg, self.dlrm
+        dev = X.device
+        T, B = int(ids.shape[0]), int(ids.shape[1])
+        if T != len(cg.emb_l):
+            raise _lib.CdlrmError(f"EvalForward: {T} id rows for {len(cg.emb_l)} tables")
+        if ids.stride(1) != 1:
+            ids = ids.contiguous()
+        ly = torch.empty(T, B, cg.dim, dtype=torch.float32, device=dev)
+        check(lib.cdlrm_embed_fwd_eval(cg._ctx, 0, T, _vp(ids.data_ptr()), ids.stride(0), B, _vp(ly.data_ptr()),
+                                       ly.stride(0), _stream_ptr(dev)))
+        x = self._mlp("bot", X)
+        if net.arch_interaction_op == "dot":
+            feats = [x] + list(ly.unbind(0))
+            if x.stride(0) != cg.dim or x.shape[1] != cg.dim:
+                raise _lib.CdlrmError("EvalForward: the bottom MLP must end in the embedding dimension")
+            itself = bool(net.arch_interaction_itself)
+            nf = T + 1
+            npair = nf * (nf + 1) // 2 if itself else nf * (nf - 1) // 2
+            R = torch.empty(B, cg.dim + npair, dtype=torch.float32, device=dev)
+            check(lib.cdlrm_interact_fwd(dev.index, _lib.ptr_array([f.data_ptr() for f in feats]), nf, cg.dim, B, cg.dim,
+                                         int(itself), _vp(R.data_ptr()), R.stride(0), _stream_ptr(dev)))
+        else:
+            R = net.interact_features(x, list(ly.unbind(0)))
+        p = self._mlp("top", R)
+        if 0.0 < net.loss_threshold < 1.0:
+            p = torch.clamp(p, min=net.loss_threshold, max=(1.0 - net.loss_threshold))
+        return p
+
+
 class DLRM_Net(nn.Module):
     """model_no_ddp.py:215-316.  bot_l / top_l are the reference's nn.Sequential stacks (same parameters, same
     numpy-RNG initialisation); on CUDA they execute through cdlrm_mlp_* (TMA + tcgen05 3xTF32 GEMMs, FP32

@@ -95,6 +95,13 @@ int cdlrm_embed_fwd(cdlrm_ctx* ctx, int table_begin, int table_count,
                     int32_t* bag_ids, int64_t ld_bag,
                     cdlrm_stream stream);
 
+/* Read-only lookup for evaluation, one id per bag: out[j] = the cache row of ids[j] when its set's tag line holds it,
+ * else its row in the loser store of the installed window, else master[ids[j]] (zero-copy).  Writes out only (no
+ * slots, aux rows, miss bitmap or dirty bits; no batch limit, no allocation).  An id outside its table raises flag 2
+ * (cdlrm_ctx_check) and gets a zero row.  out: float32 [table_count][n_idx][dim], table stride ld_out. */
+int cdlrm_embed_fwd_eval(cdlrm_ctx* ctx, int table_begin, int table_count, const int64_t* ids, int64_t ld_ids,
+                         int32_t n_idx, float* out, int64_t ld_out, cdlrm_stream stream);
+
 /* ---- backward + SGD: autograd of EmbeddingBag(sparse=True) followed by
  *      optimizer_embeds.step(), main_no_ddp.py:376,409,413 -------------------------
  * weight[slot] -= lr * sum_{j: slot_j == slot} d_out[bag(j)], duplicates merged by a
@@ -431,6 +438,34 @@ int cdlrm_rngdev_set_state(cdlrm_rngdev* rng, const uint32_t* h_state, uint64_t 
 int cdlrm_rngdev_set_option(int key, int64_t value);
 /* d_out[i] = exponential draw of the raw word pair {d_raw[2i], d_raw[2i+1]} (the transform alone) */
 int cdlrm_exp_from_raw(const uint32_t* d_raw, float* d_out, int64_t n, cdlrm_stream stream);
+
+/* ---- evaluation metrics (csrc/eval.cu): predictions z in [0, 1] and labels t in {0, 1} of any number of
+ *      batches -> counts, BCE sum and the exact ROC AUC ------------------------------------------------------------
+ * correct: round_half_even(z) == t.  loss_sum: sum of -(t max(log z, -100) + (1 - t) max(log(1 - z), -100)) in fp64
+ * from the fp32 z, in a fixed order.  auc_2u: 2U = sum over positives of (2 #negatives with a lower z + #negatives
+ * with an equal z), exact; AUC = auc_2u / (2 positives negatives).  flags: bit0 a z outside [0, 1] or NaN, bit1 a t
+ * outside {0, 1}, bit2 more samples than max_samples (the batch that overflowed is dropped).
+ * Memory: 8 bytes per sample of max_samples (<= 2^30) plus < 64 MB. */
+typedef struct cdlrm_eval cdlrm_eval;
+typedef struct cdlrm_eval_stats {
+    int64_t samples;
+    int64_t positives;
+    int64_t negatives;
+    int64_t correct;
+    double loss_sum;
+    uint64_t auc_2u;
+    uint32_t flags;
+    uint32_t reserved;
+} cdlrm_eval_stats;
+int cdlrm_eval_create(cdlrm_eval** out, int device, int64_t max_samples);
+int cdlrm_eval_destroy(cdlrm_eval* ev);
+/* forget every accumulated sample (stream order) */
+int cdlrm_eval_reset(cdlrm_eval* ev, cdlrm_stream stream);
+/* add samples z[i * ldz], t[i * ldt], i < n (float32 device arrays); capturable, allocates nothing */
+int cdlrm_eval_accumulate(cdlrm_eval* ev, const float* z, int64_t ldz, const float* t, int64_t ldt, int32_t n,
+                          cdlrm_stream stream);
+/* metrics of everything accumulated since the last reset; synchronises `stream`; leaves the samples in place */
+int cdlrm_eval_result(cdlrm_eval* ev, cdlrm_eval_stats* h_stats, cdlrm_stream stream);
 
 #ifdef __cplusplus
 }
