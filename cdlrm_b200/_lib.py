@@ -123,6 +123,8 @@ SIGNATURES = {
     "cdlrm_eval_reset": (C.c_int, [vp, vp]),
     "cdlrm_eval_accumulate": (C.c_int, [vp, vp, C.c_int64, vp, C.c_int64, C.c_int32, vp]),
     "cdlrm_eval_result": (C.c_int, [vp, vp, vp]),
+    "cdlrm_criteo_decode": (C.c_int, [C.c_int, vp, C.c_int64, C.c_int32, C.c_int32, C.c_int64, vp, C.c_int64, vp,
+                                      C.c_int64, vp, vp]),
 }
 
 

@@ -1056,11 +1056,27 @@ class Prefetcher(threading.Thread):
         (flag ``--fifo-payload`` of this package's main); the consumers accept either."""
         return getattr(self.args, "fifo_payload", None) or "tuples"
 
+    def markers(self):
+        """``ids`` payloads of a ``cache_ld`` that provides ``window_marker`` (criteo_bin.CriteoBinDataset): one marker
+        per window in training order, the windows before the ``--load-model`` resume point skipped, the short last
+        window of an epoch included.  Nothing is read here: the plan thread reads each window when it scans it."""
+        L = self.args.lookahead
+        per_epoch = -(-len(self.cache_ld) // L)
+        skip = 0
+        if getattr(self.args, "load_model", ""):
+            from .checkpoint import read_meta
+            skip = int(read_meta(self.args.load_model)["resume"]["window"])
+        for w in range(skip, self.args.nepochs * per_epoch):
+            yield self.cache_ld.window_marker(w % per_epoch, L)
+
     def payloads(self):
         """Generator of the FIFO entries in training order (what ``run`` puts)."""
         mode = self.fifo_payload
         if mode not in ("tuples", "ids"):
             raise ValueError("fifo_payload must be 'tuples' or 'ids', got %r" % (mode,))
+        if mode == "ids" and hasattr(self.cache_ld, "window_marker"):
+            yield from self.markers()
+            return
         for win in self.windows():
             if mode == "ids":
                 yield win

@@ -1260,7 +1260,10 @@ def Run(rank, m_spa, ln_emb, ln_bot, ln_top, train_ld, test_ld, batch_fifo, evic
         tr.submit_window(next_entry())
     step_no = 0
     for epoch in range(args.nepochs):
-        for j, (X, lS_o, lS_i, T) in enumerate(train_ld):
+        # a loader that can start at a batch (criteo_bin.DeviceBatches) reads nothing before the resume point
+        j0 = min(max(0, (start_w - epoch * per_epoch) * L), len(train_ld))
+        batches = enumerate(train_ld.iter_from(j0), j0) if j0 and hasattr(train_ld, "iter_from") else enumerate(train_ld)
+        for j, (X, lS_o, lS_i, T) in batches:
             if epoch * per_epoch + j // L < start_w:                                 # before the resume point
                 continue
             X, lS_o, lS_i, T = slice_batch(rank, lb, X, lS_o, lS_i, T)               # :388-391
@@ -1344,9 +1347,19 @@ def _derive_topology(args):
     """:525-616: table sizes, MLP shapes and the reference's sanity checks (same messages)."""
     ln_bot = np.fromstring(args.arch_mlp_bot, dtype=int, sep="-")
     if args.data_generation == "dataset":
-        sys.exit("ERROR: --data-generation=dataset needs the Criteo loaders (dlrm_data_pytorch.py), which are outside "
-                 "the cache hot path this package implements; use --data-generation=synthetic")
-    ln_emb = np.fromstring(args.arch_embedding_size, dtype=int, sep="-")
+        if not args.mlperf_bin_loader:
+            sys.exit("ERROR: --data-generation=dataset reads Criteo data in the MLPerf binary format only: add "
+                     "--mlperf-bin-loader (the raw text and per-day npz loaders need the upstream preprocessing)")
+        if args.world_size > 1:
+            sys.exit("ERROR: --data-generation=dataset trains on one GPU: use --world-size 1 (per-rank sample "
+                     "slices of a dataset are a follow-up)")
+        if args.mlperf_bin_shuffle:
+            sys.exit("ERROR: --mlperf-bin-shuffle is not supported: the binary loader reads the batches in file order")
+        from .criteo_bin import DENSE, table_sizes
+        ln_emb = table_sizes(args)                       # from the counts file: overrides --arch-embedding-size
+        ln_bot[0] = DENSE                                # m_den = train_data.m_den
+    else:
+        ln_emb = np.fromstring(args.arch_embedding_size, dtype=int, sep="-")
     m_den = ln_bot[0]
     m_spa = args.arch_sparse_feature_size
     num_fea = ln_emb.size + 1
@@ -1381,7 +1394,11 @@ def _rank_main(rank, args, shm_prefix=None):
     ln_emb, ln_bot, ln_top, m_spa, m_den = _derive_topology(args)
     np.random.seed(args.numpy_rand_seed)
     torch.manual_seed(args.numpy_rand_seed)
-    train_ld, test_ld, cache_ld = make_synthetic_data_and_loaders(args, ln_emb, m_den)
+    if args.data_generation == "dataset":
+        from .criteo_bin import make_criteo_bin_loaders
+        train_ld, test_ld, cache_ld, _ln = make_criteo_bin_loaders(args, torch.device("cuda", rank))
+    else:
+        train_ld, test_ld, cache_ld = make_synthetic_data_and_loaders(args, ln_emb, m_den)
     torch.cuda.set_device(rank)
     if args.world_size > 1:
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
@@ -1425,7 +1442,9 @@ def _rank_main(rank, args, shm_prefix=None):
 
 def main(argv=None):
     """python -m cdlrm_b200.main_no_ddp [the reference's flags] -- README.md:7 of the reference, with
-    ``--data-generation synthetic`` (Criteo-shaped synthetic batches, cdlrm_b200/synthetic.py)."""
+    ``--data-generation synthetic`` (Criteo-shaped synthetic batches, cdlrm_b200/synthetic.py) or
+    ``--data-generation dataset --mlperf-bin-loader`` (Criteo in the MLPerf binary format, cdlrm_b200/criteo_bin.py;
+    one GPU)."""
     args = ProcessArgs(argv)
     np.set_printoptions(precision=args.print_precision)
     torch.set_printoptions(precision=args.print_precision)

@@ -467,6 +467,19 @@ int cdlrm_eval_accumulate(cdlrm_eval* ev, const float* z, int64_t ldz, const flo
 /* metrics of everything accumulated since the last reset; synchronises `stream`; leaves the samples in place */
 int cdlrm_eval_result(cdlrm_eval* ev, cdlrm_eval_stats* h_stats, cdlrm_stream stream);
 
+/* ---- MLPerf binary Criteo records (csrc/criteo.cu): replaces the host decode of data_loader_terabyte.py,
+ *      CriteoBinDataset.__getitem__ :224-235 and _transform_features :68-87 (flag_input_torch_tensor=True) --------
+ * rec: n device records of 1 + n_dense + n_sparse int32 fields [label, dense..., categorical...] (4-byte aligned).
+ *   X[i * ld_x + c]     = logf((float)dense_c + 1.0f)         torch.log(x_int.float() + 1)
+ *   ids[k * ld_ids + i] = (int64)cat_k, floor modulo max_ind_range when max_ind_range > 0 (torch's %: the result
+ *                         takes the divisor's sign)           (x_cat % max_ind_range).long().t()
+ *   T[i]                = (float)label                        y.float()
+ * Any output may be NULL (not written); n == 0 launches nothing.  Ids are not range-checked here (the forward and
+ * the planner flag an id outside its table).  At most 95 fields per record. */
+int cdlrm_criteo_decode(int device, const int32_t* rec, int64_t n, int32_t n_dense, int32_t n_sparse,
+                        int64_t max_ind_range, float* X, int64_t ld_x, int64_t* ids, int64_t ld_ids, float* T,
+                        cdlrm_stream stream);
+
 #ifdef __cplusplus
 }
 #endif
