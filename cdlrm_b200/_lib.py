@@ -37,6 +37,8 @@ SIGNATURES = {
     "cdlrm_embed_bwd_plan": (C.c_int, [vp, C.c_int, C.c_int, vp, C.c_int64, C.c_int32, vp, vp]),
     "cdlrm_embed_bwd_sgd": (C.c_int, [vp, C.c_int, C.c_int, vp, C.c_int32, vp, C.c_int64, vp, C.c_int64,
                                       C.c_int64, C.c_float, vp]),
+    "cdlrm_embed_bwd_sgd_dlr": (C.c_int, [vp, C.c_int, C.c_int, vp, C.c_int32, vp, C.c_int64, vp, C.c_int64,
+                                          C.c_int64, vp, vp]),
     "cdlrm_embed_set_option": (C.c_int, [C.c_int, C.c_int]),
     "cdlrm_interact_set_option": (C.c_int, [C.c_int, C.c_int]),
     "cdlrm_interact_fwd": (C.c_int, [C.c_int, C.POINTER(vp), C.c_int, C.c_int64, C.c_int32, C.c_int, C.c_int,
@@ -49,11 +51,15 @@ SIGNATURES = {
     "cdlrm_mlp_set_option": (C.c_int, [C.c_int, C.c_int]),
     "cdlrm_mlp_set_trace": (C.c_int, [vp]),
     "cdlrm_mlp_sgd_split": (C.c_int, [C.c_int, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.c_float, vp, vp, C.c_int64, vp]),
+    "cdlrm_mlp_sgd_split_dlr": (C.c_int, [C.c_int, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), vp, vp, vp, C.c_int64,
+                                          vp]),
     "cdlrm_mlp_invalidate_split": (C.c_int, [vp]),
     "cdlrm_mlp_set_defer_join": (C.c_int, [vp, C.c_int]),
     "cdlrm_mlp_join": (C.c_int, [vp, vp]),
     "cdlrm_mlp_forward": (C.c_int, [vp, vp, C.c_int64, C.c_int32, C.POINTER(vp), C.POINTER(vp), vp, C.c_int64, vp]),
     "cdlrm_mlp_backward": (C.c_int, [vp, vp, C.c_int64, vp, C.c_int64, C.POINTER(vp), C.POINTER(vp), vp]),
+    "cdlrm_lr_set": (C.c_int, [C.c_int, vp, C.c_double, C.c_double, C.c_int64, C.c_int64, C.c_int64, C.c_int64, vp]),
+    "cdlrm_lr_advance": (C.c_int, [C.c_int, vp, vp]),
     "cdlrm_plan_workspace_bytes": (C.c_int64, [vp, C.c_int64]),
     "cdlrm_plan_bind_workspace": (C.c_int, [vp, vp, C.c_int64, C.c_int64]),
     "cdlrm_plan_unique": (C.c_int, [vp, vp, C.c_int64, C.c_int64, vp, vp]),
@@ -132,6 +138,12 @@ class EvalStats(C.Structure):
     """cdlrm_eval_stats (include/cdlrm_b200.h)."""
     _fields_ = [("samples", C.c_int64), ("positives", C.c_int64), ("negatives", C.c_int64), ("correct", C.c_int64),
                 ("loss_sum", C.c_double), ("auc_2u", C.c_uint64), ("flags", C.c_uint32), ("reserved", C.c_uint32)]
+
+
+class LrState(C.Structure):
+    """cdlrm_lr_state (include/cdlrm_b200.h): lives in device memory, this is its layout."""
+    _fields_ = [("lr", C.c_float * 2), ("base", C.c_double * 2), ("warmup_steps", C.c_int64),
+                ("decay_start_step", C.c_int64), ("decay_steps", C.c_int64), ("count", C.c_int64)]
 
 
 class CdlrmError(RuntimeError):

@@ -42,9 +42,15 @@ def read_meta(path):
         return json.load(f)
 
 
+# fields added after checkpoints were first written, with the value every older checkpoint was trained with
+_ADDED_DEFAULTS = {("args", "lr_num_warmup_steps"): 0, ("args", "lr_decay_start_step"): 0,
+                   ("args", "lr_num_decay_steps"): 0}
+
+
 def check_meta(saved, expected):
     """Raise ``CheckpointMismatch`` naming the first field of ``expected`` ("format", "shapes.*", "args.*") that the
-    saved meta data does not hold with the same value."""
+    saved meta data does not hold with the same value.  A field missing from the saved meta data is a mismatch, except
+    the learning-rate schedule (``args.lr_*``: a checkpoint written before it existed was trained without one)."""
     if saved.get("format") != expected["format"]:
         raise CheckpointMismatch("checkpoint field format: saved %r, this trainer reads %r"
                                  % (saved.get("format"), expected["format"]))
@@ -54,7 +60,7 @@ def check_meta(saved, expected):
                                  "(resuming at a different world size is not supported)" % (ws, we))
     for sec in ("shapes", "args"):
         for key, want in expected[sec].items():
-            got = saved.get(sec, {}).get(key, "<missing>")
+            got = saved.get(sec, {}).get(key, _ADDED_DEFAULTS.get((sec, key), "<missing>"))
             if got != want:
                 raise CheckpointMismatch("checkpoint field %s.%s: saved %r, this trainer has %r" % (sec, key, got, want))
 

@@ -124,7 +124,7 @@ enum KernelId {
     K_PROBE = 0, K_GATHER, K_POOL, K_BWD_PLAN, K_BWD_SGD, K_BWD_SGD_MULTI, K_INT_FWD, K_INT_BWD,
     K_PLAN_BITMAP_SET, K_PLAN_COMPACT, K_PLAN_PROBE, K_PLAN_SURV, K_PLAN_SELECT, K_PLAN_LISTS,
     K_MOVE_EVICT, K_MOVE_GATHER, K_MOVE_FILL, K_MOVE_SCATTER, K_AGG_MARK, K_AGG_OR, K_AGG_COLLECT,
-    K_AGG_PACK, K_AGG_UNPACK, K_MISC, K_RNG_MT, K_RNG_EXP, K_MLP_GEMM, K_MLP_SPLIT, K_EMBED_EVAL, K_EVAL, K_NULL, K_COUNT
+    K_AGG_PACK, K_AGG_UNPACK, K_MISC, K_RNG_MT, K_RNG_EXP, K_MLP_GEMM, K_MLP_SPLIT, K_EMBED_EVAL, K_EVAL, K_LR, K_NULL, K_COUNT
 };
 void cdlrm_prof_mark(int id, cudaStream_t s, int end);
 // wraps one kernel launch statement

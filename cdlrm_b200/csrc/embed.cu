@@ -735,13 +735,23 @@ __global__ void __launch_bounds__(CPL_NT, 1) bwd_plan_cluster_kernel(const Table
 constexpr int CHB = 8;          // entries in flight per lane group
 constexpr int APPLY_NT = 256;
 
-template <int G>
+// the learning rate of an update: a kernel argument, or (DLR) the value a device buffer holds when the kernel runs
+// (cdlrm_lr_advance / cdlrm_lr_set write it earlier in stream order; read after griddepcontrol.wait)
+template <bool DLR>
+__device__ __forceinline__ float load_lr(float lr, const float* d_lr) {
+    if constexpr (DLR) return *d_lr;
+    else return lr;
+}
+
+template <int G, bool DLR>
 __global__ void __launch_bounds__(APPLY_NT, 2) bwd_sgd_apply_kernel(const TableDesc* __restrict__ tabs, int tb,
                                                                      PlanView pv, int n_idx, int j0, int n,
                                                                      const int32_t* __restrict__ bag_ids, int64_t ld_bag,
                                                                      const float* __restrict__ d_out, int64_t ld_dout,
-                                                                     int64_t row_stride, float lr, int dim) {
+                                                                     int64_t row_stride, float lr_arg,
+                                                                     const float* __restrict__ d_lr, int dim) {
     pdl_enter();
+    const float lr = load_lr<DLR>(lr_arg, d_lr);
     constexpr int NGW = 32 / G;               // lane groups per warp
     constexpr int EPG = G;                    // sorted entries per group (32 / NGW)
     constexpr int NB = EPG < CHB ? EPG : CHB; // entries per batch
@@ -824,13 +834,15 @@ __global__ void __launch_bounds__(APPLY_NT, 2) bwd_sgd_apply_kernel(const TableD
 }
 
 // generic fallback (any dim / alignment): one lane group per sorted entry, always atomic
-template <int VEC>
+template <int VEC, bool DLR>
 __global__ void __launch_bounds__(256) bwd_sgd_kernel(const TableDesc* __restrict__ tabs, int tb,
                                                       PlanView pv, int n_idx, int j0, int n,
                                                       const int32_t* __restrict__ bag_ids, int64_t ld_bag,
                                                       const float* __restrict__ d_out, int64_t ld_dout,
-                                                      int64_t row_stride, float lr, int dim, int G) {
+                                                      int64_t row_stride, float lr_arg, const float* __restrict__ d_lr,
+                                                      int dim, int G) {
     using V = typename VecT<VEC>::type;
+    const float lr = load_lr<DLR>(lr_arg, d_lr);
     const int t = blockIdx.y;
     const int gl = threadIdx.x % G, group = threadIdx.x / G, NG = 256 / G;
     const int e = blockIdx.x * NG + group;
@@ -1065,11 +1077,13 @@ extern "C" int cdlrm_embed_bwd_plan(cdlrm_ctx* c, int tb, int tc, const int32_t*
     return CDLRM_OK;
 }
 
-extern "C" int cdlrm_embed_bwd_sgd(cdlrm_ctx* c, int tb, int tc, const void* plan, int32_t n_idx,
-                                   const int32_t* bag_ids, int64_t ld_bag, const float* d_out, int64_t ld_dout,
-                                   int64_t row_stride, float lr, cdlrm_stream stream) {
+template <bool DLR>
+static int bwd_sgd_launch(cdlrm_ctx* c, int tb, int tc, const void* plan, int32_t n_idx, const int32_t* bag_ids,
+                          int64_t ld_bag, const float* d_out, int64_t ld_dout, int64_t row_stride, float lr,
+                          const float* d_lr, cdlrm_stream stream) {
     ARG_CHECK(c && plan && d_out);
     ARG_CHECK(tb >= 0 && tc > 0 && tb + tc <= c->T && n_idx >= 0);
+    ARG_CHECK(!DLR || d_lr);
     if (n_idx == 0) return CDLRM_OK;
     cudaStream_t s = (cudaStream_t)stream;
     CU_CHECK(cudaSetDevice(c->device));
@@ -1089,7 +1103,7 @@ extern "C" int cdlrm_embed_bwd_sgd(cdlrm_ctx* c, int tb, int tc, const void* pla
         if (vec == 4 && cpr <= 32) {
             dim3 grid((n + APPLY_NT - 1) / APPLY_NT, tc);     // a warp per 32 sorted entries
 #define LAUNCH_SGD(GG)                                                                                         \
-    LAUNCH_PDL(K_BWD_SGD, s, (bwd_sgd_apply_kernel<GG>), grid, APPLY_NT, 0, c->d_tabs, tb, pv, n_idx, j0, n, bag_ids, ld_bag, d_out, ld_dout, row_stride, lr, c->dim)
+    LAUNCH_PDL(K_BWD_SGD, s, (bwd_sgd_apply_kernel<GG, DLR>), grid, APPLY_NT, 0, c->d_tabs, tb, pv, n_idx, j0, n, bag_ids, ld_bag, d_out, ld_dout, row_stride, lr, d_lr, c->dim)
             switch (G) {
                 case 1: LAUNCH_SGD(1); break;
                 case 2: LAUNCH_SGD(2); break;
@@ -1101,11 +1115,23 @@ extern "C" int cdlrm_embed_bwd_sgd(cdlrm_ctx* c, int tb, int tc, const void* pla
 #undef LAUNCH_SGD
         } else {
             dim3 grid((n + NG - 1) / NG, tc);
-            if (vec == 4) LAUNCH(K_BWD_SGD, s, bwd_sgd_kernel<4><<<grid, 256, 0, s>>>(c->d_tabs, tb, pv, n_idx, j0, n, bag_ids, ld_bag, d_out, ld_dout, row_stride, lr, c->dim, G));
-            else if (vec == 2) LAUNCH(K_BWD_SGD, s, bwd_sgd_kernel<2><<<grid, 256, 0, s>>>(c->d_tabs, tb, pv, n_idx, j0, n, bag_ids, ld_bag, d_out, ld_dout, row_stride, lr, c->dim, G));
-            else LAUNCH(K_BWD_SGD, s, bwd_sgd_kernel<1><<<grid, 256, 0, s>>>(c->d_tabs, tb, pv, n_idx, j0, n, bag_ids, ld_bag, d_out, ld_dout, row_stride, lr, c->dim, G));
+            if (vec == 4) LAUNCH(K_BWD_SGD, s, (bwd_sgd_kernel<4, DLR><<<grid, 256, 0, s>>>(c->d_tabs, tb, pv, n_idx, j0, n, bag_ids, ld_bag, d_out, ld_dout, row_stride, lr, d_lr, c->dim, G)));
+            else if (vec == 2) LAUNCH(K_BWD_SGD, s, (bwd_sgd_kernel<2, DLR><<<grid, 256, 0, s>>>(c->d_tabs, tb, pv, n_idx, j0, n, bag_ids, ld_bag, d_out, ld_dout, row_stride, lr, d_lr, c->dim, G)));
+            else LAUNCH(K_BWD_SGD, s, (bwd_sgd_kernel<1, DLR><<<grid, 256, 0, s>>>(c->d_tabs, tb, pv, n_idx, j0, n, bag_ids, ld_bag, d_out, ld_dout, row_stride, lr, d_lr, c->dim, G)));
         }
     }
     CU_CHECK(cudaGetLastError());
     return CDLRM_OK;
+}
+
+extern "C" int cdlrm_embed_bwd_sgd(cdlrm_ctx* c, int tb, int tc, const void* plan, int32_t n_idx,
+                                   const int32_t* bag_ids, int64_t ld_bag, const float* d_out, int64_t ld_dout,
+                                   int64_t row_stride, float lr, cdlrm_stream stream) {
+    return bwd_sgd_launch<false>(c, tb, tc, plan, n_idx, bag_ids, ld_bag, d_out, ld_dout, row_stride, lr, nullptr, stream);
+}
+
+extern "C" int cdlrm_embed_bwd_sgd_dlr(cdlrm_ctx* c, int tb, int tc, const void* plan, int32_t n_idx,
+                                       const int32_t* bag_ids, int64_t ld_bag, const float* d_out, int64_t ld_dout,
+                                       int64_t row_stride, const float* d_lr, cdlrm_stream stream) {
+    return bwd_sgd_launch<true>(c, tb, tc, plan, n_idx, bag_ids, ld_bag, d_out, ld_dout, row_stride, 0.f, d_lr, stream);
 }

@@ -557,15 +557,19 @@ struct SplitBatch {
     SplitJob job[MAX_LAYERS];
     int n;
     float lr;
+    const float* d_lr;           // split_batch_kernel<true>: the learning rate is *d_lr, read after griddepcontrol.wait
     // trailing blocks (blockIdx.x >= tiles): plain SGD on a vector that needs no split (the biases)
     int tiles;
     float* vec; const float* vec_grad; int64_t vec_n;
 };
+template <bool DLR>
 __global__ void __launch_bounds__(256) split_batch_kernel(const __grid_constant__ SplitBatch sb) {
     pdl_enter();
+    float lr = sb.lr;
+    if constexpr (DLR) lr = *sb.d_lr;
     if (sb.vec && (int)blockIdx.x >= sb.tiles) {
         const int64_t i = (int64_t)((int)blockIdx.x - sb.tiles) * 256 + threadIdx.x;
-        if (i < sb.vec_n) sb.vec[i] = fmaf(-sb.lr, sb.vec_grad[i], sb.vec[i]);
+        if (i < sb.vec_n) sb.vec[i] = fmaf(-lr, sb.vec_grad[i], sb.vec[i]);
         return;
     }
     int j = 0;
@@ -581,7 +585,7 @@ __global__ void __launch_bounds__(256) split_batch_kernel(const __grid_constant_
         if (r < jb.rows && c < jb.cols) {
             float v = jb.src[(int64_t)r * jb.lds + c];
             if (jb.grad) {
-                v = fmaf(-sb.lr, jb.grad[(int64_t)r * jb.lds + c], v);
+                v = fmaf(-lr, jb.grad[(int64_t)r * jb.lds + c], v);
                 const_cast<float*>(jb.src)[(int64_t)r * jb.lds + c] = v;
             }
             const float h = tf32_hi(v);
@@ -1153,10 +1157,12 @@ extern "C" int cdlrm_mlp_join(cdlrm_mlp* m, cdlrm_stream stream) {
 
 // SGD step of the weight matrices of up to two MLPs fused with the hi/lo split of the UPDATED weights, plus plain SGD on one extra vector (the biases): ONE launch instead of the optimizer's axpy and one
 // split launch at the head of each forward -- which sat on the critical path of the step (before the bottom MLP's
-// first GEMM, and between the interaction and the top MLP).
-extern "C" int cdlrm_mlp_sgd_split(int n_mlps, cdlrm_mlp* const* mlps, float* const* h_W, const float* const* h_dW, float lr,
-                                   float* vec, const float* vec_grad, int64_t vec_n, cdlrm_stream stream) {
+// first GEMM, and between the interaction and the top MLP).  DLR: the learning rate is *d_lr (device), not lr.
+template <bool DLR>
+static int sgd_split_launch(int n_mlps, cdlrm_mlp* const* mlps, float* const* h_W, const float* const* h_dW, float lr,
+                            const float* d_lr, float* vec, const float* vec_grad, int64_t vec_n, cdlrm_stream stream) {
     ARG_CHECK(n_mlps >= 1 && n_mlps <= 2 && mlps && h_W && h_dW && vec_n >= 0 && (vec_n == 0 || (vec && vec_grad)));
+    ARG_CHECK(!DLR || d_lr);
     cudaStream_t s = (cudaStream_t)stream;
     SplitBatch sb = {};
     int tiles = 0, j = 0;
@@ -1176,13 +1182,25 @@ extern "C" int cdlrm_mlp_sgd_split(int n_mlps, cdlrm_mlp* const* mlps, float* co
     CU_CHECK(cudaSetDevice(mlps[0]->device));
     sb.n = j;
     sb.lr = lr;
+    sb.d_lr = d_lr;
     sb.tiles = tiles;
     sb.vec = vec_n ? vec : nullptr; sb.vec_grad = vec_grad; sb.vec_n = vec_n;
     const int blocks = tiles + (int)((vec_n + 255) / 256);
-    LAUNCH_PDL(K_MLP_SPLIT, s, split_batch_kernel, blocks, 256, 0, sb);
+    LAUNCH_PDL(K_MLP_SPLIT, s, split_batch_kernel<DLR>, blocks, 256, 0, sb);
     CU_CHECK(cudaGetLastError());
     for (int a = 0; a < n_mlps; ++a) mlps[a]->w_presplit = true;
     return CDLRM_OK;
+}
+
+extern "C" int cdlrm_mlp_sgd_split(int n_mlps, cdlrm_mlp* const* mlps, float* const* h_W, const float* const* h_dW, float lr,
+                                   float* vec, const float* vec_grad, int64_t vec_n, cdlrm_stream stream) {
+    return sgd_split_launch<false>(n_mlps, mlps, h_W, h_dW, lr, nullptr, vec, vec_grad, vec_n, stream);
+}
+
+extern "C" int cdlrm_mlp_sgd_split_dlr(int n_mlps, cdlrm_mlp* const* mlps, float* const* h_W, const float* const* h_dW,
+                                       const float* d_lr, float* vec, const float* vec_grad, int64_t vec_n,
+                                       cdlrm_stream stream) {
+    return sgd_split_launch<true>(n_mlps, mlps, h_W, h_dW, 0.f, d_lr, vec, vec_grad, vec_n, stream);
 }
 
 // the weights were changed by something else than cdlrm_mlp_sgd_split: the next forward splits them again
@@ -1224,7 +1242,7 @@ extern "C" int cdlrm_mlp_forward(cdlrm_mlp* m, const float* x, int64_t ldx, int3
         }
         sb.n = L;
         sb.tiles = tiles;
-        LAUNCH_PDL(K_MLP_SPLIT, s, split_batch_kernel, tiles, 256, 0, sb);
+        LAUNCH_PDL(K_MLP_SPLIT, s, split_batch_kernel<false>, tiles, 256, 0, sb);
         CU_CHECK(cudaGetLastError());
     }
     // input

@@ -75,6 +75,9 @@ _EXTRA_FLAGS = [
     # what Prefetcher.run puts on batch_fifo: "tuples" = the reference's (rows, uniq, maps); "ids" = raw window ids
     ("fifo-payload", str, ""),
     ("no-cuda-graph", "flag", False),
+    # upstream DLRM's learning-rate policy (dlrm_s_pytorch.py: LRPolicyScheduler and these flags, same spelling and
+    # defaults): linear warmup over the first W steps, quadratic decay over N steps from step D; see lr_policy
+    ("lr-num-warmup-steps", int, 0), ("lr-decay-start-step", int, 0), ("lr-num-decay-steps", int, 0),
 ]
 
 
@@ -90,6 +93,36 @@ def build_parser():
 
 def ProcessArgs(argv=None):
     return build_parser().parse_args(argv)
+
+
+def lr_policy(b, c, W, D, N):
+    """The learning rate of step ``c`` (1-based: the k-th training step of the run has c = k) for the base rate ``b``
+    under upstream DLRM's LRPolicyScheduler with ``W = --lr-num-warmup-steps``, ``D = --lr-decay-start-step``,
+    ``N = --lr-num-decay-steps``: linear warmup for c < W, ``max(1e-7, b x^2)`` with ``x = (N - (c - D)) / N`` for
+    D <= c < D + N, else held at the last value (after the decay; between warmup and decay, where upstream holds the
+    value of step W - 1), or ``b`` when N == 0.  Where upstream has no value to hold (W < 2, c < D) this returns ``b``;
+    upstream fails there.  fp64 arithmetic rounded to fp32 once, returned as a Python float: the host mirror of
+    cdlrm_lr_advance (csrc/lr.cu), the same operations in the same order."""
+    def warmup(c):
+        return b * (1.0 - (W - c) / W)
+
+    def decay(c):
+        x = (N - (c - D)) / N
+        return max(1e-7, b * (x * x))
+
+    if c < W:
+        v = warmup(c)
+    elif D <= c < D + N:
+        v = decay(c)
+    elif N == 0:
+        v = b
+    elif c >= D + N:
+        v = decay(D + N - 1)
+    elif W >= 2:
+        v = warmup(W - 1)
+    else:
+        v = b
+    return float(np.float32(v))
 
 
 # ------------------------------------------------------------------------------------
@@ -397,6 +430,22 @@ class Trainer:
         # the sparse update runs on the lookup stream beside the bottom MLP's backward (joined by
         # optimizer_embeds.step()); CDLRM_OVERLAP_UPDATE=0: from the optimizer hook, after the whole backward
         self.overlap_update = not self.strict and os.environ.get("CDLRM_OVERLAP_UPDATE", "1") != "0"
+        # the learning rates of the step live in device memory (cdlrm_lr_state) where both updates are the fused kernels,
+        # which read them when they run: eager steps and graph replays follow the schedule and any change of
+        # param_groups[0]["lr"], which is the BASE the schedule scales.  CDLRM_MLP=torch, CDLRM_FLAT_MLP=0,
+        # CDLRM_SGD_SPLIT=0 and CDLRM_OVERLAP_UPDATE=0 keep host floats (a captured step then holds its values)
+        self.lr_schedule = tuple(int(getattr(args, k, 0)) for k in
+                                 ("lr_num_warmup_steps", "lr_decay_start_step", "lr_num_decay_steps"))
+        self.device_lr = self.flat and self.dlrm.fused_sgd_split and self.overlap_update
+        self._lr_state = self._lr_base = None
+        if any(self.lr_schedule) and not self.strict and not self.device_lr:
+            raise _lib.CdlrmError("--lr-num-warmup-steps / --lr-decay-start-step / --lr-num-decay-steps need the fused "
+                                  "updates: not with CDLRM_MLP=torch, CDLRM_FLAT_MLP=0, CDLRM_SGD_SPLIT=0 or "
+                                  "CDLRM_OVERLAP_UPDATE=0")
+        if self.device_lr:
+            self._lr_state = torch.zeros(ctypes.sizeof(_lib.LrState) // 8, dtype=torch.int64, device=self.dev)
+            lrs = self._lr_state.view(torch.float32)
+            self._lr_dense, self._lr_sparse = lrs[0:1], lrs[1:2]     # LrState.lr: [dense, sparse]
         self.planner = None
         if not self.strict:
             self.planner = WindowPlanner(self.cache_group, emb_tables, args.lookahead * args.mini_batch_size,
@@ -469,6 +518,36 @@ class Trainer:
         self._submitted_steps = []
         self._rng_snaps = {}
         self._finished = False
+        self._sync_lr()
+
+    # -- learning rate ---------------------------------------------------------------------------
+    def _lr_bases(self):
+        return float(self.optimizer_mlps.param_groups[0]["lr"]), float(self.optimizer_embeds.param_groups[0]["lr"])
+
+    def _set_lr_state(self):
+        """Write the bases, the schedule and the step count into the device state, in stream order."""
+        b = self._lr_bases()
+        if self._lr_state is not None:
+            check(lib.cdlrm_lr_set(self.dev.index, _vp(self._lr_state.data_ptr()), b[0], b[1], *self.lr_schedule,
+                                   self.global_step, _vp(torch.cuda.current_stream(self.dev).cuda_stream)))
+        self._lr_base = b
+
+    def _sync_lr(self):
+        """Before every step: a changed ``param_groups[0]["lr"]`` of either optimizer becomes the new base.  On the
+        host-float path a captured step cannot see it, so a change after the capture raises."""
+        if self._lr_bases() == self._lr_base:
+            return
+        if self._lr_state is None and getattr(self, "_graph", None) is not None:
+            raise _lib.CdlrmError("the learning rate changed after the training step was captured, and with "
+                                  "CDLRM_MLP=torch, CDLRM_FLAT_MLP=0, CDLRM_SGD_SPLIT=0 or CDLRM_OVERLAP_UPDATE=0 the "
+                                  "captured step holds the old value: use --no-cuda-graph")
+        self._set_lr_state()
+
+    def current_lr(self):
+        """(dense, sparse): the learning rates of the last step run (the step count is ``global_step``), as fp32 values
+        -- ``lr_policy`` of the bases, which are ``param_groups[0]["lr"]`` of ``optimizer_mlps`` / ``optimizer_embeds``
+        as of that step."""
+        return tuple(lr_policy(b, self.global_step, *self.lr_schedule) for b in self._lr_base)
 
     # -- look-ahead -------------------------------------------------------------------------
     def submit_window(self, win_ids, own_ids=None):
@@ -604,9 +683,15 @@ class Trainer:
 
     # -- one training step -------------------------------------------------------------------
     def _step_eager(self, X, lS_o, lS_i, T):
+        dev_lr = self._lr_state is not None
+        if dev_lr and any(self.lr_schedule):
+            # first on the training stream: ahead of the lookup stream's fork, so the sparse update there reads it too
+            check(lib.cdlrm_lr_advance(self.dev.index, _vp(self._lr_state.data_ptr()),
+                                       _vp(torch.cuda.current_stream(self.dev).cuda_stream)))
         if self.overlap_update:
             self.cache_group.overlap_update = True
-            self.cache_group.fused_lr = float(self.optimizer_embeds.param_groups[0]["lr"])
+            self.cache_group.fused_lr = (self._lr_sparse if dev_lr
+                                         else float(self.optimizer_embeds.param_groups[0]["lr"]))
         lookups, _idxs = self.cache_group(lS_o, lS_i, self.emb_tables, self.dev.index)
         Z = self.dlrm(X, lookups)
         dz = None
@@ -639,7 +724,7 @@ class Trainer:
                     early.wait()
                 work.wait()
             self.dlrm.join_mlp_grads()        # weight-gradient GEMMs ran beside everything up to here
-            self.dlrm.flat_sgd_step(self.optimizer_mlps.param_groups[0]["lr"])
+            self.dlrm.flat_sgd_step(self._lr_dense if dev_lr else self.optimizer_mlps.param_groups[0]["lr"])
             return E, Z
         self.optimizer_mlps.zero_grad(set_to_none=True)
         E.backward()
@@ -671,6 +756,10 @@ class Trainer:
         return self._graph
 
     def step(self, X, lS_o, lS_i, T):
+        """One training step (a replay of the captured step when the shapes match).  ``param_groups[0]["lr"]`` of
+        ``optimizer_mlps`` / ``optimizer_embeds`` is the base learning rate: a change takes effect at this step, scaled
+        by the schedule (``lr_policy``)."""
+        self._sync_lr()
         self.steps_since_agg += 1
         self.global_step += 1
         self.steps_in_window += 1
@@ -895,7 +984,9 @@ class Trainer:
             "args": {"seed": int(a.numpy_rand_seed), "cache_size": int(a.cache_size), "ways": int(a.num_ways),
                      "lookahead": int(a.lookahead), "global_batch": int(a.mini_batch_size), "world_size": int(self.world),
                      "table_agg_op": a.table_agg_op, "average_on_writeback": bool(a.average_on_writeback),
-                     "learning_rate": float(a.learning_rate), "lr_embeds": float(a.lr_embeds)},
+                     "learning_rate": float(a.learning_rate), "lr_embeds": float(a.lr_embeds),
+                     "lr_num_warmup_steps": self.lr_schedule[0], "lr_decay_start_step": self.lr_schedule[1],
+                     "lr_num_decay_steps": self.lr_schedule[2]},
         }
 
     def save_checkpoint(self, path, epoch=0):
@@ -990,6 +1081,7 @@ class Trainer:
         r = meta["resume"]
         self.window = self._n_submitted = int(r["window"])
         self.global_step = int(r["global_step"])
+        self._set_lr_state()                        # the schedule goes on from the step count of the checkpoint
         self.resume_epoch = int(r["epoch"])
         self.last_checkpoint_s = {"host_to_device": round(h2d, 4), "file_io": round(rd.io_s, 4)}
         if self.world > 1:
@@ -1283,6 +1375,9 @@ def Run(rank, m_spa, ln_emb, ln_bot, ln_top, train_ld, test_ld, batch_fifo, evic
                 tr.capture_graph(X, lS_o, lS_i, T)           # after two eager steps (lazy initialisation)
             t1 = time.perf_counter()
             if strict:
+                if any(tr.lr_schedule):      # upstream steps its scheduler after every optimizer step
+                    for opt, b in ((tr.optimizer_mlps, args.learning_rate), (tr.optimizer_embeds, args.lr_embeds)):
+                        opt.param_groups[0]["lr"] = lr_policy(b, step_no + 1, *tr.lr_schedule)
                 E, Z, idxs = tr.step_reference(X, lS_o, lS_i, T)
                 if args.world_size > 1:
                     if j > 0 and j % args.table_agg_freq == 0:                       # :418-423
@@ -1380,6 +1475,11 @@ def _derive_topology(args):
     if num_int != ln_top[0]:
         sys.exit("ERROR: # of feature interactions " + str(num_int) + " does not match first dimension of top mlp "
                  + str(ln_top[0]))
+    W, D, N = args.lr_num_warmup_steps, args.lr_decay_start_step, args.lr_num_decay_steps
+    if min(W, D, N) < 0:
+        sys.exit("ERROR: --lr-num-warmup-steps, --lr-decay-start-step and --lr-num-decay-steps must not be negative")
+    if D < W:
+        sys.exit("ERROR: Learning rate warmup must finish before the decay starts")
     if args.qr_flag or args.md_flag:
         sys.exit("ERROR: QR / mixed-dimension embeddings are outside the cache hot path (unreachable from the "
                  "reference's own Run as well)")

@@ -159,7 +159,7 @@ class _LookupFn(torch.autograd.Function):
     """Autograd bridge: forward = cdlrm_embed_fwd, backward = de-duplicated sparse SGD
     (cdlrm_embed_bwd_plan + cdlrm_embed_bwd_sgd).  The update is applied when
     ``optimizer_embeds.step()`` runs (see ``_install_optimizer_hook``), or immediately
-    when ``group.fused_lr`` is set."""
+    when ``group.fused_lr`` is set (a float, or a one-element float32 CUDA tensor read when the kernel runs)."""
 
     @staticmethod
     def forward(ctx, anchor, group, ids, offsets, n_idx, n_bags, tb):
@@ -230,7 +230,9 @@ class Embedding_Table_Cache_Group(nn.Module):
         self.victim_cache_entries = [None] * len(self.emb_l)
         self.record_victims = False        # True: fill victim_cache_entries (costs a device sync)
         self.assume_one_id_per_bag = None  # None: check lS_o on the host when it is a CPU tensor
-        self.fused_lr = None               # set to apply the SGD update inside backward
+        self.fused_lr = None               # set to apply the SGD update inside backward: a float, or a float32 CUDA
+                                           # tensor of one element that the update reads on the device (Trainer's
+                                           # learning-rate state: a captured step follows its changes)
         self.early_plan = True             # build the backward plan during forward, on a side stream
         self.forward_stream = None         # set: lookup kernels run on this stream; consumers call join_forward()
         # with fused_lr and forward_stream set: the sparse update is launched from backward on forward_stream, behind
@@ -497,7 +499,7 @@ class Embedding_Table_Cache_Group(nn.Module):
     def _queue_update(self, tb, slots, bag_ids, n_idx, dbase, ld, rs, keep, plan=None):
         item = (tb, slots, bag_ids, n_idx, dbase, ld, rs, keep, plan)
         if self.fused_lr is not None:
-            self._apply_update(item, float(self.fused_lr))
+            self._apply_update(item, self.fused_lr)
             if self._upd_done is not None:
                 _GROUPS.add(self)
         else:
@@ -536,10 +538,13 @@ class Embedding_Table_Cache_Group(nn.Module):
             base = (self._plan_buf.data_ptr() + 255) // 256 * 256
             check(lib.cdlrm_embed_bwd_plan(self._ctx, tb, T, _vp(slots.data_ptr()), slots.stride(0), n_idx,
                                            _vp(base), s))
-        check(lib.cdlrm_embed_bwd_sgd(self._ctx, tb, T, _vp(base), n_idx,
-                                      _vp(bag_ids.data_ptr()) if bag_ids is not None else None,
-                                      bag_ids.stride(0) if bag_ids is not None else 0,
-                                      _vp(dbase.data_ptr()), ld, rs, lr, s))
+        bag = (_vp(bag_ids.data_ptr()) if bag_ids is not None else None, bag_ids.stride(0) if bag_ids is not None else 0)
+        if isinstance(lr, torch.Tensor):
+            check(lib.cdlrm_embed_bwd_sgd_dlr(self._ctx, tb, T, _vp(base), n_idx, *bag, _vp(dbase.data_ptr()), ld, rs,
+                                              _vp(lr.data_ptr()), s))
+        else:
+            check(lib.cdlrm_embed_bwd_sgd(self._ctx, tb, T, _vp(base), n_idx, *bag, _vp(dbase.data_ptr()), ld, rs,
+                                          float(lr), s))
         if us is not None:
             self._upd_done = torch.cuda.Event()
             self._upd_done.record(us)
@@ -992,19 +997,25 @@ class DLRM_Net(nn.Module):
         same launch also leaves the hi / lo operand copies of the UPDATED weights behind (cdlrm_mlp_sgd_split), so
         that the next forward of either MLP starts with its first GEMM instead of a split launch.  Dense parameters
         changed by anything else afterwards (``.data.copy_``) need ``invalidate_weight_splits()``;
-        ``load_state_dict`` and ``.to()`` do it themselves."""
+        ``load_state_dict`` and ``.to()`` do it themselves.  ``lr``: a float, or a one-element float32 CUDA tensor that
+        the kernel reads when it runs (fused path only: cdlrm_mlp_sgd_split_dlr)."""
         sts = [self._mlp_state.get("bot"), self._mlp_state.get("top")]
         if (self.mlp_impl == "tcgen05" and self.fused_sgd_split
                 and all(st is not None and st.handle is not None for st in sts)):
             lin = [m for st in sts for m in st.linears]
             n_w = self.flat_weight_elems
-            check(lib.cdlrm_mlp_sgd_split(
+            dev_lr = isinstance(lr, torch.Tensor)
+            check((lib.cdlrm_mlp_sgd_split_dlr if dev_lr else lib.cdlrm_mlp_sgd_split)(
                 2, _lib.ptr_array([st.handle.value for st in sts]),
                 _lib.ptr_array([m.weight.data_ptr() for m in lin]),
-                _lib.ptr_array([g.data_ptr() for st in sts for g in st.flat_grads[0]]), float(lr),   # views of the bucket
+                _lib.ptr_array([g.data_ptr() for st in sts for g in st.flat_grads[0]]),   # views of the bucket
+                _vp(lr.data_ptr()) if dev_lr else float(lr),
                 _vp(self.flat_params.data_ptr() + 4 * n_w), _vp(self.flat_grads.data_ptr() + 4 * n_w),
                 self.flat_params.numel() - n_w, _stream_ptr(self.flat_params.device)))
             return
+        if isinstance(lr, torch.Tensor):
+            raise _lib.CdlrmError("flat_sgd_step: a device learning rate needs the fused SGD + split "
+                                  "(tcgen05 MLPs, CDLRM_SGD_SPLIT=1)")
         self.flat_params.add_(self.flat_grads, alpha=-float(lr))
 
     def invalidate_weight_splits(self):

@@ -121,6 +121,14 @@ int cdlrm_embed_bwd_sgd(cdlrm_ctx* ctx, int table_begin, int table_count,
                         const int32_t* bag_ids, int64_t ld_bag,
                         const float* d_out, int64_t ld_dout, int64_t dout_row_stride,
                         float lr, cdlrm_stream stream);
+/* The same update with the learning rate read from device memory when the kernels run (*d_lr, one float: a
+ * cdlrm_lr_state's lr[1]), so that a CUDA graph replays whatever value the buffer holds; equal bit for bit to
+ * cdlrm_embed_bwd_sgd with lr = *d_lr. */
+int cdlrm_embed_bwd_sgd_dlr(cdlrm_ctx* ctx, int table_begin, int table_count,
+                            const void* plan, int32_t n_idx,
+                            const int32_t* bag_ids, int64_t ld_bag,
+                            const float* d_out, int64_t ld_dout, int64_t dout_row_stride,
+                            const float* d_lr, cdlrm_stream stream);
 
 /* ---- interaction: DLRM_Net.interact_features ("dot"), model_no_ddp.py:272-293 ---
  * feat[0] = x, feat[1..] = ly; h_feat is a host array of n_feat device pointers to
@@ -177,6 +185,10 @@ int cdlrm_mlp_set_option(int key, int value);
  * (cdlrm_mlp_invalidate_split otherwise). */
 int cdlrm_mlp_sgd_split(int n_mlps, cdlrm_mlp* const* mlps, float* const* h_W, const float* const* h_dW, float lr,
                         float* vec, const float* vec_grad, int64_t vec_n, cdlrm_stream stream);
+/* The same step with the learning rate read from device memory when the kernel runs (*d_lr: a cdlrm_lr_state's
+ * lr[0]); equal bit for bit to cdlrm_mlp_sgd_split with lr = *d_lr. */
+int cdlrm_mlp_sgd_split_dlr(int n_mlps, cdlrm_mlp* const* mlps, float* const* h_W, const float* const* h_dW,
+                            const float* d_lr, float* vec, const float* vec_grad, int64_t vec_n, cdlrm_stream stream);
 int cdlrm_mlp_invalidate_split(cdlrm_mlp* mlp);
 int cdlrm_mlp_set_defer_join(cdlrm_mlp* mlp, int on);
 int cdlrm_mlp_join(cdlrm_mlp* mlp, cdlrm_stream stream);
@@ -187,6 +199,31 @@ int cdlrm_mlp_forward(cdlrm_mlp* mlp, const float* x, int64_t ldx, int32_t batch
                       float* y, int64_t ldy, cdlrm_stream stream);
 int cdlrm_mlp_backward(cdlrm_mlp* mlp, const float* dy, int64_t lddy, float* dx, int64_t lddx,
                        float* const* h_dW, float* const* h_db, cdlrm_stream stream);
+
+/* ---- learning-rate schedule: upstream DLRM's LRPolicyScheduler (dlrm_s_pytorch.py, --lr-num-warmup-steps W,
+ *      --lr-decay-start-step D, --lr-num-decay-steps N), evaluated on the device --------------------------------
+ * A caller-owned device buffer holds the learning rates of the current step, which the *_dlr update entry points
+ * read, so that a captured training step follows the schedule and host-side changes of the base on replay.
+ * For base b and the 1-based step count c, in fp64 rounded to fp32 once:
+ *   c < W                    b * (1 - (W - c) / W)                               (warmup)
+ *   D <= c < D + N           max(1e-7, b * x * x),  x = (N - (c - D)) / N         (decay)
+ *   otherwise, N == 0        b
+ *   otherwise, c >= D + N    the value at c = D + N - 1
+ *   otherwise, W >= 2        the value at c = W - 1  (held between warmup and decay, as upstream does)
+ *   otherwise                b */
+typedef struct cdlrm_lr_state {
+    float lr[2];                 /* [dense, sparse]: learning rates of the current step (step count `count`) */
+    double base[2];              /* [dense, sparse]: base learning rates b */
+    int64_t warmup_steps, decay_start_step, decay_steps;   /* W, D, N */
+    int64_t count;               /* steps run so far */
+} cdlrm_lr_state;
+/* Writes bases, schedule and count, and lr[g] = lr(count) for both groups: with W = D = N = 0 that is fp32(base),
+ * and nothing else needs to run per step.  A one-thread kernel in stream order (no host-to-device copy, which could
+ * queue behind bulk copies on the copy engine).  Refuses W, D or N negative, D < W, a negative count. */
+int cdlrm_lr_set(int device, cdlrm_lr_state* d_state, double base_dense, double base_sparse, int64_t warmup_steps,
+                 int64_t decay_start_step, int64_t decay_steps, int64_t count, cdlrm_stream stream);
+/* One step: count += 1, lr[g] = lr(count).  Capturable; launched at the start of every step when a schedule is set. */
+int cdlrm_lr_advance(int device, cdlrm_lr_state* d_state, cdlrm_stream stream);
 
 /* ---- window planner: Prefetcher.process_batch_slice (cache_manager.py:27-46, the
  *      torch.unique at :32) + the decision part of CacheEmbeddings
