@@ -39,6 +39,11 @@ SIGNATURES = {
                                       C.c_int64, C.c_float, vp]),
     "cdlrm_embed_bwd_sgd_dlr": (C.c_int, [vp, C.c_int, C.c_int, vp, C.c_int32, vp, C.c_int64, vp, C.c_int64,
                                           C.c_int64, vp, vp]),
+    "cdlrm_embed_victim_update": (C.c_int, [vp, C.c_int, C.c_int, vp, C.c_int64, vp, C.c_int64, C.c_int32, vp,
+                                            C.c_int64, vp, C.c_int64, C.c_int64, C.c_float, vp]),
+    "cdlrm_embed_victim_update_dlr": (C.c_int, [vp, C.c_int, C.c_int, vp, C.c_int64, vp, C.c_int64, C.c_int32, vp,
+                                                C.c_int64, vp, C.c_int64, C.c_int64, vp, vp]),
+    "cdlrm_move_carry_losers": (C.c_int, [vp, C.c_int, vp, C.c_int64, vp, vp]),
     "cdlrm_embed_set_option": (C.c_int, [C.c_int, C.c_int]),
     "cdlrm_interact_set_option": (C.c_int, [C.c_int, C.c_int]),
     "cdlrm_interact_fwd": (C.c_int, [C.c_int, C.POINTER(vp), C.c_int, C.c_int64, C.c_int32, C.c_int, C.c_int,

@@ -199,6 +199,11 @@ class WindowPlanner:
         self._ce_no = 0
         self._ce_ev = None
         self._pending_wb = None          # ce: (record, average) of the boundary whose evicted rows are not yet written back
+        # --evict-victim-cache: the loser store of the installed window is trained in place (cdlrm_embed_victim_update);
+        # at the next boundary its rows are carried into the next window's prefetched rows and written back to the master
+        self.evict_victim_cache = False
+        self._bound = None               # record whose loser store is bound (installed window)
+        self._pending_store = None       # ce: record whose store rows are not yet written back
         self._shard = None               # (rank, world, host process group): loser store sharded over the node
         self._fill_shard = None          # (rank, world, host process group): fill prefetch sharded over the node
         self._peer_bufs = {}             # name -> (capacity rows, [device address of every rank's shard buffer])
@@ -478,6 +483,12 @@ class WindowPlanner:
                 # master (fwd_miss_kernel falls back when the binary search misses) -- same rows either way
                 tot = sum(rec.L)
                 cap_rows = self._agreed_loser_cap()
+                if tot > cap_rows and self.evict_victim_cache:
+                    # the misses served from the master would be trained nowhere, and race with the next prefetch
+                    raise _lib.CdlrmError(
+                        "--evict-victim-cache needs the whole loser store of a window in HBM: this window needs %.2f GB, "
+                        "the budget is %.2f GB (raise CDLRM_LOSER_STORE_GB, or shrink --lookahead)"
+                        % (tot * 4 * self.dim / 1e9, cap_rows * 4 * self.dim / 1e9))
                 if tot > cap_rows:
                     rec.L = [int(x * cap_rows // tot) for x in rec.L]
             self.last_timing = {"phase_a_s": round(t_b - t_a, 4), "rng_s": round(t_c - t_b, 4),
@@ -566,6 +577,9 @@ class WindowPlanner:
         """ce mode: write the evicted rows of the last installed window back into the host master (device -> pinned
         chunk by the copy engine, chunk -> master rows by host threads).  Called from the thread that plans the next
         window, before anything of that window reads the master; a no-op when nothing is pending."""
+        store, self._pending_store = self._pending_store, None
+        if store is not None:
+            self._write_store(store, ce=True)
         pend, self._pending_wb = self._pending_wb, None
         if pend is None:
             return
@@ -599,6 +613,40 @@ class WindowPlanner:
                 _vp(bufs[0].data_ptr()), _vp(bufs[1].data_ptr()), rows_per, int(average), self.host_threads, _sp(s)))
         rec.wb_done = torch.cuda.Event(enable_timing=True)
         rec.wb_done.record(s)
+
+    def _write_store(self, rec, ce):
+        """master[k][id] = the store row of id, for every id of the loser store of ``rec``: a plain write (the row is the
+        master row plus this window's updates), on the planner's stream.  ``ce``: copy engine + host threads
+        (cdlrm_host_writeback_rows, returns when the rows are in the master); else zero-copy scatter kernels."""
+        ks = [k for k in range(self.T) if rec.L[k]]
+        if not ks:
+            return
+        s = self.stream
+        if not ce:
+            with torch.cuda.stream(s):
+                for k in ks:
+                    check(lib.cdlrm_move_scatter_master2(self.ctx, k, _vp(rec.loser_ids[rec.loser_off[k]:].data_ptr()), None,
+                                                         rec.L[k], _vp(rec.loser_stage[rec.loser_soff[k]:].data_ptr()), 0,
+                                                         _sp(s)))
+            return
+        hid, offs = self._ids_to_host("store_ids", rec.loser_ids, [(rec.loser_off[k], rec.L[k]) for k in ks])
+        rows_per, bufs, _evs = self._ce_chunks()
+        Ws = [self.emb_tables.emb_l[k].weight.data for k in ks]
+        check(lib.cdlrm_host_writeback_rows(
+            self.dev.index, len(ks), _lib.ptr_array([W.data_ptr() for W in Ws]), _lib.i64_array([W.shape[0] for W in Ws]),
+            self.dim, _lib.ptr_array([hid.data_ptr() + 8 * o for o in offs]), None, _lib.i64_array([rec.L[k] for k in ks]),
+            _lib.ptr_array([rec.loser_stage[rec.loser_soff[k]:].data_ptr() for k in ks]),
+            _vp(bufs[0].data_ptr()), _vp(bufs[1].data_ptr()), rows_per, 0, self.host_threads, _sp(s)))
+
+    def write_store_to_master(self):
+        """--evict-victim-cache: write the rows of the installed window's loser store into the master now (they are
+        also the rows its next boundary carries and writes back, so this changes nothing that follows).  Runs after
+        the current stream's work; returns when the rows are in the master."""
+        if not self.evict_victim_cache or self._bound is None:
+            return
+        self.stream.wait_stream(torch.cuda.current_stream(self.dev))
+        self._write_store(self._bound, ce=self.pcie_mode == "ce" and not self.emb_tables.emb_l[0].weight.is_cuda)
+        self.stream.synchronize()
 
     # -- export of the cached rows into the master ----------------------------------------------------
     # HBM staging of a copy-engine export, in rows of the grow-only "evict" buffer: the list is packed and written back
@@ -756,6 +804,8 @@ class WindowPlanner:
             n_fill = max(sum(rec.F), 1)
             self._pinned("wb_ids", 8 * n_fill)
             self._pinned("wb_prim", n_fill)
+            if self.evict_victim_cache and rec.L is not None:
+                self._pinned("store_ids", 8 * max(sum(rec.L), 1))     # this store's write-back, two boundaries on
             self._ce_chunks()
             for name, ids_dev, jobs in (("fill_ids", rec.fill_ids, fill_jobs), ("loser_ids", rec.loser_ids, loser_jobs)):
                 if jobs:
@@ -802,6 +852,18 @@ class WindowPlanner:
                                                _vp(prim.data_ptr()), rec.E[k],
                                                _vp(rec.evict_stage[eoff[k]:].data_ptr()), 0, 0, _sp(s)))
             tm.append(time.perf_counter())
+            if self.evict_victim_cache and self._bound is not None:
+                # the bound store is still the finished window's: ids it trained are prefetched stale in this window's
+                # fill and loser rows (gathered from the master while it trained); its rows replace them
+                for k in range(self.T):
+                    if rec.F[k]:
+                        check(lib.cdlrm_move_carry_losers(self.ctx, k, _vp(rec.fill_ids[rec.off[k]:].data_ptr()), rec.F[k],
+                                                          _vp(rec.fill_stage[rec.fill_soff[k]:].data_ptr()), _sp(s)))
+                    if rec.L is not None and rec.L[k]:
+                        check(lib.cdlrm_move_carry_losers(self.ctx, k, _vp(rec.loser_ids[rec.loser_off[k]:].data_ptr()),
+                                                          rec.L[k], _vp(rec.loser_stage[rec.loser_soff[k]:].data_ptr()),
+                                                          _sp(s)))
+            tm.append(time.perf_counter())
             for k in range(self.T):
                 if rec.F[k] and rec.fill_peers is not None:
                     # share r of the list comes out of rank r's staging buffer (local HBM or NVLink peer memory)
@@ -840,6 +902,15 @@ class WindowPlanner:
         tm.append(time.perf_counter())
         ws = self.stream
         ws.wait_event(moved)       # later planner-stream work (next prefetch) may reuse the staging buffers
+        prev, self._bound = self._bound, (rec if rec.L is not None else None)
+        if self.evict_victim_cache and prev is not None and write_master:
+            # the finished window's store goes back to the master before anything of the window after next reads it:
+            # ce by the next flush_writeback (the plan thread, before its plan); sm right here on the planner stream.
+            # Its buffers are the ones the next stage() fills: both come after this in planner-stream order
+            if self.pcie_mode == "ce" and not self.emb_tables.emb_l[0].weight.is_cuda:
+                self._pending_store = prev
+            else:
+                self._write_store(prev, ce=False)
         if write_master and sum(rec.wb_n) and self.pcie_mode == "ce" and not self.emb_tables.emb_l[0].weight.is_cuda:
             # copy engine + host threads: done by the thread that plans the next window (flush_writeback), before
             # anything of that window reads the master; callers that read the master themselves call it first
@@ -859,7 +930,8 @@ class WindowPlanner:
         rec.wb_done.record(self.stream)
         tm.append(time.perf_counter())
         self.last_install_ms = {n: round(1e3 * (y - x), 2) for n, x, y in
-                                zip(("wait_and_buffers", "evict_launches", "fill_launches", "bind_losers", "writeback_launches"),
+                                zip(("wait_and_buffers", "evict_launches", "carry_launches", "fill_launches", "bind_losers",
+                                     "writeback_launches"),
                                     tm, tm[1:])}
         return rec
 

@@ -44,13 +44,14 @@ def read_meta(path):
 
 # fields added after checkpoints were first written, with the value every older checkpoint was trained with
 _ADDED_DEFAULTS = {("args", "lr_num_warmup_steps"): 0, ("args", "lr_decay_start_step"): 0,
-                   ("args", "lr_num_decay_steps"): 0}
+                   ("args", "lr_num_decay_steps"): 0, ("args", "evict_victim_cache"): False}
 
 
 def check_meta(saved, expected):
     """Raise ``CheckpointMismatch`` naming the first field of ``expected`` ("format", "shapes.*", "args.*") that the
     saved meta data does not hold with the same value.  A field missing from the saved meta data is a mismatch, except
-    the learning-rate schedule (``args.lr_*``: a checkpoint written before it existed was trained without one)."""
+    the learning-rate schedule (``args.lr_*``: a checkpoint written before it existed was trained without one) and
+    ``args.evict_victim_cache`` (false: written before the flag was implemented)."""
     if saved.get("format") != expected["format"]:
         raise CheckpointMismatch("checkpoint field format: saved %r, this trainer reads %r"
                                  % (saved.get("format"), expected["format"]))

@@ -124,7 +124,8 @@ enum KernelId {
     K_PROBE = 0, K_GATHER, K_POOL, K_BWD_PLAN, K_BWD_SGD, K_BWD_SGD_MULTI, K_INT_FWD, K_INT_BWD,
     K_PLAN_BITMAP_SET, K_PLAN_COMPACT, K_PLAN_PROBE, K_PLAN_SURV, K_PLAN_SELECT, K_PLAN_LISTS,
     K_MOVE_EVICT, K_MOVE_GATHER, K_MOVE_FILL, K_MOVE_SCATTER, K_AGG_MARK, K_AGG_OR, K_AGG_COLLECT,
-    K_AGG_PACK, K_AGG_UNPACK, K_MISC, K_RNG_MT, K_RNG_EXP, K_MLP_GEMM, K_MLP_SPLIT, K_EMBED_EVAL, K_EVAL, K_LR, K_NULL, K_COUNT
+    K_AGG_PACK, K_AGG_UNPACK, K_MISC, K_RNG_MT, K_RNG_EXP, K_MLP_GEMM, K_MLP_SPLIT, K_EMBED_EVAL, K_EVAL, K_LR, K_NULL,
+    K_EMBED_VICTIM, K_MOVE_CARRY, K_COUNT
 };
 void cdlrm_prof_mark(int id, cudaStream_t s, int end);
 // wraps one kernel launch statement
@@ -191,6 +192,32 @@ inline void cdlrm_launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, si
         cdlrm_launch_pdl(kern, dim3(grid), dim3(block), (smem), (stream), __VA_ARGS__); \
         cdlrm_prof_mark((id), (stream), 1);                                            \
     } while (0)
+
+// Index of `id` in the ascending ids of a loser store (bucket index, then binary search), or -1 when the store does
+// not hold it.
+__device__ __forceinline__ int64_t loser_index(const LoserDesc* __restrict__ L, int64_t id) {
+    const int64_t n = L->n;
+    int64_t lo = 0, hi = n;                // first index with ids[idx] >= id
+    if (L->bucket) {                       // bucket index: the answer lies in [bucket[b], bucket[b + 1]]
+        const int64_t bk = id >> L->shift;
+        lo = __ldg(L->bucket + bk);
+        hi = __ldg(L->bucket + bk + 1);
+    }
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (__ldg(L->ids + mid) < id) lo = mid + 1; else hi = mid;
+    }
+    return (lo < n && __ldg(L->ids + lo) == id) ? lo : -1;
+}
+
+// Row `idx` of a loser store: local HBM, or (sharded store) the HBM of rank idx / shard over NVLink.
+__device__ __forceinline__ const float* loser_row(const LoserDesc* __restrict__ L, int64_t idx, int dim) {
+    if (L->shard) {
+        const int64_t owner = idx / L->shard;
+        return L->peer[owner] + (idx - owner * L->shard) * dim;
+    }
+    return L->rows + idx * dim;
+}
 
 __device__ __forceinline__ int64_t set_index(int64_t id, int64_t S) {
     // torch.remainder semantics (non-negative result for S > 0)

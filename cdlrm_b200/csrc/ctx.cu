@@ -261,7 +261,7 @@ static const char* const g_knames[K_COUNT] = {
     "plan_bitmap_set", "plan_compact", "plan_probe", "plan_surv", "plan_select", "plan_lists",
     "move_evict", "move_gather", "move_fill", "move_scatter", "agg_mark", "agg_or", "agg_collect",
     "agg_pack", "agg_unpack", "misc", "rng_mt19937", "rng_exp", "mlp_gemm", "mlp_split", "embed_fwd_eval", "eval_metrics",
-    "lr_schedule", "null"};
+    "lr_schedule", "null", "embed_victim", "move_carry"};
 
 void cdlrm_prof_mark(int id, cudaStream_t s, int end) {
     if (!end) g_launches.fetch_add(1, std::memory_order_relaxed);

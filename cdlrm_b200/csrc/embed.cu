@@ -98,24 +98,8 @@ __device__ __forceinline__ int64_t probe_slot(const TableDesc& T, int64_t id, in
 __device__ __forceinline__ const float* miss_row(const LoserDesc* __restrict__ L, const float* __restrict__ master,
                                                  int64_t id, int dim) {
     if (L) {
-        const int64_t n = L->n;
-        int64_t lo = 0, hi = n;                // first index with ids[idx] >= id
-        if (L->bucket) {                       // bucket index: the answer lies in [bucket[b], bucket[b + 1]]
-            const int64_t bk = id >> L->shift;
-            lo = __ldg(L->bucket + bk);
-            hi = __ldg(L->bucket + bk + 1);
-        }
-        while (lo < hi) {
-            const int64_t mid = (lo + hi) >> 1;
-            if (__ldg(L->ids + mid) < id) lo = mid + 1; else hi = mid;
-        }
-        if (lo < n && __ldg(L->ids + lo) == id) {
-            if (L->shard) {                    // sharded store: the row is in the HBM of rank lo / shard (NVLink)
-                const int64_t owner = lo / L->shard;
-                return L->peer[owner] + (lo - owner * L->shard) * dim;
-            }
-            return L->rows + lo * dim;         // local HBM
-        }
+        const int64_t idx = loser_index(L, id);
+        if (idx >= 0) return loser_row(L, idx, dim);
     }
     return master + id * dim;
 }
@@ -861,6 +845,118 @@ __global__ void __launch_bounds__(256) bwd_sgd_kernel(const TableDesc* __restric
     if (gl == 0 && T.dirty) atomicOr(T.dirty + (slot >> 5), 1u << (slot & 31));
 }
 
+// ------------------------------------------------------------------------------
+// Update of the misses (--evict-victim-cache): a miss of the step is a position whose slot is an aux slot; its row
+// came from the loser store of the installed window, and its sparse update goes into that store row, not only into
+// the aux row the next forward overwrites.  Per table and store row: the gradient rows of every position that
+// missed on it, summed in ascending position, then ONE weight = fma(-lr, sum, weight) -- what bwd_sgd_apply_kernel
+// does for a cached slot.  Duplicate misses of an id sit in separate aux slots and are summed once.
+// CTA c of a table owns the ids whose hash is c (mod gridDim.x), so every store row has one owner CTA: it keeps its
+// misses as keys (store index << 32 | position) in shared memory, sorts them (bitonic: the keys are distinct), and
+// its warps walk the runs of equal store index, one float4 column per lane, U runs in flight.
+// A miss whose id is not in the store raises flag 4 (cdlrm_ctx_check) and is not applied.
+// ------------------------------------------------------------------------------
+constexpr int VICTIM_NT = 512;
+
+template <int VEC, bool DLR>
+__global__ void __launch_bounds__(VICTIM_NT) victim_update_kernel(const TableDesc* __restrict__ tabs, int tb,
+                                                                  const LoserDesc* __restrict__ losers,
+                                                                  const int32_t* __restrict__ slots, int64_t ld_slots,
+                                                                  const int64_t* __restrict__ ids, int64_t ld_ids,
+                                                                  int n_idx, const int32_t* __restrict__ bag_ids,
+                                                                  int64_t ld_bag, const float* __restrict__ d_out,
+                                                                  int64_t ld_dout, int64_t row_stride, float lr_arg,
+                                                                  const float* __restrict__ d_lr, int dim, int ways,
+                                                                  int cap, uint32_t* __restrict__ flags) {
+    pdl_enter();
+    using V = typename VecT<VEC>::type;
+    extern __shared__ __align__(16) unsigned long long s_key[];
+    __shared__ int s_n;
+    const int t = blockIdx.y, C = gridDim.x;
+    const TableDesc& T = tabs[tb + t];
+    const LoserDesc* __restrict__ L = losers ? losers + tb + t : nullptr;
+    const int64_t aux_base = T.num_sets * ways;
+    if (threadIdx.x == 0) s_n = 0;
+    __syncthreads();
+    const int32_t* tsl = slots + (int64_t)t * ld_slots;
+    const int64_t* tid = ids + (int64_t)t * ld_ids;
+    for (int j = threadIdx.x; j < n_idx; j += VICTIM_NT) {
+        const int64_t sl = tsl[j];
+        if (sl < aux_base || sl >= T.cache_rows) continue;       // cached, or unresolved (slot -1, flagged by the forward)
+        const int64_t id = tid[j];
+        if ((int)((((uint64_t)id * 0x9E3779B97F4A7C15ull) >> 32) % (uint64_t)C) != (int)blockIdx.x) continue;
+        const int64_t li = (L && !L->shard) ? loser_index(L, id) : -1;
+        if (li < 0) {
+            atomicOr(flags, 4u);
+            continue;
+        }
+        const int e = atomicAdd(&s_n, 1);
+        if (e < cap) s_key[e] = ((unsigned long long)li << 32) | (uint32_t)j;
+    }
+    __syncthreads();
+    const int n = min(s_n, cap);
+    if (n == 0) return;
+    int kp = 1;
+    while (kp < n) kp <<= 1;
+    for (int i = n + threadIdx.x; i < kp; i += VICTIM_NT) s_key[i] = ~0ull;
+    __syncthreads();
+    for (int size = 2; size <= kp; size <<= 1) {
+        for (int stride = size >> 1; stride > 0; stride >>= 1) {
+            for (int i = threadIdx.x; i < (kp >> 1); i += VICTIM_NT) {
+                const int lo = 2 * i - (i & (stride - 1)), hi = lo + stride;
+                const unsigned long long a = s_key[lo], b = s_key[hi];
+                if ((a > b) == ((lo & size) == 0)) { s_key[lo] = b; s_key[hi] = a; }
+            }
+            __syncthreads();
+        }
+    }
+    const float lr = load_lr<DLR>(lr_arg, d_lr);
+    float* __restrict__ rows = const_cast<float*>(L->rows);
+    const float* __restrict__ gbase = d_out + (int64_t)t * ld_dout;
+    const int32_t* __restrict__ tbag = bag_ids ? bag_ids + (int64_t)t * ld_bag : nullptr;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int cpr = dim / VEC;
+    constexpr int U = 4;
+    for (int base = warp * 32; base < n; base += VICTIM_NT) {
+        const int e = base + lane;
+        const unsigned long long k = e < n ? s_key[e] : ~0ull;
+        const unsigned long long kprev = (e > 0 && e < n) ? s_key[e - 1] : ~0ull;
+        uint32_t heads = __ballot_sync(0xffffffffu, e < n && (k >> 32) != (kprev >> 32));
+        while (heads) {
+            int h[U];
+#pragma unroll
+            for (int u = 0; u < U; ++u) {
+                h[u] = heads ? base + __ffs(heads) - 1 : -1;
+                if (heads) heads &= heads - 1;
+            }
+            for (int c = lane; c < cpr; c += 32) {
+                V acc[U], wv[U];
+#pragma unroll
+                for (int u = 0; u < U; ++u) {
+                    if (h[u] < 0) continue;
+                    const unsigned long long kh = s_key[h[u]];
+                    const int p = tbag ? tbag[(uint32_t)kh] : (int)(uint32_t)kh;
+                    vzero(acc[u]);
+                    acc[u] = vadd(acc[u], reinterpret_cast<const V*>(gbase + (int64_t)p * row_stride)[c]);
+                    wv[u] = reinterpret_cast<const V*>(rows + (int64_t)(kh >> 32) * dim)[c];
+                }
+#pragma unroll
+                for (int u = 0; u < U; ++u) {
+                    if (h[u] < 0) continue;
+                    const unsigned long long li = s_key[h[u]] >> 32;
+                    for (int x = h[u] + 1; x < n; ++x) {
+                        const unsigned long long kx = s_key[x];
+                        if ((kx >> 32) != li) break;
+                        const int p = tbag ? tbag[(uint32_t)kx] : (int)(uint32_t)kx;
+                        acc[u] = vadd(acc[u], reinterpret_cast<const V*>(gbase + (int64_t)p * row_stride)[c]);
+                    }
+                    reinterpret_cast<V*>(rows + (int64_t)li * dim)[c] = vfma(-lr, acc[u], wv[u]);
+                }
+            }
+        }
+    }
+}
+
 inline int pow2_ceil(int v) {
     int p = 1;
     while (p < v) p <<= 1;
@@ -1134,4 +1230,59 @@ extern "C" int cdlrm_embed_bwd_sgd_dlr(cdlrm_ctx* c, int tb, int tc, const void*
                                        const int32_t* bag_ids, int64_t ld_bag, const float* d_out, int64_t ld_dout,
                                        int64_t row_stride, const float* d_lr, cdlrm_stream stream) {
     return bwd_sgd_launch<true>(c, tb, tc, plan, n_idx, bag_ids, ld_bag, d_out, ld_dout, row_stride, 0.f, d_lr, stream);
+}
+
+template <bool DLR>
+static int victim_launch(cdlrm_ctx* c, int tb, int tc, const int32_t* slots, int64_t ld_slots, const int64_t* ids,
+                         int64_t ld_ids, int32_t n_idx, const int32_t* bag_ids, int64_t ld_bag, const float* d_out,
+                         int64_t ld_dout, int64_t row_stride, float lr, const float* d_lr, cdlrm_stream stream) {
+    ARG_CHECK(c && slots && ids && d_out);
+    ARG_CHECK(tb >= 0 && tc > 0 && tb + tc <= c->T && n_idx >= 0);
+    ARG_CHECK(!DLR || d_lr);
+    // misses of a table: at most one per aux row and one per position; one CTA may have to hold all of them
+    const int64_t cap = c->aux < n_idx ? c->aux : n_idx;
+    if (cap == 0) return CDLRM_OK;
+    if (cap > CDLRM_SORT_MAX) {
+        cdlrm_set_error("cdlrm_embed_victim_update: up to %d misses per table (aux rows and ids per table), got %lld",
+                        CDLRM_SORT_MAX, (long long)cap);
+        return CDLRM_ERR_ARG;
+    }
+    cudaStream_t s = (cudaStream_t)stream;
+    CU_CHECK(cudaSetDevice(c->device));
+    int rc = cdlrm_sync_tabs(c, s);
+    if (rc) return rc;
+    const int vec = pick_vec(c->dim, d_out, nullptr, ld_dout, row_stride);
+    const int smem = pow2_ceil((int)cap) * (int)sizeof(unsigned long long);
+    int C = n_idx / 512;                   // CTAs per table: ids are spread over them by hash
+    C = C < 1 ? 1 : (C > 16 ? 16 : C);
+    const dim3 grid(C, tc);
+#define LAUNCH_VICTIM(VV)                                                                                            \
+    do {                                                                                                             \
+        CU_CHECK(cdlrm_smem_optin((const void*)victim_update_kernel<VV, DLR>, smem));                                \
+        LAUNCH_PDL(K_EMBED_VICTIM, s, (victim_update_kernel<VV, DLR>), grid, VICTIM_NT, smem, c->d_tabs, tb,       \
+                   c->d_losers, slots, ld_slots, ids, ld_ids, n_idx, bag_ids, ld_bag, d_out, ld_dout, row_stride, lr, \
+                   d_lr, c->dim, c->ways, (int)cap, c->d_flags);                                                     \
+    } while (0)
+    if (vec == 4) LAUNCH_VICTIM(4);
+    else if (vec == 2) LAUNCH_VICTIM(2);
+    else LAUNCH_VICTIM(1);
+#undef LAUNCH_VICTIM
+    CU_CHECK(cudaGetLastError());
+    return CDLRM_OK;
+}
+
+extern "C" int cdlrm_embed_victim_update(cdlrm_ctx* c, int tb, int tc, const int32_t* slots, int64_t ld_slots,
+                                         const int64_t* ids, int64_t ld_ids, int32_t n_idx, const int32_t* bag_ids,
+                                         int64_t ld_bag, const float* d_out, int64_t ld_dout, int64_t row_stride,
+                                         float lr, cdlrm_stream stream) {
+    return victim_launch<false>(c, tb, tc, slots, ld_slots, ids, ld_ids, n_idx, bag_ids, ld_bag, d_out, ld_dout,
+                                row_stride, lr, nullptr, stream);
+}
+
+extern "C" int cdlrm_embed_victim_update_dlr(cdlrm_ctx* c, int tb, int tc, const int32_t* slots, int64_t ld_slots,
+                                             const int64_t* ids, int64_t ld_ids, int32_t n_idx, const int32_t* bag_ids,
+                                             int64_t ld_bag, const float* d_out, int64_t ld_dout, int64_t row_stride,
+                                             const float* d_lr, cdlrm_stream stream) {
+    return victim_launch<true>(c, tb, tc, slots, ld_slots, ids, ld_ids, n_idx, bag_ids, ld_bag, d_out, ld_dout,
+                               row_stride, 0.f, d_lr, stream);
 }

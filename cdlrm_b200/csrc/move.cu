@@ -314,6 +314,44 @@ extern "C" int cdlrm_ctx_bind_losers(cdlrm_ctx* c, const int64_t* const* h_ids, 
     return launch_loser_buckets(c, h, s);
 }
 
+// Boundary carry (--evict-victim-cache): rows[i] = the bound loser store's row of ids[i] when the store holds ids[i].
+// The next window's fill and loser rows were prefetched from the master while this window trained its store rows.
+template <int VEC>
+__global__ void __launch_bounds__(256) carry_kernel(const LoserDesc* __restrict__ L, const int64_t* __restrict__ ids,
+                                                    int64_t n, float* __restrict__ rows, int dim, int G) {
+    using V = typename VT<VEC>::type;
+    const int gl = threadIdx.x % G, group = threadIdx.x / G, NG = blockDim.x / G;
+    const int cpr = dim / VEC;
+    for (int64_t i = (int64_t)blockIdx.x * NG + group; i < n; i += (int64_t)gridDim.x * NG) {
+        const int64_t li = loser_index(L, ids[i]);
+        if (li < 0) continue;
+        const V* src = reinterpret_cast<const V*>(loser_row(L, li, dim));
+        V* dst = reinterpret_cast<V*>(rows + i * dim);
+        for (int c = gl; c < cpr; c += G) dst[c] = src[c];
+    }
+}
+
+extern "C" int cdlrm_move_carry_losers(cdlrm_ctx* c, int k, const int64_t* ids, int64_t n, float* rows_inout,
+                                       cdlrm_stream stream) {
+    ARG_CHECK(c && k >= 0 && k < c->T && n >= 0);
+    if (n == 0 || !c->d_losers) return CDLRM_OK;         // nothing to copy, or no store was ever bound
+    ARG_CHECK(ids && rows_inout);
+    cudaStream_t s = (cudaStream_t)stream;
+    CU_CHECK(cudaSetDevice(c->device));
+    const int vec = vec_for(c->dim, rows_inout, nullptr);
+    const int cpr = c->dim / vec;
+    const int G = pow2_ceil(cpr) > 32 ? 32 : pow2_ceil(cpr);
+    const int NG = 256 / G;
+    int64_t blocks = (n + NG - 1) / NG;
+    if (blocks > (int64_t)c->num_sms * 16) blocks = (int64_t)c->num_sms * 16;
+    const LoserDesc* L = c->d_losers + k;
+    if (vec == 4) LAUNCH(K_MOVE_CARRY, s, (carry_kernel<4><<<(int)blocks, 256, 0, s>>>(L, ids, n, rows_inout, c->dim, G)));
+    else if (vec == 2) LAUNCH(K_MOVE_CARRY, s, (carry_kernel<2><<<(int)blocks, 256, 0, s>>>(L, ids, n, rows_inout, c->dim, G)));
+    else LAUNCH(K_MOVE_CARRY, s, (carry_kernel<1><<<(int)blocks, 256, 0, s>>>(L, ids, n, rows_inout, c->dim, G)));
+    CU_CHECK(cudaGetLastError());
+    return CDLRM_OK;
+}
+
 extern "C" int cdlrm_ctx_bind_losers_sharded(cdlrm_ctx* c, const int64_t* const* h_ids, const int64_t* h_n,
                                              const int64_t* h_shard, int world, const float* const* h_peer,
                                              cdlrm_stream stream) {

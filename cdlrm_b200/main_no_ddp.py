@@ -31,6 +31,11 @@ from .model_no_ddp import (DLRM_Net, Embedding_Table_Cache_Group, Embedding_Tabl
 
 _vp = ctypes.c_void_p
 
+# --evict-victim-cache keeps the updates of the misses in the look-ahead trainer's loser store
+_VICTIM_REFUSAL = ("--evict-victim-cache trains on one GPU with the look-ahead trainer: use --world-size 1 and no "
+                   "--strict-reference (there is no loser store on the reference's path, and at N > 1 the ranks' private "
+                   "stores would need a cross-rank average of their rows, a follow-up)")
+
 # Trainer.evaluate: loss = mean BCE, accuracy = share of round(z) == t, auc = exact ROC AUC (NaN with one class only)
 EvalResult = collections.namedtuple("EvalResult", "samples loss accuracy auc positives negatives")
 _ONE_ID_PER_BAG = "evaluate needs one id per bag: lS_o must be arange(batch) for every table"
@@ -446,12 +451,18 @@ class Trainer:
             self._lr_state = torch.zeros(ctypes.sizeof(_lib.LrState) // 8, dtype=torch.int64, device=self.dev)
             lrs = self._lr_state.view(torch.float32)
             self._lr_dense, self._lr_sparse = lrs[0:1], lrs[1:2]     # LrState.lr: [dense, sparse]
+        # --evict-victim-cache: a lookup that misses the cache gets the update a cached one gets (DESIGN.md section 14)
+        self.evict_victim_cache = bool(getattr(args, "evict_victim_cache", False)) and not getattr(args, "inference_only", False)
+        if self.evict_victim_cache and (self.strict or world > 1):
+            raise _lib.CdlrmError(_VICTIM_REFUSAL)
+        self.cache_group.evict_victim_cache = self.evict_victim_cache
         self.planner = None
         if not self.strict:
             self.planner = WindowPlanner(self.cache_group, emb_tables, args.lookahead * args.mini_batch_size,
                                          rng=VictimRngDevice(args.numpy_rand_seed, self.dev), stream=self.side,
                                          lookahead_tags=True)
             self.planner.collect_losers = True     # un-cached ids of a window are served from an HBM loser store
+            self.planner.evict_victim_cache = self.evict_victim_cache
             self.planner.primary_evictions_only = True   # the write-back needs the winner of a replaced slot only
             # master <-> HBM traffic of the planner: host threads + cudaMemcpyAsync ("ce": the chunk loops are native,
             # hostio.cu; hardly slows the step that runs beside it) when this rank has host cores to spare, else
@@ -961,6 +972,7 @@ class Trainer:
                                   f"{self._window_steps} steps of window {self.window - 1} have run)")
         self._quiesce()
         self._aggregate_replicas()
+        self.planner.write_store_to_master()
         n = 0
         if self.rank == 0 or self.wb_sharded:
             n = self.planner.write_cached_to_master((self.rank, self.world) if self.wb_sharded else (0, 1))
@@ -986,7 +998,7 @@ class Trainer:
                      "table_agg_op": a.table_agg_op, "average_on_writeback": bool(a.average_on_writeback),
                      "learning_rate": float(a.learning_rate), "lr_embeds": float(a.lr_embeds),
                      "lr_num_warmup_steps": self.lr_schedule[0], "lr_decay_start_step": self.lr_schedule[1],
-                     "lr_num_decay_steps": self.lr_schedule[2]},
+                     "lr_num_decay_steps": self.lr_schedule[2], "evict_victim_cache": self.evict_victim_cache},
         }
 
     def save_checkpoint(self, path, epoch=0):
@@ -1007,6 +1019,7 @@ class Trainer:
         state, draws, ev = snap
         ev.synchronize()
         self._aggregate_replicas()
+        self.planner.write_store_to_master()      # --evict-victim-cache: the installed window's trained loser rows
         meta = dict(self.checkpoint_fields(),
                     resume={"epoch": int(epoch), "window": int(w), "global_step": int(self.global_step)},
                     rng={"state": [int(x) for x in state.numpy().view(np.uint32)], "draws": int(draws)})
@@ -1046,7 +1059,10 @@ class Trainer:
         if self._installed is not None or self.global_step or self._n_submitted:
             raise _lib.CdlrmError("load_checkpoint needs a freshly built Trainer")
         meta = ckpt.read_meta(path)
-        ckpt.check_meta(meta, self.checkpoint_fields())
+        expected = self.checkpoint_fields()
+        if getattr(self.args, "inference_only", False):    # evaluation reads the tables however the misses were trained
+            expected["args"]["evict_victim_cache"] = bool(meta.get("args", {}).get("evict_victim_cache", False))
+        ckpt.check_meta(meta, expected)
         rd = ckpt.Reader(path, meta)
         dev, cg = self.dev, self.cache_group
         h2d = 0.0
@@ -1480,6 +1496,8 @@ def _derive_topology(args):
         sys.exit("ERROR: --lr-num-warmup-steps, --lr-decay-start-step and --lr-num-decay-steps must not be negative")
     if D < W:
         sys.exit("ERROR: Learning rate warmup must finish before the decay starts")
+    if args.evict_victim_cache and not args.inference_only and (args.world_size > 1 or args.strict_reference):
+        sys.exit("ERROR: " + _VICTIM_REFUSAL)
     if args.qr_flag or args.md_flag:
         sys.exit("ERROR: QR / mixed-dimension embeddings are outside the cache hot path (unreachable from the "
                  "reference's own Run as well)")

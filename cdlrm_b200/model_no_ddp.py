@@ -169,6 +169,7 @@ class _LookupFn(torch.autograd.Function):
         ctx.slots = slots
         ctx.bag_ids = bag_ids
         ctx.n_idx = n_idx
+        ctx.ids = ids if group.evict_victim_cache else None
         # the backward's de-duplication plan only needs the slots: build it now on a side
         # stream so that it overlaps the MLP forward instead of sitting on the critical path
         ctx.plan = group._early_plan(tb, slots, n_idx) if group.early_plan else None
@@ -197,7 +198,7 @@ class _LookupFn(torch.autograd.Function):
             zero = torch.zeros_like(g0)
             keep = torch.stack([g if g is not None else zero for g in grads]).contiguous()
             base, rs, ld = keep, d, keep.stride(0)
-        group._queue_update(ctx.tb, ctx.slots, ctx.bag_ids, ctx.n_idx, base, ld, rs, keep, ctx.plan)
+        group._queue_update(ctx.tb, ctx.slots, ctx.bag_ids, ctx.n_idx, base, ld, rs, keep, ctx.plan, ctx.ids)
         return (None,) * 7
 
 
@@ -239,6 +240,9 @@ class Embedding_Table_Cache_Group(nn.Module):
         # the event that marks the lookups' gradients ready, beside the rest of the backward (the bottom MLP);
         # optimizer_embeds.step() (pre-step hook) joins it
         self.overlap_update = False
+        # --evict-victim-cache: the sparse update of a miss also goes into its row of the installed window's loser store
+        # (cdlrm_embed_victim_update), so that the cache geometry does not change what the model learns
+        self.evict_victim_cache = False
         self._upd_done = None
         self._fwd_done = None
         self._plan_stream = None
@@ -469,6 +473,9 @@ class Embedding_Table_Cache_Group(nn.Module):
                              "(model_no_ddp.py:177-179)")
         if f.value & 2:
             raise IndexError("sparse index outside its embedding table")
+        if f.value & 4:
+            raise _lib.CdlrmError("--evict-victim-cache: a lookup missed on an id that is not in the loser store of the "
+                                  "installed window, so its update had nowhere to go (a batch outside its window?)")
         return f.value
 
     # -- backward + SGD (main_no_ddp.py:376,409,413) ----------------------------------------------
@@ -496,8 +503,8 @@ class Embedding_Table_Cache_Group(nn.Module):
         slots.record_stream(ps)
         return (buf, base, done)
 
-    def _queue_update(self, tb, slots, bag_ids, n_idx, dbase, ld, rs, keep, plan=None):
-        item = (tb, slots, bag_ids, n_idx, dbase, ld, rs, keep, plan)
+    def _queue_update(self, tb, slots, bag_ids, n_idx, dbase, ld, rs, keep, plan=None, ids=None):
+        item = (tb, slots, bag_ids, n_idx, dbase, ld, rs, keep, plan, ids)
         if self.fused_lr is not None:
             self._apply_update(item, self.fused_lr)
             if self._upd_done is not None:
@@ -507,7 +514,7 @@ class Embedding_Table_Cache_Group(nn.Module):
             _GROUPS.add(self)
 
     def _apply_update(self, item, lr):
-        tb, slots, bag_ids, n_idx, dbase, ld, rs, _keep, plan = item
+        tb, slots, bag_ids, n_idx, dbase, ld, rs, _keep, plan, ids = item
         if n_idx == 0:
             return
         dev = self.device
@@ -522,7 +529,7 @@ class Embedding_Table_Cache_Group(nn.Module):
                 us.wait_event(ready)
             else:
                 us.wait_stream(cur)
-            for t in (dbase, slots, bag_ids):
+            for t in (dbase, slots, bag_ids, ids):
                 if t is not None:
                     t.record_stream(us)
             cur = us
@@ -545,6 +552,14 @@ class Embedding_Table_Cache_Group(nn.Module):
         else:
             check(lib.cdlrm_embed_bwd_sgd(self._ctx, tb, T, _vp(base), n_idx, *bag, _vp(dbase.data_ptr()), ld, rs,
                                           float(lr), s))
+        if ids is not None:
+            # the misses' updates into the loser store, same stream and learning rate
+            vic = (self._ctx, tb, T, _vp(slots.data_ptr()), slots.stride(0), _vp(ids.data_ptr()), ids.stride(0), n_idx,
+                   *bag, _vp(dbase.data_ptr()), ld, rs)
+            if isinstance(lr, torch.Tensor):
+                check(lib.cdlrm_embed_victim_update_dlr(*vic, _vp(lr.data_ptr()), s))
+            else:
+                check(lib.cdlrm_embed_victim_update(*vic, float(lr), s))
         if us is not None:
             self._upd_done = torch.cuda.Event()
             self._upd_done.record(us)

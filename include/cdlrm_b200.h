@@ -74,7 +74,8 @@ int cdlrm_ctx_reserve(cdlrm_ctx* ctx, int64_t max_idx);
 /* tags[k][:] = -1 for all tables (live and plan copies) */
 int cdlrm_tags_reset(cdlrm_ctx* ctx, cdlrm_stream stream);
 /* sticky device-side error flags (bit0: aux region overflow, model_no_ddp.py:177-179
- * would raise IndexError); synchronises `stream`; clears the flags */
+ * would raise IndexError; bit1: id outside its table; bit2: a miss whose id is not in the bound loser store,
+ * cdlrm_embed_victim_update); synchronises `stream`; clears the flags */
 int cdlrm_ctx_check(cdlrm_ctx* ctx, cdlrm_stream stream, uint32_t* h_flags);
 
 /* ---- forward: Embedding_Table_Cache_Group.forward, model_no_ddp.py:149-212 ------
@@ -129,6 +130,25 @@ int cdlrm_embed_bwd_sgd_dlr(cdlrm_ctx* ctx, int table_begin, int table_count,
                             const int32_t* bag_ids, int64_t ld_bag,
                             const float* d_out, int64_t ld_dout, int64_t dout_row_stride,
                             const float* d_lr, cdlrm_stream stream);
+
+/* ---- update of the misses (--evict-victim-cache; the reference parses the flag and drops these updates) ----------
+ * A miss of the step is a position j whose slot is an aux slot (>= num_sets * num_ways); its row came from the loser
+ * store bound with cdlrm_ctx_bind_losers.  Per table and store row i:
+ *     store[i] = fma(-lr, sum of d_out[bag(j)] over the misses j on i in ascending j, store[i])
+ * (bag(j) = bag_ids[j], or j with bag_ids == NULL; d_out rows as in cdlrm_embed_bwd_sgd).  A miss whose id is not in
+ * the store raises flag 4 (cdlrm_ctx_check) and is not applied.  Deterministic, capturable, allocates nothing; at most
+ * CDLRM_SORT_MAX misses per table (min(aux_rows, n_idx) <= CDLRM_SORT_MAX). */
+int cdlrm_embed_victim_update(cdlrm_ctx* ctx, int table_begin, int table_count,
+                              const int32_t* slots, int64_t ld_slots, const int64_t* ids, int64_t ld_ids, int32_t n_idx,
+                              const int32_t* bag_ids, int64_t ld_bag,
+                              const float* d_out, int64_t ld_dout, int64_t dout_row_stride,
+                              float lr, cdlrm_stream stream);
+/* The same with the learning rate read from *d_lr when the kernel runs (a cdlrm_lr_state's lr[1]). */
+int cdlrm_embed_victim_update_dlr(cdlrm_ctx* ctx, int table_begin, int table_count,
+                                  const int32_t* slots, int64_t ld_slots, const int64_t* ids, int64_t ld_ids,
+                                  int32_t n_idx, const int32_t* bag_ids, int64_t ld_bag,
+                                  const float* d_out, int64_t ld_dout, int64_t dout_row_stride,
+                                  const float* d_lr, cdlrm_stream stream);
 
 /* ---- interaction: DLRM_Net.interact_features ("dot"), model_no_ddp.py:272-293 ---
  * feat[0] = x, feat[1..] = ly; h_feat is a host array of n_feat device pointers to
@@ -328,6 +348,11 @@ int cdlrm_move_gather_master(cdlrm_ctx* ctx, int table, const int64_t* ids, int6
  * master[k][fill_ids[i]] directly); live tags[k][slot % S][slot / S] = fill_ids[i] */
 int cdlrm_move_fill(cdlrm_ctx* ctx, int table, const int64_t* fill_ids, const int32_t* fill_slots,
                     int64_t n, const float* rows, const int64_t* src_index, cdlrm_stream stream);
+/* rows_inout[i] = the row of ids[i] in the currently bound loser store of table k, for every ids[i] the store holds;
+ * the other rows are left alone (--evict-victim-cache: the next window's prefetched rows of ids trained in this
+ * window's store).  No store ever bound: nothing to do. */
+int cdlrm_move_carry_losers(cdlrm_ctx* ctx, int table, const int64_t* ids, int64_t n, float* rows_inout,
+                            cdlrm_stream stream);
 
 /* ---- table aggregation: broadcast_and_aggregate, main_no_ddp.py:250-292 ---------
  * collect: ascending list of dirty slots per table (torch.unique(sorted=True) :270);
